@@ -23,6 +23,11 @@ roofline, clocks sampled during its timed region, and - at N = 1 - a cpu_baselin
   python bench.py [--gpus N] [--steps K] [--warmup W] [--configs C4S,C3,C5]   our arm (one process per GPU under torchrun)
   python bench.py --impl reference [...]                                      CPU arm: the oracle's restatement of the
                                                                               reference loop on all host threads
+
+--dump-outputs DIR writes what the headline's timed call returned in its last step as DIR/<name>.npy (float64): poses.npy
+(S, 7) and one result_<field>.npy (S,) per locreg_result field, S = every scan of the step (all ranks, rank order; the
+reference arm: its sample).  The inputs are seeded, so two builds run with the same arguments can be compared output for
+output.
 """
 import argparse
 import json
@@ -47,7 +52,8 @@ C4_SCANS = 4096
 def parse():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=10)
+    ap.add_argument("--steps", type=int, default=10,
+                    help="timed steps of the headline, C4S and C3 (C5 times one relocalisation of more than 8192 hypotheses)")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--scans-per-gpu", type=int, default=512)
@@ -59,7 +65,11 @@ def parse():
     ap.add_argument("--hyp", type=int, default=65536, help="C5: number of pose hypotheses (64x64 xy grid x 16 yaws)")
     ap.add_argument("--ndt-map-points", type=int, default=20_000_000)
     ap.add_argument("--c4-scans", type=int, default=C4_SCANS)
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the headline's outputs of its last timed step to DIR/<name>.npy")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    return args
 
 
 def make_world(args):
@@ -130,6 +140,25 @@ def _pose_delta(a, b):
     return 2.0 * float(np.arccos(min(1.0, d))), float(np.linalg.norm(a[4:] - b[4:]))
 
 
+MAX_DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, poses, results):
+    """--dump-outputs: `poses` (S, 7) and `results` (result field -> S values) as float64 out_dir/<name>.npy.  Past
+    MAX_DUMP_BYTES in all, a fixed seeded sample of the scans is written, their indices as scan_index.npy."""
+    arrays = {"poses": np.asarray(poses, np.float64)}
+    arrays.update({"result_" + k: np.asarray(v, np.float64) for k, v in results.items()})
+    S = len(arrays["poses"])
+    row_bytes = sum(a.nbytes for a in arrays.values()) // max(S, 1)
+    if S * row_bytes > MAX_DUMP_BYTES:
+        keep = np.sort(np.random.default_rng(0).choice(S, MAX_DUMP_BYTES // (row_bytes + 8), replace=False))
+        arrays = {k: a[keep] for k, a in arrays.items()}
+        arrays["scan_index"] = keep.astype(np.float64)
+    os.makedirs(out_dir, exist_ok=True)
+    for k, a in arrays.items():
+        np.save(os.path.join(out_dir, k + ".npy"), a)
+
+
 def cpu_baseline_icp(map_cloud, clouds, offsets, init, n_scans, threads):
     """Times the oracle (std-only restatement of IcpRegistration, literal always-on ANN kd-tree search = what the
     reference runs) on `n_scans` scans with `threads` host threads.  Map build is not included (as for the GPU).
@@ -181,8 +210,10 @@ def run_reference(args):
         ref.align_batch(clouds, offsets, init, threads=threads)
     t0 = time.perf_counter()
     for _ in range(args.steps):
-        _, _, used = ref.align_batch(clouds, offsets, init, threads=threads)
+        poses, res, used = ref.align_batch(clouds, offsets, init, threads=threads)
     dt = time.perf_counter() - t0
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, poses, {k: [r[k] for r in res] for k in res[0]})
     pts = int(offsets[-1]) * args.steps
     val = pts / dt
     line = {"impl": "reference", "metric": METRIC, "value": val, "unit": UNIT, "n_gpus": args.gpus, "steps": args.steps,
@@ -261,6 +292,14 @@ class Ctx:
             self.dist.all_reduce(t, op=self.dist.ReduceOp.MAX if op == "max" else self.dist.ReduceOp.SUM)
         return [float(x) for x in t.cpu()]
 
+    def gather(self, t):
+        """Rows of an equally shaped device tensor of every rank, in rank order, on the host."""
+        if self.world_size > 1:
+            out = self.torch.empty((self.world_size * t.shape[0],) + tuple(t.shape[1:]), dtype=t.dtype, device=self.dev)
+            self.dist.all_gather_into_tensor(out, t.contiguous())
+            t = out
+        return t.cpu().numpy()
+
     def close(self):
         self.sampler.stop()
         if self.world_size > 1:
@@ -308,6 +347,12 @@ def bench_icp(ctx, reg, map_cloud, clouds, offsets, init, gt, map_build):
     ctx.barrier()
     wall1 = time.perf_counter()
     dev_ms = ev0.elapsed_time(ev1)
+    if args.dump_outputs:  # what the last timed step handed its caller: poses and locreg_result records
+        from loc_lib_b200 import _lib
+        poses, rec = ctx.gather(d_pout), ctx.gather(d_res.view(B, -1))
+        rec = np.frombuffer(rec.tobytes(), np.dtype(_lib.Result))
+        if ctx.rank == 0:
+            dump_outputs(args.dump_outputs, poses, {k: rec[k] for k in rec.dtype.names if k != "pad_"})
 
     # ---- end to end through host buffers
     for _ in range(2):
@@ -400,7 +445,7 @@ def bench_c4_strong(ctx, reg, clouds, offsets, init, gt, S_global):
     d_pin = torch.from_numpy(init).to(dev)
     d_pout = torch.zeros_like(d_pin)
     d_res = torch.zeros(max(S_local, 1) * 48, dtype=torch.uint8, device=dev)
-    steps = max(1, min(args.steps, 10))
+    steps = args.steps
 
     def step_resident():
         reg.ScanMatchBatchDevice(d_src.data_ptr(), d_off.data_ptr(), d_pin.data_ptr(), S_local, n_pts, d_pout.data_ptr(), d_res.data_ptr())
@@ -601,7 +646,7 @@ def bench_reloc(ctx, reg, world, map_cloud):
     warm = hyp[:: max(1, len(hyp) // (256 * ctx.world_size))][:256 * ctx.world_size]
     for _ in range(2):
         reg.RelocaliseSharded(scan, warm)
-    steps = 1 if len(hyp) > 8192 else max(1, min(args.steps, 5))
+    steps = 1 if len(hyp) > 8192 else args.steps
     times, kernel, launches = [], [], 0
     ctx.barrier()
     wall0 = time.perf_counter()

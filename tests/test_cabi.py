@@ -3,6 +3,7 @@ reference's option defaults, validates arguments, and FAILS LOUDLY without a GPU
 import ctypes as C
 import os
 import re
+import shutil
 import subprocess
 
 import numpy as np
@@ -35,7 +36,10 @@ def test_header_symbols_exported():
 
 def test_library_is_sm100a_and_self_contained():
     so = os.path.join(ROOT, "loc_lib_b200", "liblocreg.so")
-    out = subprocess.run(["cuobjdump", "-lelf", so], capture_output=True, text=True).stdout
+    # the CUDA tools need not be on PATH: fall back to the toolkit of the nvcc csrc/Makefile builds with
+    nvcc = os.environ.get("NVCC", "/usr/local/cuda/bin/nvcc")
+    cuobjdump = shutil.which("cuobjdump") or os.path.join(os.path.dirname(nvcc), "cuobjdump")
+    out = subprocess.run([cuobjdump, "-lelf", so], capture_output=True, text=True).stdout
     assert "sm_100a" in out
     needed = subprocess.run(["readelf", "-d", so], capture_output=True, text=True).stdout
     assert "liboracle" not in needed and "hostsim" not in needed  # the product never links test infrastructure
