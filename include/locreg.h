@@ -125,6 +125,22 @@ int locreg_align(locreg_handle* h, const float* src, size_t n, size_t stride_byt
 int locreg_compute_hb(locreg_handle* h, const float* src, size_t n, size_t stride_bytes, const double* pose,
                       double* H36, double* B6, locreg_result* res);
 
+/* LoamRegistration::ScanMatch's loop (loam_registration.cpp:38-99, SURVEY 3.3) on the device, with no host round trip
+ * between iterations.  Per trip, at the current pose: the surf cloud's H/B on the `surf` handle (LOCREG_ICP_P2PLANE)
+ * and the edge cloud's on the `edge` handle (LOCREG_ICP_P2LINE), each with its own handle's gates, exactly as
+ * locreg_compute_hb computes them; H = Hs + He, B = Bs + Be (the halves' degenerate flags do not gate the sum);
+ * dx = H^-1 B; R <- R Exp(dx[0:3]), t <- t + dx[3:6]; stop when |dx| < eps or after max_iteration trips.  A trip with
+ * det(H) == 0 makes no update.  The loop starts from pose_in as given (zero_initial_translation does not apply); the
+ * handles' own max_iteration / eps are not used.  The two halves of a trip run concurrently on the two handles'
+ * streams (serially when both were given the same stream with locreg_set_stream).  Clouds share one stride; either may
+ * be empty (that half contributes zeros).  pose_out is always written.  res2 (may be NULL) has 2 entries, [0] surf and
+ * [1] edge: iters / updates / converged / pose_written are the loop's (equal in both), degenerate / n_effective /
+ * n_inlier / sum_sq_res that half's last evaluation, as locreg_compute_hb reports it at that pose.
+ * locreg_last_timing(surf) reports the call's kernels.  Both handles need a target (LOCREG_E_STATE). */
+int locreg_align_loam(locreg_handle* surf, locreg_handle* edge, const float* surf_xyz, size_t n_surf, const float* edge_xyz,
+                      size_t n_edge, size_t stride_bytes, const double* pose_in, int32_t max_iteration, double eps,
+                      double* pose_out, locreg_result* res2);
+
 /* Parity probe for SearchPointInterface::FindNearstPoints (search_point_interface.h:9-24; kdtree.cpp:272-283):
  * exact k-NN (k = 1 or 5) under the total order (float32 dis2, index); idx is nq*k, -1 padded. ICP handles only.
  * Runs the production search: stage 1 per thread, then the queued rest per warp (small probes, like one scan) or per

@@ -216,6 +216,46 @@ class CudaNdtRegistration : public CudaRegistrationBase {
     NdtOptions options_;
 };
 
+// LoamRegistration::ScanMatch's loop (loam_registration.cpp:38-99, SURVEY.md 3.3) on the device: a P2Plane
+// CudaIcpRegistration for the surf cloud and a P2Line one for the edge cloud, each with its own options and gates; one
+// Align call runs every Gauss-Newton trip (both halves' H and B summed, one step) with no host round trip in between
+// (locreg_align_loam).  max_iteration and eps are the LOAM loop's (LoamOption), not either half's.  It does not implement
+// MatchingInterface's two-cloud overloads: the names here say which cloud is which.
+class CudaLoamMatcher {
+   public:
+    CudaLoamMatcher(IcpOptions surf_options, IcpOptions edge_options, int max_iteration = 10, double eps = 1e-2, int device = 0)
+        : surf_(Checked(surf_options, IcpMethod::P2PLANE, "surf"), device),
+          edge_(Checked(edge_options, IcpMethod::P2LINE, "edge"), device),
+          max_iteration_(max_iteration), eps_(eps) {}
+
+    void SetTargets(const CloudPtr& surf_map, const CloudPtr& edge_map) {
+        surf_.SetInputTarget(surf_map);
+        edge_.SetInputTarget(edge_map);
+    }
+    // result_pose is always written.  LastResults()[0] / [1]: the loop's trips, updates and convergence, and the surf /
+    // edge half's last evaluation.
+    void Align(const CloudPtr& surf, const CloudPtr& edge, const SE3& predict_pose, SE3& result_pose) {
+        locreg_detail::check(locreg_align_loam(surf_.Handle(), edge_.Handle(), locreg_detail::cloud_xyz(*surf), surf->points.size(),
+                                               locreg_detail::cloud_xyz(*edge), edge->points.size(), sizeof(PointType),
+                                               predict_pose.data(), max_iteration_, eps_, result_pose.data(), last_results_),
+                             "locreg_align_loam");
+    }
+    const locreg_result* LastResults() const { return last_results_; }
+    CudaIcpRegistration& Surf() { return surf_; }
+    CudaIcpRegistration& Edge() { return edge_; }
+
+   private:
+    static IcpOptions Checked(IcpOptions o, IcpMethod want, const char* half) {
+        if (o.method_ != want) throw std::runtime_error(std::string("CudaLoamMatcher: the ") + half + " half needs " +
+                                                        (want == IcpMethod::P2PLANE ? "P2PLANE" : "P2LINE") + " options");
+        return o;
+    }
+    CudaIcpRegistration surf_, edge_;
+    int max_iteration_;
+    double eps_;
+    locreg_result last_results_[2] = {};
+};
+
 // ---- the two callers' loops around ScanMatch, with the map state on the device ------------------------------------
 // Loc::Update without the ROS / ESKF parts (loc.cpp:208-246): ScanMatch from the constant-velocity prediction, and a new
 // local map (crop of the device-resident global map) whenever the pose comes within `margin` of the box edge.

@@ -918,27 +918,11 @@ __device__ __forceinline__ bool apply_outcome(int outcome, DevResult& r) {
     return outcome == 2 || outcome == 3 || outcome == 4;
 }
 
-// One warp per scan.  mode 1: Gauss-Newton iteration (update the pose; stop on convergence or after
-// max_iteration trips); mode 0: evaluation only (compute_hb, relocalisation's final score pass): record the sums,
-// leave the pose.  acc_out (optional, 32 doubles per scan) receives the raw sums.
-// partials_b (optional): a second partial row per tile (k_icp_pending, icp_fused.cuh), added after the first ones.
-template <int METHOD>
-__global__ void __launch_bounds__(128) k_icp_solve(IcpParams prm, BatchView bv, AlignState* states,
-                                                   const double* __restrict__ partials, const double* __restrict__ partials_b,
-                                                   int mode, double* acc_out) {
-    __shared__ double sums[4][32];
-    const unsigned int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-    const unsigned int s = blockIdx.x * 4 + warp;
-    if (s >= bv.S) return;
-    AlignState* st = states + s;
-    if (mode == 1 && st->stop) return;
-    unsigned int t0, t1;
-    if (bv.tile_begin) { t0 = bv.tile_begin[s]; t1 = bv.tile_begin[s + 1]; }
-    else {
-        t0 = s * bv.tiles_per_item;
-        t1 = t0 + (bv.n_single + kTile - 1) / kTile;
-    }
-    // four interleaved running sums keep four loads in flight (the loop is pure latency); fixed order all the same
+// Sum over tiles [t0, t1) of partial-row entry `lane` (< 30; other lanes get 0), in a fixed order: four interleaved
+// running sums keep four loads in flight (the loop is pure latency).  partials_b (optional): a second partial row per
+// tile (k_icp_pending, icp_fused.cuh), added after the first ones.
+__device__ __forceinline__ double icp_sum_tiles(const double* __restrict__ partials, const double* __restrict__ partials_b,
+                                                unsigned int t0, unsigned int t1, unsigned int lane) {
     double v0 = 0, v1 = 0, v2 = 0, v3 = 0;
     if (lane < 30) {
         const double* col = partials + lane;
@@ -964,7 +948,30 @@ __global__ void __launch_bounds__(128) k_icp_solve(IcpParams prm, BatchView bv, 
             v1 = v2 = v3 = 0;
         }
     }
-    sums[warp][lane] = (v0 + v1) + (v2 + v3);
+    return (v0 + v1) + (v2 + v3);
+}
+
+// One warp per scan.  mode 1: Gauss-Newton iteration (update the pose; stop on convergence or after
+// max_iteration trips); mode 0: evaluation only (compute_hb, relocalisation's final score pass): record the sums,
+// leave the pose.  acc_out (optional, 32 doubles per scan) receives the raw sums.
+// partials_b (optional): a second partial row per tile (k_icp_pending, icp_fused.cuh), added after the first ones.
+template <int METHOD>
+__global__ void __launch_bounds__(128) k_icp_solve(IcpParams prm, BatchView bv, AlignState* states,
+                                                   const double* __restrict__ partials, const double* __restrict__ partials_b,
+                                                   int mode, double* acc_out) {
+    __shared__ double sums[4][32];
+    const unsigned int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+    const unsigned int s = blockIdx.x * 4 + warp;
+    if (s >= bv.S) return;
+    AlignState* st = states + s;
+    if (mode == 1 && st->stop) return;
+    unsigned int t0, t1;
+    if (bv.tile_begin) { t0 = bv.tile_begin[s]; t1 = bv.tile_begin[s + 1]; }
+    else {
+        t0 = s * bv.tiles_per_item;
+        t1 = t0 + (bv.n_single + kTile - 1) / kTile;
+    }
+    sums[warp][lane] = icp_sum_tiles(partials, partials_b, t0, t1, lane);
     __syncwarp();
     if (lane == 0) {
         const double* acc30 = sums[warp];
@@ -977,6 +984,51 @@ __global__ void __launch_bounds__(128) k_icp_solve(IcpParams prm, BatchView bv, 
             st->res.iters += 1;
             const int outcome = icp_gn_update<METHOD>(acc30, static_cast<unsigned int>(acc30[28]), prm, T);
             if (apply_outcome(outcome, st->res) || st->res.iters >= prm.max_iteration) st->stop = 1;
+            pose_store(T, st->pose);
+        }
+    }
+}
+
+// One Gauss-Newton trip of LoamRegistration::ScanMatch (SURVEY.md 3.3): the P2Plane (surf) half's and the P2Line
+// (edge) half's partial rows are summed separately, in k_icp_solve's order, then added; H dx = B is solved and the
+// pose updated as in the ICP loop, but with neither icp_gn_update's min_effective_pts gate (the halves' own flags do
+// not gate the sum) nor P2P's /16.  A singular sum makes no update (outcome 0).  One warp, one state; half[0] / half[1]
+// receive each half's counts and degenerate flag as locreg_compute_hb reports them at the trip's pose.
+__global__ void __launch_bounds__(32) k_loam_solve(AlignState* st, unsigned int tiles_surf, const double* __restrict__ surf,
+                                                   const double* __restrict__ surf_b, int min_eff_surf, unsigned int tiles_edge,
+                                                   const double* __restrict__ edge, const double* __restrict__ edge_b,
+                                                   int min_eff_edge, double eps, int max_iteration, DevResult* half) {
+    __shared__ double sums[3][32];
+    const unsigned int lane = threadIdx.x & 31;
+    if (st->stop) return;
+    const double s = icp_sum_tiles(surf, surf_b, 0, tiles_surf, lane);
+    const double e = icp_sum_tiles(edge, edge_b, 0, tiles_edge, lane);
+    sums[0][lane] = s;
+    sums[1][lane] = e;
+    sums[2][lane] = s + e;
+    __syncwarp();
+    if (lane < 3) {  // lanes 0 / 1: the halves' own records (their degenerate flags need det of their own H); lane 2: the update
+        const double* acc = sums[lane];
+        double dx[6];
+        const bool solvable = gn_solve6(acc, acc + 21, dx);
+        if (lane < 2) {
+            DevResult& r = half[lane];
+            result_from_acc(r, acc);
+            r.degenerate = (!solvable || r.n_effective < (lane == 0 ? min_eff_surf : min_eff_edge)) ? 1 : 0;
+        } else {
+            result_from_acc(st->res, acc);
+            Pose T;
+            pose_load(T, st->pose);
+            st->res.iters += 1;
+            int outcome = 0;
+            if (solvable) {
+                pose_update(T, dx);
+                double nrm = 0;
+#pragma unroll
+                for (int i = 0; i < 6; ++i) nrm += dx[i] * dx[i];
+                outcome = sqrt(nrm) < eps ? 2 : 1;
+            }
+            if (apply_outcome(outcome, st->res) || st->res.iters >= max_iteration) st->stop = 1;
             pose_store(T, st->pose);
         }
     }

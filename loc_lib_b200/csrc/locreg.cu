@@ -84,6 +84,7 @@ struct locreg_handle {
     std::vector<cudaEvent_t> chunk_events;     // locreg_align_batch
     std::vector<cudaStream_t> chunk_streams;   // compute streams of the chunks after the first (they run concurrently)
     std::vector<cudaEvent_t> chunk_done;       // ... and the events that join them into `stream`
+    cudaEvent_t loam_ev[2] = {nullptr, nullptr}; // locreg_align_loam (surf handle): [0] state ready / solved, [1] edge half evaluated
     DeviceVoxelMap icp_map;     // level 0: cells of knn_cell_size, neighbourhood lists
     DeviceVoxelMap icp_coarse[kCoarseLevels];  // cells 4x, 16x larger, block tables only (far queries)
     DeviceVoxelMap icp_mid;     // cells 2x larger, neighbourhood lists: stage 2 of the search (LOCREG_MID=0: off)
@@ -105,7 +106,7 @@ struct locreg_handle {
     int comm_rank = 0, comm_world = 1;
     DevBuf d_gather_pose, d_gather_res, d_bcast;
     DevBuf d_raw, d_src4, d_out, d_partials, d_state, d_acc, d_gate, d_nn, d_offsets, d_poses_in, d_poses_out, d_results,
-        d_scores, d_misc, d_target, d_nnpos, d_tile_begin, d_tiles, d_states, d_ringq, d_ringc, d_sortq, d_sortb, d_sorth, d_rescanq, d_rescanc, d_lmap_new, d_global, d_local, d_same, d_plane, d_pstat, d_track;
+        d_scores, d_misc, d_target, d_nnpos, d_tile_begin, d_tiles, d_states, d_ringq, d_ringc, d_sortq, d_sortb, d_sorth, d_rescanq, d_rescanc, d_loam, d_lmap_new, d_global, d_local, d_same, d_plane, d_pstat, d_track;
     size_t n_global = 0, global_stride = 0;  // Loc's global map kept on the device (locreg_set_global_map)
     // Lio's sliding local map (locreg_local_map_add_keyframe): transformed key frames + the filtered local map
     struct KeyFrame { void* p = nullptr; size_t n = 0; };
@@ -498,23 +499,55 @@ void icp_launch_solve(locreg_handle* h, const IcpJob& job, int mode, double* acc
               h->d_partials.as<double>() + job.partials_off, partials_b, mode, acc_out);
     prof_mark(h, 2, false);
 }
+// Search mode of Gauss-Newton trip `it` of a job whose per-point scratch holds its own previous trips.
+int icp_loop_nn_mode(int it) {
+    static const int tp_iters = getenv("LOCREG_TWOPASS_ITERS") ? atoi(getenv("LOCREG_TWOPASS_ITERS")) : 1;  // iterations whose scan uses the threshold pre-pass (the unseeded one; 1 measured best: 11.2 ms vs 11.5 at 2, 12.0 at 3)
+    static const int track = getenv("LOCREG_TRACK") ? atoi(getenv("LOCREG_TRACK")) : 1;  // 0: every query scans its list every time
+    static const int track_from = getenv("LOCREG_TRACK_FROM") ? atoi(getenv("LOCREG_TRACK_FROM")) : 3;  // measured: 2 and 3 alike, 4 +1 % on batches; single scans converge sooner
+    // the first tracked iteration searches every point (no margins yet): the three-kernel pipeline; from then on the
+    // streaming pass of icp_fused.cuh (P2Plane)
+    const int seeded = track && it >= track_from ? (kNnSeeds | kNnTrack | (it > track_from ? kNnFused : kNnFirstTrack)) : kNnSeeds;
+    return it == 0 ? kNnTwoPass : (it < tp_iters ? (kNnSeeds | kNnTwoPass) : seeded);
+}
 // The whole Gauss-Newton loop, queued on the stream without a host round-trip; stopped scans make their tiles exit.
 template <int METHOD>
 void icp_run_loop(locreg_handle* h, const IcpJob& job, int final_eval) {
     for (int it = 0; it < h->opt.max_iteration; ++it) {
-        static const int tp_iters = getenv("LOCREG_TWOPASS_ITERS") ? atoi(getenv("LOCREG_TWOPASS_ITERS")) : 1;  // iterations whose scan uses the threshold pre-pass (the unseeded one; 1 measured best: 11.2 ms vs 11.5 at 2, 12.0 at 3)
-        static const int track = getenv("LOCREG_TRACK") ? atoi(getenv("LOCREG_TRACK")) : 1;  // 0: every query scans its list every time
-        static const int track_from = getenv("LOCREG_TRACK_FROM") ? atoi(getenv("LOCREG_TRACK_FROM")) : 3;  // measured: 2 and 3 alike, 4 +1 % on batches; single scans converge sooner
-        // the first tracked iteration searches every point (no margins yet): the three-kernel pipeline; from then on the
-        // streaming pass of icp_fused.cuh (P2Plane)
-        const int seeded = track && it >= track_from ? (kNnSeeds | kNnTrack | (it > track_from ? kNnFused : kNnFirstTrack)) : kNnSeeds;
-        const double* pb = icp_launch_eval<METHOD>(h, job, 0, it == 0 ? kNnTwoPass : (it < tp_iters ? (kNnSeeds | kNnTwoPass) : seeded), nullptr, nullptr);
+        const double* pb = icp_launch_eval<METHOD>(h, job, 0, icp_loop_nn_mode(it), nullptr, nullptr);
         icp_launch_solve<METHOD>(h, job, 1, nullptr, pb);
     }
     if (final_eval) {
         const double* pb = icp_launch_eval<METHOD>(h, job, 1, h->opt.max_iteration > 0 ? kNnSeeds : kNnTwoPass, nullptr, nullptr);
         icp_launch_solve<METHOD>(h, job, 0, nullptr, pb);
     }
+}
+// LoamRegistration::ScanMatch's loop (SURVEY.md 3.3), all trips queued with no host round trip.  Each trip evaluates the
+// surf half (P2Plane) on surf's stream and scratch and the edge half (P2Line) on edge's, both at the one pose in the
+// state both jobs point at, so the two evaluations run side by side; k_loam_solve then joins their partial rows on
+// surf's stream.  loam_ev[0] (surf stream: state uploaded / trip solved) holds the edge half back until the pose it
+// reads is final and the edge partial rows it overwrites have been read; loam_ev[1] (edge stream: edge half evaluated)
+// holds the solve back.  With both handles on one stream the same calls run serially.  An empty half launches nothing
+// and its zero tiles sum to zeros.
+void loam_run_loop(locreg_handle* surf, locreg_handle* edge, const IcpJob& js, const IcpJob& je, int max_iteration,
+                   double eps, DevResult* d_half) {
+    LR_CUDA(cudaEventRecord(surf->loam_ev[0], surf->stream));
+    for (int it = 0; it < max_iteration; ++it) {
+        const int nn_mode = icp_loop_nn_mode(it);
+        LR_CUDA(cudaStreamWaitEvent(edge->stream, surf->loam_ev[0], 0));
+        const double* eb = icp_launch_eval<kIcpP2Line>(edge, je, 0, nn_mode, nullptr, nullptr);
+        LR_CUDA(cudaEventRecord(surf->loam_ev[1], edge->stream));
+        const double* sb = icp_launch_eval<kIcpP2Plane>(surf, js, 0, nn_mode, nullptr, nullptr);
+        LR_CUDA(cudaStreamWaitEvent(surf->stream, surf->loam_ev[1], 0));
+        prof_mark(surf, 2, true);
+        LR_LAUNCH(k_loam_solve, 1, 32, 0, surf->stream, js.states, js.n_tiles, surf->d_partials.as<double>(), sb,
+                  surf->opt.min_effective_pts, je.n_tiles, edge->d_partials.as<double>(), eb, edge->opt.min_effective_pts, eps,
+                  max_iteration, d_half);
+        prof_mark(surf, 2, false);
+        LR_CUDA(cudaEventRecord(surf->loam_ev[0], surf->stream));
+    }
+    // join: whatever the edge stream still has (its cloud copy when no trip ran) is done before surf's stream goes on
+    LR_CUDA(cudaEventRecord(surf->loam_ev[1], edge->stream));
+    LR_CUDA(cudaStreamWaitEvent(surf->stream, surf->loam_ev[1], 0));
 }
 // One scan, whole loop in ONE cooperative launch (icp_persist.cuh).  Returns false when the job does not suit it (then
 // the per-iteration pipeline runs): the persistent grid holds one block per SM, a scan of more tiles than 8x that would
@@ -748,6 +781,7 @@ int locreg_destroy(locreg_handle* h) {
     if (h->ev1) cudaEventDestroy(h->ev1);
     for (cudaEvent_t e : h->chunk_events) cudaEventDestroy(e);
     for (cudaEvent_t e : h->chunk_done) cudaEventDestroy(e);
+    for (cudaEvent_t e : h->loam_ev) if (e) cudaEventDestroy(e);
     for (cudaStream_t st : h->chunk_streams) cudaStreamDestroy(st);
     if (h->copy_stream) cudaStreamDestroy(h->copy_stream);
     if (h->comm && nccl_api().ok()) nccl_api().CommDestroy(h->comm);
@@ -892,6 +926,59 @@ int locreg_compute_hb(locreg_handle* h, const float* src, size_t n, size_t strid
         const bool few = r.n_effective < h->opt.min_effective_pts;
         r.degenerate = (!solvable || (few && h->opt.method != LOCREG_NDT_DIRECT)) ? 1 : 0;  // direct NDT only looks at det(H) here
         fill_result(res, r);
+        return LOCREG_OK;
+    });
+}
+
+int locreg_align_loam(locreg_handle* surf, locreg_handle* edge, const float* surf_xyz, size_t n_surf, const float* edge_xyz,
+                      size_t n_edge, size_t stride, const double* pose_in, int32_t max_iteration, double eps, double* pose_out,
+                      locreg_result* res2) {
+    if (!surf || !edge) { g_last_error = "null handle"; return LOCREG_E_ARG; }
+    if (surf == edge) { g_last_error = "locreg_align_loam needs two distinct handles (surf and edge)"; return LOCREG_E_ARG; }
+    if (surf->device != edge->device) { g_last_error = "surf and edge handles are on different devices"; return LOCREG_E_ARG; }
+    if (surf->opt.method != LOCREG_ICP_P2PLANE || edge->opt.method != LOCREG_ICP_P2LINE) {
+        g_last_error = "locreg_align_loam needs a LOCREG_ICP_P2PLANE surf handle and a LOCREG_ICP_P2LINE edge handle";
+        return LOCREG_E_ARG;
+    }
+    int rc = check_cloud_args(surf_xyz, n_surf, stride);
+    if (rc) return rc;
+    rc = check_cloud_args(edge_xyz, n_edge, stride);
+    if (rc) return rc;
+    if (!pose_in || !pose_out) { g_last_error = "null pose"; return LOCREG_E_ARG; }
+    return guarded(surf, [&]() {
+        if (!surf->has_target || !edge->has_target) {
+            g_last_error = surf->has_target ? "SetInputTarget has not been called on the edge handle"
+                                            : "SetInputTarget has not been called on the surf handle";
+            return LOCREG_E_STATE;
+        }
+        for (cudaEvent_t& e : surf->loam_ev)
+            if (!e) LR_CUDA(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
+        const float4* src_s = stage_cloud(surf, surf_xyz, n_surf, stride, false);
+        const float4* src_e = stage_cloud(edge, edge_xyz, n_edge, stride, false);
+        init_state(surf, pose_in);  // CaculateMatrixHAndB ignores zero_initial_translation: so does the LOAM loop
+        surf->d_loam.reserve(2 * sizeof(DevResult));
+        DevResult* d_half = surf->d_loam.as<DevResult>();
+        LR_CUDA(cudaMemsetAsync(d_half, 0, 2 * sizeof(DevResult), surf->stream));
+        surf->begin_timing();
+        const IcpJob js = icp_single_job(surf, src_s, static_cast<unsigned int>(n_surf));
+        IcpJob je = icp_single_job(edge, src_e, static_cast<unsigned int>(n_edge));
+        je.states = js.states;  // one state, one pose: both halves evaluate at it
+        loam_run_loop(surf, edge, js, je, max_iteration, eps, d_half);
+        surf->h_small.reserve(4096);
+        AlignState* hs = surf->h_small.as<AlignState>() + 1;
+        DevResult* hh = reinterpret_cast<DevResult*>(hs + 1);
+        LR_CUDA(cudaMemcpyAsync(hs, js.states, sizeof(AlignState), cudaMemcpyDeviceToHost, surf->stream));
+        LR_CUDA(cudaMemcpyAsync(hh, d_half, 2 * sizeof(DevResult), cudaMemcpyDeviceToHost, surf->stream));
+        surf->end_timing();  // synchronises surf's stream, which has joined edge's
+        std::memcpy(pose_out, hs->pose, 7 * sizeof(double));
+        for (int i = 0; res2 && i < 2; ++i) {  // the loop's bookkeeping, the half's last evaluation
+            DevResult r = hh[i];
+            r.iters = hs->res.iters;
+            r.updates = hs->res.updates;
+            r.converged = hs->res.converged;
+            r.pose_written = hs->res.pose_written;
+            fill_result(res2 + i, r);
+        }
         return LOCREG_OK;
     });
 }

@@ -348,6 +348,51 @@ class IcpRegistration(_Registration):
         super().__init__(o, device)
 
 
+class LoamRegistration:
+    """LoamRegistration::ScanMatch (loam_registration.cpp:38-99, SURVEY.md 3.3) over two IcpRegistration handles: a
+    P2Plane one for the surf cloud and a P2Line one for the edge cloud, each with its own options and gates.  Every
+    Gauss-Newton trip sums the two halves' H and B and takes one step; the whole loop stays on the device
+    (locreg_align_loam).  max_iteration and eps belong to the LOAM loop (LoamOption), not to either half."""
+
+    def __init__(self, surf_options=None, edge_options=None, max_iteration=10, eps=1e-2, device=0):
+        surf_options = surf_options or IcpOptions(method_=IcpMethod.P2PLANE)
+        edge_options = edge_options or IcpOptions(method_=IcpMethod.P2LINE)
+        if surf_options.method_ != IcpMethod.P2PLANE or edge_options.method_ != IcpMethod.P2LINE:
+            raise _lib.LocregError("LoamRegistration needs P2PLANE options for the surf half and P2LINE options for the edge half")
+        self.surf = IcpRegistration(surf_options, device)
+        self.edge = IcpRegistration(edge_options, device)
+        self.max_iteration = int(max_iteration)
+        self.eps = float(eps)
+        self.last_result = None
+
+    def SetInputTarget(self, surf_map, edge_map):
+        self.surf.SetInputTarget(surf_map)
+        self.edge.SetInputTarget(edge_map)
+        return True
+
+    def ScanMatch(self, surf_cloud, edge_cloud, predict_pose):
+        """Returns (pose, (res_surf, res_edge)): iters / updates / converged are the loop's, the counts and the degenerate
+        flag each half's last evaluation."""
+        a, n_s, s_s = _cloud(surf_cloud)
+        b, n_e, s_e = _cloud(edge_cloud)
+        if s_e != s_s:  # the C ABI takes one stride for both clouds
+            b = np.ascontiguousarray(np.pad(b[:, :3], ((0, 0), (0, s_s // 4 - 3))), np.float32)
+        pin = _pose(predict_pose)
+        pout = pin.copy()
+        res = (_lib.Result * 2)()
+        _lib.check(_lib.lib().locreg_align_loam(self.surf._h, self.edge._h, a.ctypes.data, n_s, b.ctypes.data, n_e, s_s,
+                                                pin.ctypes.data, self.max_iteration, self.eps, pout.ctypes.data, res))
+        self.last_result = (res[0].as_dict(), res[1].as_dict())
+        return pout, self.last_result
+
+    def last_timing(self):
+        return self.surf.last_timing()
+
+    def close(self):
+        self.surf.close()
+        self.edge.close()
+
+
 class NdtRegistration(_Registration):
     """NdtRegistration(NdtOptions) (ndt_registration.cpp:20-28): DIRECT_NDT, or INCREMENTAL_NDT where every
     SetInputTarget ADDS its cloud to an LRU cache of capacity_ voxels (ndt_registration.cpp:150-183)."""
