@@ -140,6 +140,19 @@ int locreg_compute_hb(locreg_handle* h, const float* src, size_t n, size_t strid
 int locreg_align_loam(locreg_handle* surf, locreg_handle* edge, const float* surf_xyz, size_t n_surf, const float* edge_xyz,
                       size_t n_edge, size_t stride_bytes, const double* pose_in, int32_t max_iteration, double eps,
                       double* pose_out, locreg_result* res2);
+/* S independent locreg_align_loam calls against the current surf and edge targets, in one device-resident loop: every
+ * trip evaluates all S scans' surf halves on the surf handle and their edge halves on the edge handle, then one warp
+ * per scan solves.  Scan s is surf points [surf_offsets[s], surf_offsets[s+1]) of surf_xyz and edge points
+ * [edge_offsets[s], edge_offsets[s+1]) of edge_xyz (offsets relative to their cloud pointer; both clouds share one
+ * stride; any half may be empty).  poses_in / poses_out are S*7 doubles; poses_out is always written.  results (may
+ * be NULL) has 2*S entries: [2s] and [2s+1] are scan s's res2 of locreg_align_loam.  Each scan's pose and results are
+ * bit-identical to a locreg_align_loam call on that scan alone; a scan that stops early does not affect the others.
+ * Arguments are checked before any device work (LOCREG_E_ARG: handles as in locreg_align_loam, offsets negative or
+ * decreasing, stride or pointers, S >= 2^31; LOCREG_E_STATE: a handle without a target).  S == 0 does nothing.
+ * locreg_last_timing(surf) reports the call's kernels. */
+int locreg_align_loam_batch(locreg_handle* surf, locreg_handle* edge, const float* surf_xyz, const int64_t* surf_offsets,
+                            const float* edge_xyz, const int64_t* edge_offsets, size_t stride_bytes, const double* poses_in,
+                            size_t S, int32_t max_iteration, double eps, double* poses_out, locreg_result* results);
 
 /* Parity probe for SearchPointInterface::FindNearstPoints (search_point_interface.h:9-24; kdtree.cpp:272-283):
  * exact k-NN (k = 1 or 5) under the total order (float32 dis2, index); idx is nq*k, -1 padded. ICP handles only.

@@ -951,6 +951,15 @@ __device__ __forceinline__ double icp_sum_tiles(const double* __restrict__ parti
     return (v0 + v1) + (v2 + v3);
 }
 
+// Tiles [t0, t1) of item s: from tile_begin (a batch), else tiles_per_item / n_single (one scan, or hypotheses of one).
+__device__ __forceinline__ void item_tiles(const BatchView& bv, unsigned int s, unsigned int& t0, unsigned int& t1) {
+    if (bv.tile_begin) { t0 = bv.tile_begin[s]; t1 = bv.tile_begin[s + 1]; }
+    else {
+        t0 = s * bv.tiles_per_item;
+        t1 = t0 + (bv.n_single + kTile - 1) / kTile;
+    }
+}
+
 // One warp per scan.  mode 1: Gauss-Newton iteration (update the pose; stop on convergence or after
 // max_iteration trips); mode 0: evaluation only (compute_hb, relocalisation's final score pass): record the sums,
 // leave the pose.  acc_out (optional, 32 doubles per scan) receives the raw sums.
@@ -966,11 +975,7 @@ __global__ void __launch_bounds__(128) k_icp_solve(IcpParams prm, BatchView bv, 
     AlignState* st = states + s;
     if (mode == 1 && st->stop) return;
     unsigned int t0, t1;
-    if (bv.tile_begin) { t0 = bv.tile_begin[s]; t1 = bv.tile_begin[s + 1]; }
-    else {
-        t0 = s * bv.tiles_per_item;
-        t1 = t0 + (bv.n_single + kTile - 1) / kTile;
-    }
+    item_tiles(bv, s, t0, t1);
     sums[warp][lane] = icp_sum_tiles(partials, partials_b, t0, t1, lane);
     __syncwarp();
     if (lane == 0) {
@@ -989,30 +994,38 @@ __global__ void __launch_bounds__(128) k_icp_solve(IcpParams prm, BatchView bv, 
     }
 }
 
-// One Gauss-Newton trip of LoamRegistration::ScanMatch (SURVEY.md 3.3): the P2Plane (surf) half's and the P2Line
-// (edge) half's partial rows are summed separately, in k_icp_solve's order, then added; H dx = B is solved and the
-// pose updated as in the ICP loop, but with neither icp_gn_update's min_effective_pts gate (the halves' own flags do
-// not gate the sum) nor P2P's /16.  A singular sum makes no update (outcome 0).  One warp, one state; half[0] / half[1]
-// receive each half's counts and degenerate flag as locreg_compute_hb reports them at the trip's pose.
-__global__ void __launch_bounds__(32) k_loam_solve(AlignState* st, unsigned int tiles_surf, const double* __restrict__ surf,
-                                                   const double* __restrict__ surf_b, int min_eff_surf, unsigned int tiles_edge,
-                                                   const double* __restrict__ edge, const double* __restrict__ edge_b,
-                                                   int min_eff_edge, double eps, int max_iteration, DevResult* half) {
-    __shared__ double sums[3][32];
-    const unsigned int lane = threadIdx.x & 31;
+// One Gauss-Newton trip of LoamRegistration::ScanMatch (SURVEY.md 3.3), one warp per scan: the P2Plane (surf) half's and
+// the P2Line (edge) half's partial rows are summed separately, in k_icp_solve's order, then added; H dx = B is solved and
+// the pose updated as in the ICP loop, but with neither icp_gn_update's min_effective_pts gate (the halves' own flags do
+// not gate the sum) nor P2P's /16.  A singular sum makes no update (outcome 0).  bs / be: the two halves' views of the
+// same S scans (each half's tiles of scan s from its own view); states[s] is scan s's one pose, both halves evaluate at
+// it.  half[2s] / half[2s + 1] receive scan s's surf / edge counts and degenerate flag as locreg_compute_hb reports them
+// at the trip's pose.  A stopped scan's warp exits.
+__global__ void __launch_bounds__(128) k_loam_solve(BatchView bs, const double* __restrict__ surf, const double* __restrict__ surf_b,
+                                                    int min_eff_surf, BatchView be, const double* __restrict__ edge,
+                                                    const double* __restrict__ edge_b, int min_eff_edge, AlignState* states,
+                                                    double eps, int max_iteration, DevResult* half) {
+    __shared__ double sums[4][3][32];
+    const unsigned int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+    const unsigned int s = blockIdx.x * 4 + warp;
+    if (s >= bs.S) return;
+    AlignState* st = states + s;
     if (st->stop) return;
-    const double s = icp_sum_tiles(surf, surf_b, 0, tiles_surf, lane);
-    const double e = icp_sum_tiles(edge, edge_b, 0, tiles_edge, lane);
-    sums[0][lane] = s;
-    sums[1][lane] = e;
-    sums[2][lane] = s + e;
+    unsigned int t0, t1;
+    item_tiles(bs, s, t0, t1);
+    const double a = icp_sum_tiles(surf, surf_b, t0, t1, lane);
+    item_tiles(be, s, t0, t1);
+    const double e = icp_sum_tiles(edge, edge_b, t0, t1, lane);
+    sums[warp][0][lane] = a;
+    sums[warp][1][lane] = e;
+    sums[warp][2][lane] = a + e;
     __syncwarp();
     if (lane < 3) {  // lanes 0 / 1: the halves' own records (their degenerate flags need det of their own H); lane 2: the update
-        const double* acc = sums[lane];
+        const double* acc = sums[warp][lane];
         double dx[6];
         const bool solvable = gn_solve6(acc, acc + 21, dx);
         if (lane < 2) {
-            DevResult& r = half[lane];
+            DevResult& r = half[2 * static_cast<size_t>(s) + lane];
             result_from_acc(r, acc);
             r.degenerate = (!solvable || r.n_effective < (lane == 0 ? min_eff_surf : min_eff_edge)) ? 1 : 0;
         } else {

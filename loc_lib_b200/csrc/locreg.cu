@@ -521,13 +521,14 @@ void icp_run_loop(locreg_handle* h, const IcpJob& job, int final_eval) {
         icp_launch_solve<METHOD>(h, job, 0, nullptr, pb);
     }
 }
-// LoamRegistration::ScanMatch's loop (SURVEY.md 3.3), all trips queued with no host round trip.  Each trip evaluates the
-// surf half (P2Plane) on surf's stream and scratch and the edge half (P2Line) on edge's, both at the one pose in the
-// state both jobs point at, so the two evaluations run side by side; k_loam_solve then joins their partial rows on
-// surf's stream.  loam_ev[0] (surf stream: state uploaded / trip solved) holds the edge half back until the pose it
-// reads is final and the edge partial rows it overwrites have been read; loam_ev[1] (edge stream: edge half evaluated)
-// holds the solve back.  With both handles on one stream the same calls run serially.  An empty half launches nothing
-// and its zero tiles sum to zeros.
+// LoamRegistration::ScanMatch's loop (SURVEY.md 3.3) for the S scans of js / je, all trips queued with no host round
+// trip.  Each trip evaluates the surf halves (P2Plane) on surf's stream and scratch and the edge halves (P2Line) on
+// edge's, each scan's two halves at the one pose in the state both jobs point at, so the two evaluations run side by
+// side; k_loam_solve then joins their partial rows on surf's stream, one warp per scan.  loam_ev[0] (surf stream: states
+// initialised / trip solved) holds the edge half back until the poses it reads are final and the edge partial rows it
+// overwrites have been read; loam_ev[1] (edge stream: edge half evaluated) holds the solve back.  With both handles on
+// one stream the same calls run serially.  An empty half launches nothing and its zero tiles sum to zeros; stopped
+// scans make their tiles and their solve warp exit.
 void loam_run_loop(locreg_handle* surf, locreg_handle* edge, const IcpJob& js, const IcpJob& je, int max_iteration,
                    double eps, DevResult* d_half) {
     LR_CUDA(cudaEventRecord(surf->loam_ev[0], surf->stream));
@@ -539,9 +540,9 @@ void loam_run_loop(locreg_handle* surf, locreg_handle* edge, const IcpJob& js, c
         const double* sb = icp_launch_eval<kIcpP2Plane>(surf, js, 0, nn_mode, nullptr, nullptr);
         LR_CUDA(cudaStreamWaitEvent(surf->stream, surf->loam_ev[1], 0));
         prof_mark(surf, 2, true);
-        LR_LAUNCH(k_loam_solve, 1, 32, 0, surf->stream, js.states, js.n_tiles, surf->d_partials.as<double>(), sb,
-                  surf->opt.min_effective_pts, je.n_tiles, edge->d_partials.as<double>(), eb, edge->opt.min_effective_pts, eps,
-                  max_iteration, d_half);
+        LR_LAUNCH(k_loam_solve, (js.bv.S + 3) / 4, 128, 0, surf->stream, js.bv, surf->d_partials.as<double>(), sb,
+                  surf->opt.min_effective_pts, je.bv, edge->d_partials.as<double>(), eb, edge->opt.min_effective_pts, js.states,
+                  eps, max_iteration, d_half);
         prof_mark(surf, 2, false);
         LR_CUDA(cudaEventRecord(surf->loam_ev[0], surf->stream));
     }
@@ -930,9 +931,7 @@ int locreg_compute_hb(locreg_handle* h, const float* src, size_t n, size_t strid
     });
 }
 
-int locreg_align_loam(locreg_handle* surf, locreg_handle* edge, const float* surf_xyz, size_t n_surf, const float* edge_xyz,
-                      size_t n_edge, size_t stride, const double* pose_in, int32_t max_iteration, double eps, double* pose_out,
-                      locreg_result* res2) {
+static int loam_check_handles(const locreg_handle* surf, const locreg_handle* edge) {
     if (!surf || !edge) { g_last_error = "null handle"; return LOCREG_E_ARG; }
     if (surf == edge) { g_last_error = "locreg_align_loam needs two distinct handles (surf and edge)"; return LOCREG_E_ARG; }
     if (surf->device != edge->device) { g_last_error = "surf and edge handles are on different devices"; return LOCREG_E_ARG; }
@@ -940,47 +939,133 @@ int locreg_align_loam(locreg_handle* surf, locreg_handle* edge, const float* sur
         g_last_error = "locreg_align_loam needs a LOCREG_ICP_P2PLANE surf handle and a LOCREG_ICP_P2LINE edge handle";
         return LOCREG_E_ARG;
     }
-    int rc = check_cloud_args(surf_xyz, n_surf, stride);
+    return LOCREG_OK;
+}
+
+// One half of a LOAM call: offsets (S + 1, host, relative to xyz) of the batch, or nullptr for one scan of n points.
+struct LoamHalf {
+    const float* xyz;
+    const int64_t* offsets;
+    size_t n;
+};
+
+// Offsets of one half of locreg_align_loam_batch: non-negative and non-decreasing, the cloud they cover valid.
+static int loam_check_half(const LoamHalf& c, size_t stride, size_t S, const char* name) {
+    if (!c.offsets) { g_last_error = "null argument"; return LOCREG_E_ARG; }
+    for (size_t s = 0; s < S; ++s)
+        if (c.offsets[s] < 0 || c.offsets[s + 1] < c.offsets[s]) {
+            g_last_error = std::string(name) + " offsets must be non-negative and non-decreasing";
+            return LOCREG_E_ARG;
+        }
+    return check_cloud_args(c.xyz, static_cast<size_t>(c.offsets[S] - c.offsets[0]), stride);
+}
+
+// Stages one half's cloud with one copy on its handle's stream; a batch's offsets go to the device relative to it.
+static const float4* loam_stage_half(locreg_handle* h, const LoamHalf& c, size_t stride, size_t S) {
+    if (!c.offsets) return stage_cloud(h, c.xyz, c.n, stride, false);
+    const size_t base = static_cast<size_t>(c.offsets[0]), n_pts = static_cast<size_t>(c.offsets[S]) - base;
+    h->h_small.reserve((S + 1) * sizeof(long long));
+    long long* rel = h->h_small.as<long long>();
+    for (size_t s = 0; s <= S; ++s) rel[s] = c.offsets[s] - static_cast<long long>(base);
+    h->d_offsets.reserve((S + 1) * sizeof(long long));
+    LR_CUDA(cudaMemcpyAsync(h->d_offsets.p, rel, (S + 1) * sizeof(long long), cudaMemcpyHostToDevice, h->stream));
+    return stage_cloud(h, reinterpret_cast<const float*>(reinterpret_cast<const char*>(c.xyz) + base * stride), n_pts, stride, false);
+}
+
+// One half's job over the S scans (one scan: offsets == nullptr).
+static IcpJob loam_half_job(locreg_handle* h, const LoamHalf& c, const float4* src4, size_t S) {
+    if (!c.offsets) {
+        h->d_state.reserve(sizeof(AlignState));
+        return icp_single_job(h, src4, static_cast<unsigned int>(c.n));
+    }
+    const size_t n_pts = static_cast<size_t>(c.offsets[S] - c.offsets[0]);
+    IcpJob job = icp_batch_job(h, src4, h->d_offsets.as<long long>(), static_cast<unsigned int>(S), n_pts);
+    if (n_pts == 0) job.n_tiles = 0;  // no point in the whole half: its evaluation launches nothing (its tiles would all exit)
+    return job;
+}
+
+// locreg_align_loam (S = 1, no offsets) and locreg_align_loam_batch: S independent LOAM loops in one.  The states live
+// with the surf job (the edge job points at them); surf->d_loam holds the poses, the loop results and the halves'
+// records, copied back in one piece through surf->h_out.
+static int loam_align(locreg_handle* surf, locreg_handle* edge, const LoamHalf& cs, const LoamHalf& ce, size_t stride,
+                      const double* poses_in, size_t S, int32_t max_iteration, double eps, double* poses_out, locreg_result* results) {
+    if (!surf->has_target || !edge->has_target) {
+        g_last_error = surf->has_target ? "SetInputTarget has not been called on the edge handle"
+                                        : "SetInputTarget has not been called on the surf handle";
+        return LOCREG_E_STATE;
+    }
+    for (cudaEvent_t& e : surf->loam_ev)
+        if (!e) LR_CUDA(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
+    const unsigned int Su = static_cast<unsigned int>(S);
+    // d_loam / h_out: [S x 7 poses][S loop results][2S halves]
+    const size_t res_off = S * 7 * sizeof(double), half_off = res_off + S * sizeof(DevResult), bytes = half_off + 2 * S * sizeof(DevResult);
+    surf->d_loam.reserve(bytes);
+    surf->h_out.reserve(bytes);
+    unsigned char* const d = surf->d_loam.as<unsigned char>();
+    unsigned char* const hb = surf->h_out.as<unsigned char>();
+    double* const d_poses = reinterpret_cast<double*>(d);
+    DevResult* const d_res = reinterpret_cast<DevResult*>(d + res_off);
+    DevResult* const d_half = reinterpret_cast<DevResult*>(d + half_off);
+    const float4* src_s = loam_stage_half(surf, cs, stride, S);
+    const float4* src_e = loam_stage_half(edge, ce, stride, S);
+    std::memcpy(hb, poses_in, S * 7 * sizeof(double));
+    LR_CUDA(cudaMemcpyAsync(d_poses, hb, S * 7 * sizeof(double), cudaMemcpyHostToDevice, surf->stream));
+    LR_CUDA(cudaMemsetAsync(d_half, 0, 2 * S * sizeof(DevResult), surf->stream));
+    surf->begin_timing();
+    IcpJob js = loam_half_job(surf, cs, src_s, S);
+    IcpJob je = loam_half_job(edge, ce, src_e, S);
+    je.states = js.states;  // one state, one pose per scan: both halves evaluate at it
+    // CaculateMatrixHAndB ignores zero_initial_translation: so does the LOAM loop
+    LR_LAUNCH(k_states_init, (Su + 255) / 256, 256, 0, surf->stream, d_poses, Su, max_iteration, 0, js.states);
+    loam_run_loop(surf, edge, js, je, max_iteration, eps, d_half);
+    LR_LAUNCH(k_states_export, (Su + 255) / 256, 256, 0, surf->stream, js.states, Su, d_poses, d_res);
+    LR_CUDA(cudaMemcpyAsync(hb, d, bytes, cudaMemcpyDeviceToHost, surf->stream));
+    surf->end_timing();  // synchronises surf's stream, which has joined edge's
+    std::memcpy(poses_out, hb, S * 7 * sizeof(double));
+    const DevResult* hr = reinterpret_cast<const DevResult*>(hb + res_off);
+    const DevResult* hh = reinterpret_cast<const DevResult*>(hb + half_off);
+    for (size_t i = 0; results && i < 2 * S; ++i) {  // the loop's bookkeeping, the half's last evaluation
+        DevResult r = hh[i];
+        const DevResult& loop = hr[i / 2];
+        r.iters = loop.iters;
+        r.updates = loop.updates;
+        r.converged = loop.converged;
+        r.pose_written = loop.pose_written;
+        fill_result(results + i, r);
+    }
+    return LOCREG_OK;
+}
+
+int locreg_align_loam(locreg_handle* surf, locreg_handle* edge, const float* surf_xyz, size_t n_surf, const float* edge_xyz,
+                      size_t n_edge, size_t stride, const double* pose_in, int32_t max_iteration, double eps, double* pose_out,
+                      locreg_result* res2) {
+    int rc = loam_check_handles(surf, edge);
+    if (rc) return rc;
+    rc = check_cloud_args(surf_xyz, n_surf, stride);
     if (rc) return rc;
     rc = check_cloud_args(edge_xyz, n_edge, stride);
     if (rc) return rc;
     if (!pose_in || !pose_out) { g_last_error = "null pose"; return LOCREG_E_ARG; }
     return guarded(surf, [&]() {
-        if (!surf->has_target || !edge->has_target) {
-            g_last_error = surf->has_target ? "SetInputTarget has not been called on the edge handle"
-                                            : "SetInputTarget has not been called on the surf handle";
-            return LOCREG_E_STATE;
-        }
-        for (cudaEvent_t& e : surf->loam_ev)
-            if (!e) LR_CUDA(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
-        const float4* src_s = stage_cloud(surf, surf_xyz, n_surf, stride, false);
-        const float4* src_e = stage_cloud(edge, edge_xyz, n_edge, stride, false);
-        init_state(surf, pose_in);  // CaculateMatrixHAndB ignores zero_initial_translation: so does the LOAM loop
-        surf->d_loam.reserve(2 * sizeof(DevResult));
-        DevResult* d_half = surf->d_loam.as<DevResult>();
-        LR_CUDA(cudaMemsetAsync(d_half, 0, 2 * sizeof(DevResult), surf->stream));
-        surf->begin_timing();
-        const IcpJob js = icp_single_job(surf, src_s, static_cast<unsigned int>(n_surf));
-        IcpJob je = icp_single_job(edge, src_e, static_cast<unsigned int>(n_edge));
-        je.states = js.states;  // one state, one pose: both halves evaluate at it
-        loam_run_loop(surf, edge, js, je, max_iteration, eps, d_half);
-        surf->h_small.reserve(4096);
-        AlignState* hs = surf->h_small.as<AlignState>() + 1;
-        DevResult* hh = reinterpret_cast<DevResult*>(hs + 1);
-        LR_CUDA(cudaMemcpyAsync(hs, js.states, sizeof(AlignState), cudaMemcpyDeviceToHost, surf->stream));
-        LR_CUDA(cudaMemcpyAsync(hh, d_half, 2 * sizeof(DevResult), cudaMemcpyDeviceToHost, surf->stream));
-        surf->end_timing();  // synchronises surf's stream, which has joined edge's
-        std::memcpy(pose_out, hs->pose, 7 * sizeof(double));
-        for (int i = 0; res2 && i < 2; ++i) {  // the loop's bookkeeping, the half's last evaluation
-            DevResult r = hh[i];
-            r.iters = hs->res.iters;
-            r.updates = hs->res.updates;
-            r.converged = hs->res.converged;
-            r.pose_written = hs->res.pose_written;
-            fill_result(res2 + i, r);
-        }
-        return LOCREG_OK;
+        return loam_align(surf, edge, LoamHalf{surf_xyz, nullptr, n_surf}, LoamHalf{edge_xyz, nullptr, n_edge}, stride, pose_in, 1,
+                          max_iteration, eps, pose_out, res2);
     });
+}
+
+int locreg_align_loam_batch(locreg_handle* surf, locreg_handle* edge, const float* surf_xyz, const int64_t* surf_offsets,
+                            const float* edge_xyz, const int64_t* edge_offsets, size_t stride, const double* poses_in, size_t S,
+                            int32_t max_iteration, double eps, double* poses_out, locreg_result* results) {
+    int rc = loam_check_handles(surf, edge);
+    if (rc) return rc;
+    if (S >= (1ull << 31)) { g_last_error = "too many scans"; return LOCREG_E_ARG; }
+    if (S == 0) return LOCREG_OK;
+    const LoamHalf cs{surf_xyz, surf_offsets, 0}, ce{edge_xyz, edge_offsets, 0};
+    rc = loam_check_half(cs, stride, S, "surf");
+    if (rc) return rc;
+    rc = loam_check_half(ce, stride, S, "edge");
+    if (rc) return rc;
+    if (!poses_in || !poses_out) { g_last_error = "null pose"; return LOCREG_E_ARG; }
+    return guarded(surf, [&]() { return loam_align(surf, edge, cs, ce, stride, poses_in, S, max_iteration, eps, poses_out, results); });
 }
 
 int locreg_knn(locreg_handle* h, const float* queries, size_t nq, size_t stride, int32_t k, int32_t* idx) {

@@ -373,10 +373,7 @@ class LoamRegistration:
     def ScanMatch(self, surf_cloud, edge_cloud, predict_pose):
         """Returns (pose, (res_surf, res_edge)): iters / updates / converged are the loop's, the counts and the degenerate
         flag each half's last evaluation."""
-        a, n_s, s_s = _cloud(surf_cloud)
-        b, n_e, s_e = _cloud(edge_cloud)
-        if s_e != s_s:  # the C ABI takes one stride for both clouds
-            b = np.ascontiguousarray(np.pad(b[:, :3], ((0, 0), (0, s_s // 4 - 3))), np.float32)
+        a, n_s, s_s, b, n_e = self._clouds(surf_cloud, edge_cloud)
         pin = _pose(predict_pose)
         pout = pin.copy()
         res = (_lib.Result * 2)()
@@ -384,6 +381,32 @@ class LoamRegistration:
                                                 pin.ctypes.data, self.max_iteration, self.eps, pout.ctypes.data, res))
         self.last_result = (res[0].as_dict(), res[1].as_dict())
         return pout, self.last_result
+
+    def ScanMatchBatch(self, surf_clouds, surf_offsets, edge_clouds, edge_offsets, predict_poses):
+        """S independent ScanMatch calls in one device-resident loop (locreg_align_loam_batch).  Scan s is
+        surf_clouds[surf_offsets[s]:surf_offsets[s + 1]] and edge_clouds[edge_offsets[s]:edge_offsets[s + 1]].
+        Returns (poses (S, 7), [(res_surf, res_edge)] * S), each scan's exactly what its ScanMatch call returns."""
+        a, _, s_s, b, _ = self._clouds(surf_clouds, edge_clouds)
+        so = np.ascontiguousarray(surf_offsets, np.int64)
+        eo = np.ascontiguousarray(edge_offsets, np.int64)
+        S = so.shape[0] - 1
+        if S < 0 or eo.shape != so.shape:
+            raise _lib.LocregError("surf_offsets and edge_offsets need S + 1 entries each")
+        pin = np.ascontiguousarray(predict_poses, np.float64).reshape(S, 7)
+        pout = pin.copy()
+        res = (_lib.Result * (2 * S))()
+        _lib.check(_lib.lib().locreg_align_loam_batch(self.surf._h, self.edge._h, a.ctypes.data, so.ctypes.data, b.ctypes.data,
+                                                      eo.ctypes.data, s_s, pin.ctypes.data, S, self.max_iteration, self.eps,
+                                                      pout.ctypes.data, res))
+        return pout, [(res[2 * s].as_dict(), res[2 * s + 1].as_dict()) for s in range(S)]
+
+    @staticmethod
+    def _clouds(surf_cloud, edge_cloud):
+        a, n_s, s_s = _cloud(surf_cloud)
+        b, n_e, s_e = _cloud(edge_cloud)
+        if s_e != s_s:  # the C ABI takes one stride for both clouds
+            b = np.ascontiguousarray(np.pad(b[:, :3], ((0, 0), (0, s_s // 4 - 3))), np.float32)
+        return a, n_s, s_s, b, n_e
 
     def last_timing(self):
         return self.surf.last_timing()
