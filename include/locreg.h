@@ -216,6 +216,35 @@ int locreg_shard_range(size_t n, int32_t rank, int32_t world, size_t* lo, size_t
 int locreg_relocalise_sharded(locreg_handle* h, const float* src, size_t n, size_t stride_bytes, const double* poses_in,
                               size_t n_hyp, double* best_pose, int64_t* best_idx, double* best_score);
 
+/* LOAM global relocalisation: n_hyp locreg_align_loam calls of ONE surf / edge scan from different initial poses, in
+ * one device-resident loop (hypotheses run in waves that bound the per-point scratch; the waves do not change results).
+ *   loop     hypothesis i runs the LOAM loop of locreg_align_loam from poses_in[i] (7 doubles) as given, with the same
+ *            max_iteration / eps, the same singular-H rule and each half's own gates; zero_initial_translation does
+ *            not apply.
+ *   score    after the loop both halves are evaluated once more at the final pose; score = (sum_sq_res_surf +
+ *            sum_sq_res_edge) / (n_inlier_surf + n_inlier_edge) from that pass: the plain sum of what the two halves
+ *            report, unweighted.  +inf when det(H_surf + H_edge) == 0 there or neither half has an inlier; the halves'
+ *            own degenerate flags do not gate it.
+ *   best     the argmin of locreg_pack_score(score, index), lowest index winning ties; index 0 when every score is
+ *            +inf.  best_pose is poses_out[best] bit for bit.
+ * scores (n_hyp) and poses_out (n_hyp * 7) may be NULL.  Clouds share one stride; either may be empty (that half
+ * contributes zeros).  locreg_last_timing(surf) reports the call's kernels.  Arguments are checked before any device
+ * work: LOCREG_E_ARG for the handles as in locreg_align_loam, bad cloud arguments, a null poses_in, n_hyp == 0 or
+ * n_hyp >= 2^31; LOCREG_E_STATE for a handle without a target. */
+int locreg_relocalise_loam(locreg_handle* surf, locreg_handle* edge, const float* surf_xyz, size_t n_surf,
+                           const float* edge_xyz, size_t n_edge, size_t stride_bytes, const double* poses_in, size_t n_hyp,
+                           int32_t max_iteration, double eps, double* best_pose, int64_t* best_idx, double* best_score,
+                           double* scores, double* poses_out);
+/* locreg_relocalise_loam over all ranks of the SURF handle's communicator (the edge handle's is not used; none: world
+ * = 1).  Every rank passes the same clouds and all n_hyp hypotheses and registers hypotheses rank, rank + world, ...;
+ * then, on surf's stream, one ncclAllReduce(MIN) of the packed key and the owner's ncclBroadcast of pose + score, as in
+ * locreg_relocalise_sharded.  best_* are identical on every rank.  locreg_last_timing(surf) covers the kernels and the
+ * collectives.  Argument errors as in locreg_relocalise_loam. */
+int locreg_relocalise_loam_sharded(locreg_handle* surf, locreg_handle* edge, const float* surf_xyz, size_t n_surf,
+                                   const float* edge_xyz, size_t n_edge, size_t stride_bytes, const double* poses_in,
+                                   size_t n_hyp, int32_t max_iteration, double eps, double* best_pose, int64_t* best_idx,
+                                   double* best_score);
+
 /* Batch offline mapping over all ranks (BASELINE config 4).  The batch has S_global scans; this rank owns the block
  * [lo, hi) = locreg_shard_range(S_global, rank, world) and passes ONLY that block: srcs / offsets (S_local + 1
  * entries, relative to srcs) / poses_in (S_local * 7) with S_local = hi - lo.  No collective on the data path; at the

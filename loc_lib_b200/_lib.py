@@ -21,7 +21,7 @@ SYMBOLS = [
     "locreg_local_map_add_keyframe", "locreg_local_map_get", "locreg_local_map_clear",
     "locreg_comm_unique_id", "locreg_comm_init", "locreg_comm_destroy", "locreg_comm_info", "locreg_shard_range",
     "locreg_relocalise_sharded", "locreg_align_batch_sharded", "locreg_index_info", "locreg_align_loam",
-    "locreg_align_loam_batch",
+    "locreg_align_loam_batch", "locreg_relocalise_loam", "locreg_relocalise_loam_sharded",
 ]
 
 
@@ -64,6 +64,8 @@ def lib():
         L.locreg_compute_hb.argtypes = [vp, vp, sz, sz, vp, vp, vp, C.POINTER(Result)]
         L.locreg_align_loam.argtypes = [vp, vp, vp, sz, vp, sz, sz, vp, i32, C.c_double, vp, vp]
         L.locreg_align_loam_batch.argtypes = [vp, vp, vp, vp, vp, vp, sz, vp, sz, i32, C.c_double, vp, vp]
+        L.locreg_relocalise_loam.argtypes = [vp, vp, vp, sz, vp, sz, sz, vp, sz, i32, C.c_double, vp, vp, vp, vp, vp]
+        L.locreg_relocalise_loam_sharded.argtypes = [vp, vp, vp, sz, vp, sz, sz, vp, sz, i32, C.c_double, vp, vp, vp]
         L.locreg_knn.argtypes = [vp, vp, sz, sz, i32, vp]
         L.locreg_debug_points.argtypes = [vp, vp, sz, sz, vp, vp, vp]
         L.locreg_align_batch.argtypes = [vp, vp, vp, sz, vp, sz, vp, vp]

@@ -1000,17 +1000,19 @@ __global__ void __launch_bounds__(128) k_icp_solve(IcpParams prm, BatchView bv, 
 // not gate the sum) nor P2P's /16.  A singular sum makes no update (outcome 0).  bs / be: the two halves' views of the
 // same S scans (each half's tiles of scan s from its own view); states[s] is scan s's one pose, both halves evaluate at
 // it.  half[2s] / half[2s + 1] receive scan s's surf / edge counts and degenerate flag as locreg_compute_hb reports them
-// at the trip's pose.  A stopped scan's warp exits.
+// at the trip's pose.  mode 1: the trip; a stopped scan's warp exits.  mode 0: evaluation only (LOAM relocalisation's
+// score pass), for every scan: st->res receives the summed counts and sum of squares and degenerate = singular sum; the
+// pose, iters, updates and converged stay as they are.
 __global__ void __launch_bounds__(128) k_loam_solve(BatchView bs, const double* __restrict__ surf, const double* __restrict__ surf_b,
                                                     int min_eff_surf, BatchView be, const double* __restrict__ edge,
                                                     const double* __restrict__ edge_b, int min_eff_edge, AlignState* states,
-                                                    double eps, int max_iteration, DevResult* half) {
+                                                    double eps, int max_iteration, int mode, DevResult* half) {
     __shared__ double sums[4][3][32];
     const unsigned int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     const unsigned int s = blockIdx.x * 4 + warp;
     if (s >= bs.S) return;
     AlignState* st = states + s;
-    if (st->stop) return;
+    if (mode == 1 && st->stop) return;
     unsigned int t0, t1;
     item_tiles(bs, s, t0, t1);
     const double a = icp_sum_tiles(surf, surf_b, t0, t1, lane);
@@ -1028,6 +1030,9 @@ __global__ void __launch_bounds__(128) k_loam_solve(BatchView bs, const double* 
             DevResult& r = half[2 * static_cast<size_t>(s) + lane];
             result_from_acc(r, acc);
             r.degenerate = (!solvable || r.n_effective < (lane == 0 ? min_eff_surf : min_eff_edge)) ? 1 : 0;
+        } else if (mode == 0) {
+            result_from_acc(st->res, acc);
+            st->res.degenerate = solvable ? 0 : 1;
         } else {
             result_from_acc(st->res, acc);
             Pose T;

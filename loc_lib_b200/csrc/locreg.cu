@@ -528,24 +528,27 @@ void icp_run_loop(locreg_handle* h, const IcpJob& job, int final_eval) {
 // initialised / trip solved) holds the edge half back until the poses it reads are final and the edge partial rows it
 // overwrites have been read; loam_ev[1] (edge stream: edge half evaluated) holds the solve back.  With both handles on
 // one stream the same calls run serially.  An empty half launches nothing and its zero tiles sum to zeros; stopped
-// scans make their tiles and their solve warp exit.
+// scans make their tiles and their solve warp exit.  final_eval: after the trips, both halves are evaluated once more at
+// every scan's final pose, stopped or not, and an evaluation-only k_loam_solve (mode 0) records the summed sums in the
+// states (LOAM relocalisation's score pass, as icp_run_loop's).
 void loam_run_loop(locreg_handle* surf, locreg_handle* edge, const IcpJob& js, const IcpJob& je, int max_iteration,
-                   double eps, DevResult* d_half) {
-    LR_CUDA(cudaEventRecord(surf->loam_ev[0], surf->stream));
-    for (int it = 0; it < max_iteration; ++it) {
-        const int nn_mode = icp_loop_nn_mode(it);
+                   double eps, DevResult* d_half, int final_eval = 0) {
+    const auto trip = [&](int ignore_stop, int nn_mode, int mode) {
         LR_CUDA(cudaStreamWaitEvent(edge->stream, surf->loam_ev[0], 0));
-        const double* eb = icp_launch_eval<kIcpP2Line>(edge, je, 0, nn_mode, nullptr, nullptr);
+        const double* eb = icp_launch_eval<kIcpP2Line>(edge, je, ignore_stop, nn_mode, nullptr, nullptr);
         LR_CUDA(cudaEventRecord(surf->loam_ev[1], edge->stream));
-        const double* sb = icp_launch_eval<kIcpP2Plane>(surf, js, 0, nn_mode, nullptr, nullptr);
+        const double* sb = icp_launch_eval<kIcpP2Plane>(surf, js, ignore_stop, nn_mode, nullptr, nullptr);
         LR_CUDA(cudaStreamWaitEvent(surf->stream, surf->loam_ev[1], 0));
         prof_mark(surf, 2, true);
         LR_LAUNCH(k_loam_solve, (js.bv.S + 3) / 4, 128, 0, surf->stream, js.bv, surf->d_partials.as<double>(), sb,
                   surf->opt.min_effective_pts, je.bv, edge->d_partials.as<double>(), eb, edge->opt.min_effective_pts, js.states,
-                  eps, max_iteration, d_half);
+                  eps, max_iteration, mode, d_half);
         prof_mark(surf, 2, false);
         LR_CUDA(cudaEventRecord(surf->loam_ev[0], surf->stream));
-    }
+    };
+    LR_CUDA(cudaEventRecord(surf->loam_ev[0], surf->stream));
+    for (int it = 0; it < max_iteration; ++it) trip(0, icp_loop_nn_mode(it), 1);
+    if (final_eval) trip(1, max_iteration > 0 ? kNnSeeds : kNnTwoPass, 0);
     // join: whatever the edge stream still has (its cloud copy when no trip ran) is done before surf's stream goes on
     LR_CUDA(cudaEventRecord(surf->loam_ev[1], edge->stream));
     LR_CUDA(cudaStreamWaitEvent(surf->stream, surf->loam_ev[1], 0));
@@ -987,8 +990,7 @@ static IcpJob loam_half_job(locreg_handle* h, const LoamHalf& c, const float4* s
 // locreg_align_loam (S = 1, no offsets) and locreg_align_loam_batch: S independent LOAM loops in one.  The states live
 // with the surf job (the edge job points at them); surf->d_loam holds the poses, the loop results and the halves'
 // records, copied back in one piece through surf->h_out.
-static int loam_align(locreg_handle* surf, locreg_handle* edge, const LoamHalf& cs, const LoamHalf& ce, size_t stride,
-                      const double* poses_in, size_t S, int32_t max_iteration, double eps, double* poses_out, locreg_result* results) {
+static int loam_prepare(locreg_handle* surf, const locreg_handle* edge) {
     if (!surf->has_target || !edge->has_target) {
         g_last_error = surf->has_target ? "SetInputTarget has not been called on the edge handle"
                                         : "SetInputTarget has not been called on the surf handle";
@@ -996,6 +998,13 @@ static int loam_align(locreg_handle* surf, locreg_handle* edge, const LoamHalf& 
     }
     for (cudaEvent_t& e : surf->loam_ev)
         if (!e) LR_CUDA(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
+    return LOCREG_OK;
+}
+
+static int loam_align(locreg_handle* surf, locreg_handle* edge, const LoamHalf& cs, const LoamHalf& ce, size_t stride,
+                      const double* poses_in, size_t S, int32_t max_iteration, double eps, double* poses_out, locreg_result* results) {
+    const int rc = loam_prepare(surf, edge);
+    if (rc) return rc;
     const unsigned int Su = static_cast<unsigned int>(S);
     // d_loam / h_out: [S x 7 poses][S loop results][2S halves]
     const size_t res_off = S * 7 * sizeof(double), half_off = res_off + S * sizeof(DevResult), bytes = half_off + 2 * S * sizeof(DevResult);
@@ -1415,6 +1424,39 @@ uint64_t locreg_pack_score(double score, uint32_t index) {
     return (static_cast<uint64_t>(bits) << 32) | index;
 }
 
+// Hypotheses per wave of a relocalisation of n_hyp hypotheses.  Hypotheses run in waves so that the per-point neighbour
+// scratch (K rows per point) stays bounded; the rest of the per-point scratch - planes, margins, queues - scales with it
+// (~4.5 GiB in all for P2Plane at 1 GiB of neighbours).  n_mem: points registered per hypothesis, over every job of the
+// wave (sizes the memory); n_rows: points of the largest one job (its scratch rows are 32-bit).
+static size_t reloc_wave_size(size_t n_hyp, size_t n_mem, size_t n_rows, int K) {
+    const size_t per_hyp = std::max<size_t>(n_mem, 1) * K * sizeof(unsigned int);
+    // LOCREG_RELOC_WAVE_GIB: neighbour scratch per wave in GiB.  Default 4 (7857 hypotheses of a 27 k-point scan, ~20 GB
+    // of scratch in all; measured on 8192 hypotheses: 1.82 s at 1 GiB, 1.75 s at 2, 1.69 s at 4 - larger waves fill the
+    // bins of the spatially ordered stage-2 queue better), never more than a third of the free device memory
+    static const double wave_gib = getenv("LOCREG_RELOC_WAVE_GIB") ? std::min(16.0, std::max(1e-5, atof(getenv("LOCREG_RELOC_WAVE_GIB")))) : 4.0;
+    size_t free_b = 0, total_b = 0;
+    LR_CUDA(cudaMemGetInfo(&free_b, &total_b));
+    const size_t per_hyp_all = std::max<size_t>(n_mem, 1) * (K * sizeof(unsigned int) + 80);  // + planes, margins, queues, flags
+    size_t wave = std::max<size_t>(1, std::min<size_t>(n_hyp, static_cast<size_t>(wave_gib * static_cast<double>(size_t(1) << 30)) / per_hyp));
+    wave = std::max<size_t>(1, std::min<size_t>(wave, free_b / 3 / per_hyp_all));
+    wave = std::min<size_t>(wave, (size_t(1) << 32) / std::max<size_t>(n_rows, 1) - 1);  // scratch rows are 32-bit
+    return wave;
+}
+
+// W hypotheses of ONE cloud of n points as one job: BatchView.offsets == nullptr, every item registers the whole cloud
+// and owns tiles [i * tiles_per_item, ...).  An empty cloud launches nothing (its items sum zero tiles).
+static IcpJob hypothesis_job(const float4* src4, size_t n, unsigned int W, AlignState* states) {
+    IcpJob job;
+    job.bv.src = src4; job.bv.offsets = nullptr; job.bv.tile_begin = nullptr; job.bv.tiles = nullptr;
+    job.bv.n_single = static_cast<unsigned int>(n);
+    job.bv.tiles_per_item = std::max<unsigned int>(1u, (static_cast<unsigned int>(n) + kTile - 1) / kTile);
+    job.bv.S = W;
+    job.states = states;
+    job.n_tiles = static_cast<unsigned int>(n ? static_cast<size_t>(job.bv.tiles_per_item) * W : 0);
+    job.n_scratch_points = static_cast<size_t>(n) * W;
+    return job;
+}
+
 // n_local hypotheses (host, 7 doubles each) of ONE scan -> h->d_poses_out / d_results / d_scores and the packed best key
 // in device memory (returned pointer); the index in the key is index_base + i * index_stride.  Everything is queued on
 // the handle's stream; nothing is synchronised.
@@ -1437,31 +1479,12 @@ static unsigned long long* relocalise_core(locreg_handle* h, const float4* src4,
         NDT_DISPATCH(h, ndt_run_batch(h, PB, src4, nullptr, h->d_poses_in.as<double>(), h->d_poses_out.as<double>(),
                                       h->d_results.as<DevResult>(), static_cast<unsigned int>(n_local), static_cast<unsigned int>(n), 1));
     } else if (n_local) {
-        // hypotheses run in waves so that the per-point neighbour scratch stays below ~1 GiB (the rest of the per-point
-        // scratch - planes, margins, queues - scales with it: ~4.5 GiB in all for P2Plane)
         const int K = h->opt.method == LOCREG_ICP_P2P ? 1 : 5;
-        const size_t per_hyp = std::max<size_t>(n, 1) * K * sizeof(unsigned int);
-        // LOCREG_RELOC_WAVE_GIB: neighbour scratch per wave in GiB.  Default 4 (7857 hypotheses of a 27 k-point scan, ~20 GB
-        // of scratch in all; measured on 8192 hypotheses: 1.82 s at 1 GiB, 1.75 s at 2, 1.69 s at 4 - larger waves fill the
-        // bins of the spatially ordered stage-2 queue better), never more than a third of the free device memory
-        static const double wave_gib = getenv("LOCREG_RELOC_WAVE_GIB") ? std::min(16.0, std::max(1e-5, atof(getenv("LOCREG_RELOC_WAVE_GIB")))) : 4.0;
-        size_t free_b = 0, total_b = 0;
-        LR_CUDA(cudaMemGetInfo(&free_b, &total_b));
-        const size_t per_hyp_all = std::max<size_t>(n, 1) * (K * sizeof(unsigned int) + 80);  // + planes, margins, queues, flags
-        size_t wave = std::max<size_t>(1, std::min<size_t>(n_local, static_cast<size_t>(wave_gib * static_cast<double>(size_t(1) << 30)) / per_hyp));
-        wave = std::max<size_t>(1, std::min<size_t>(wave, free_b / 3 / per_hyp_all));
-        wave = std::min<size_t>(wave, (size_t(1) << 32) / std::max<size_t>(n, 1) - 1);  // scratch rows are 32-bit
+        const size_t wave = reloc_wave_size(n_local, n, n, K);
         h->d_states.reserve(wave * sizeof(AlignState));
         for (size_t w0 = 0; w0 < n_local; w0 += wave) {
             const unsigned int W = static_cast<unsigned int>(std::min(wave, n_local - w0));
-            IcpJob job;
-            job.bv.src = src4; job.bv.offsets = nullptr; job.bv.tile_begin = nullptr; job.bv.tiles = nullptr;
-            job.bv.n_single = static_cast<unsigned int>(n);
-            job.bv.tiles_per_item = std::max<unsigned int>(1u, (static_cast<unsigned int>(n) + kTile - 1) / kTile);
-            job.bv.S = W;
-            job.states = h->d_states.as<AlignState>();
-            job.n_tiles = static_cast<unsigned int>(n ? static_cast<size_t>(job.bv.tiles_per_item) * W : 0);
-            job.n_scratch_points = static_cast<size_t>(n) * W;
+            const IcpJob job = hypothesis_job(src4, n, W, h->d_states.as<AlignState>());
             LR_LAUNCH(k_states_init, (W + 255) / 256, 256, 0, h->stream, h->d_poses_in.as<double>() + w0 * 7, W, h->opt.max_iteration, h->opt.zero_initial_translation, job.states);
             ICP_DISPATCH(h, icp_run_loop<M>(h, job, 1));
             LR_LAUNCH(k_states_export, (W + 255) / 256, 256, 0, h->stream, job.states, W, h->d_poses_out.as<double>() + w0 * 7,
@@ -1558,6 +1581,61 @@ int locreg_comm_info(locreg_handle* h, int32_t* rank, int32_t* world, int32_t* n
     return LOCREG_OK;
 }
 
+}  // extern "C"
+
+// The sharded relocalisations' deal and exchange, on h's stream and communicator (none: a world of one).  Every rank holds
+// all n_hyp hypotheses and registers its share of the strided deal, hypotheses rank, rank + world, ...:
+// run(mine, n_local, rank, world) queues that (mine: host) and returns the device key of its best, with the poses and
+// scores in h->d_poses_out / d_scores.  Then one MIN all-reduce over the packed (score, global index) keys and the
+// winner's owner broadcasts pose + score; best_* come back identical on every rank.  The caller's clouds are staged
+// before: the deal reuses h->h_in once h's stream has drained.
+template <class Run>
+static void relocalise_exchange(locreg_handle* h, const double* poses_in, size_t n_hyp, double* best_pose, int64_t* best_idx,
+                                double* best_score, Run&& run) {
+    const unsigned int rank = static_cast<unsigned int>(h->comm_rank), world = static_cast<unsigned int>(h->comm_world);
+    const size_t n_local = n_hyp > rank ? (n_hyp - rank + world - 1) / world : 0;
+    LR_CUDA(cudaStreamSynchronize(h->stream));  // stage_cloud's copy out of h_in has finished: the buffer can be reused
+    h->h_in.reserve(std::max<size_t>(n_local, 1) * 7 * sizeof(double));
+    double* mine = h->h_in.as<double>();
+    for (size_t i = 0; i < n_local; ++i) std::memcpy(mine + i * 7, poses_in + (rank + i * world) * 7, 7 * sizeof(double));
+    unsigned long long* d_key = run(static_cast<const double*>(mine), n_local, rank, world);
+    // the one exchange step, on the same stream: MIN over the packed (score, global index) keys, then the winner's
+    // owner broadcasts pose + score
+    h->d_bcast.reserve(16 * sizeof(double));
+    double* d_b = h->d_bcast.as<double>();
+    unsigned long long* d_gkey = reinterpret_cast<unsigned long long*>(d_b + 8);
+    const NcclApi& nc = nccl_api();
+    {
+        NvtxRange r("locreg:relocalise:allreduce_min");
+        if (h->comm) LR_NCCL(nc.AllReduce(d_key, d_gkey, 1, ncclUint64, ncclMin, h->comm, h->stream));
+        else LR_CUDA(cudaMemcpyAsync(d_gkey, d_key, sizeof(unsigned long long), cudaMemcpyDeviceToDevice, h->stream));
+    }
+    h->h_small.reserve(4096);
+    unsigned long long* h_key = reinterpret_cast<unsigned long long*>(h->h_small.as<unsigned char>() + 2048);
+    LR_CUDA(cudaMemcpyAsync(h_key, d_gkey, sizeof(unsigned long long), cudaMemcpyDeviceToHost, h->stream));
+    LR_CUDA(cudaStreamSynchronize(h->stream));  // the owner of the winner is a host decision (the root of the broadcast)
+    const uint32_t gi = static_cast<uint32_t>(*h_key & 0xFFFFFFFFull);
+    const bool none = gi == 0xFFFFFFFFu;  // no rank had a hypothesis
+    const unsigned int owner = none ? 0u : gi % world;
+    if (owner == rank && !none) {
+        const size_t li = (gi - rank) / world;
+        LR_CUDA(cudaMemcpyAsync(d_b, h->d_poses_out.as<double>() + li * 7, 7 * sizeof(double), cudaMemcpyDeviceToDevice, h->stream));
+        LR_CUDA(cudaMemcpyAsync(d_b + 7, h->d_scores.as<double>() + li, sizeof(double), cudaMemcpyDeviceToDevice, h->stream));
+    }
+    if (h->comm) {
+        NvtxRange r("locreg:relocalise:broadcast_pose");
+        LR_NCCL(nc.Broadcast(d_b, d_b, 8, ncclDouble, static_cast<int>(owner), h->comm, h->stream));
+    }
+    double* h_b = h->h_small.as<double>() + 128;
+    LR_CUDA(cudaMemcpyAsync(h_b, d_b, 8 * sizeof(double), cudaMemcpyDeviceToHost, h->stream));
+    h->end_timing();  // synchronises the stream: kernels + both collectives
+    if (best_idx) *best_idx = none ? -1 : static_cast<int64_t>(gi);
+    if (best_pose && !none) std::memcpy(best_pose, h_b, 7 * sizeof(double));
+    if (best_score) *best_score = none ? INFINITY : h_b[7];
+}
+
+extern "C" {
+
 int locreg_relocalise_sharded(locreg_handle* h, const float* src, size_t n, size_t stride, const double* poses_in, size_t n_hyp,
                               double* best_pose, int64_t* best_idx, double* best_score) {
     const int rc = check_cloud_args(src, n, stride);
@@ -1565,48 +1643,116 @@ int locreg_relocalise_sharded(locreg_handle* h, const float* src, size_t n, size
     if (!poses_in || n_hyp == 0 || n_hyp >= (1ull << 31)) { g_last_error = "invalid hypotheses"; return LOCREG_E_ARG; }
     return guarded(h, [&]() {
         if (!h->has_target) { g_last_error = "SetInputTarget has not been called"; return LOCREG_E_STATE; }
-        const unsigned int rank = static_cast<unsigned int>(h->comm_rank), world = static_cast<unsigned int>(h->comm_world);
         const float4* src4 = stage_cloud(h, src, n, stride, false);
-        // this rank's share of the strided deal: hypotheses rank, rank + world, ...
-        const size_t n_local = n_hyp > rank ? (n_hyp - rank + world - 1) / world : 0;
-        LR_CUDA(cudaStreamSynchronize(h->stream));  // stage_cloud's copy out of h_in has finished: the buffer can be reused
-        h->h_in.reserve(std::max<size_t>(n_local, 1) * 7 * sizeof(double));
-        double* mine = h->h_in.as<double>();
-        for (size_t i = 0; i < n_local; ++i) std::memcpy(mine + i * 7, poses_in + (rank + i * world) * 7, 7 * sizeof(double));
-        unsigned long long* d_key = relocalise_core(h, src4, n, mine, n_local, rank, world);
-        // the one exchange step, on the same stream: MIN over the packed (score, global index) keys, then the winner's
-        // owner broadcasts pose + score
-        h->d_bcast.reserve(16 * sizeof(double));
-        double* d_b = h->d_bcast.as<double>();
-        unsigned long long* d_gkey = reinterpret_cast<unsigned long long*>(d_b + 8);
-        const NcclApi& nc = nccl_api();
-        {
-            NvtxRange r("locreg:relocalise:allreduce_min");
-            if (h->comm) LR_NCCL(nc.AllReduce(d_key, d_gkey, 1, ncclUint64, ncclMin, h->comm, h->stream));
-            else LR_CUDA(cudaMemcpyAsync(d_gkey, d_key, sizeof(unsigned long long), cudaMemcpyDeviceToDevice, h->stream));
+        relocalise_exchange(h, poses_in, n_hyp, best_pose, best_idx, best_score,
+                            [&](const double* mine, size_t n_local, unsigned int rank, unsigned int world) {
+                                return relocalise_core(h, src4, n, mine, n_local, rank, world);
+                            });
+        return LOCREG_OK;
+    });
+}
+
+// LOAM relocalisation: n_local hypotheses (host, 7 doubles each) of ONE surf / edge scan.  Each runs the LOAM loop of
+// locreg_align_loam from its pose; then the score pass evaluates both halves once more at the final pose and an
+// evaluation-only k_loam_solve leaves the summed counts in the loop's result, from which k_score_argmin takes
+// (sum_sq_surf + sum_sq_edge) / (n_inlier_surf + n_inlier_edge), +inf for a singular summed H or no inlier.  Poses,
+// results and scores land in surf's d_poses_out / d_results / d_scores; returns the device key of the best (index
+// index_base + i * index_stride).  Queued on surf's stream, which joins edge's; nothing is synchronised.  One wave size
+// serves both halves: its memory is sized by n_s + n_e points per hypothesis, its 32-bit scratch rows by the larger half.
+static unsigned long long* loam_relocalise_core(locreg_handle* surf, locreg_handle* edge, const float4* src_s, size_t n_s,
+                                                const float4* src_e, size_t n_e, const double* poses_in, size_t n_local,
+                                                int32_t max_iteration, double eps, unsigned int index_base, unsigned int index_stride) {
+    NvtxRange r("locreg:relocalise_loam");
+    const size_t cap = std::max<size_t>(n_local, 1);
+    surf->d_poses_in.reserve(cap * 7 * sizeof(double));
+    surf->d_poses_out.reserve(cap * 7 * sizeof(double));
+    surf->d_results.reserve(cap * sizeof(DevResult));
+    surf->d_scores.reserve(cap * sizeof(double));
+    surf->d_misc.reserve(64);
+    unsigned long long* d_key = reinterpret_cast<unsigned long long*>(surf->d_misc.as<unsigned char>() + 32);
+    if (n_local) LR_CUDA(cudaMemcpyAsync(surf->d_poses_in.p, poses_in, n_local * 7 * sizeof(double), cudaMemcpyHostToDevice, surf->stream));
+    surf->begin_timing();
+    if (n_local) {
+        const size_t wave = reloc_wave_size(n_local, n_s + n_e, std::max(n_s, n_e), 5);
+        surf->d_states.reserve(wave * sizeof(AlignState));
+        surf->d_loam.reserve(2 * wave * sizeof(DevResult));  // the halves' own records, which k_loam_solve writes
+        for (size_t w0 = 0; w0 < n_local; w0 += wave) {
+            const unsigned int W = static_cast<unsigned int>(std::min(wave, n_local - w0));
+            const IcpJob js = hypothesis_job(src_s, n_s, W, surf->d_states.as<AlignState>());
+            const IcpJob je = hypothesis_job(src_e, n_e, W, js.states);  // one state, one pose per hypothesis
+            // the pose as given: the LOAM loop ignores zero_initial_translation
+            LR_LAUNCH(k_states_init, (W + 255) / 256, 256, 0, surf->stream, surf->d_poses_in.as<double>() + w0 * 7, W, max_iteration, 0, js.states);
+            loam_run_loop(surf, edge, js, je, max_iteration, eps, surf->d_loam.as<DevResult>(), 1);
+            LR_LAUNCH(k_states_export, (W + 255) / 256, 256, 0, surf->stream, js.states, W, surf->d_poses_out.as<double>() + w0 * 7,
+                      surf->d_results.as<DevResult>() + w0);
         }
-        h->h_small.reserve(4096);
-        unsigned long long* h_key = reinterpret_cast<unsigned long long*>(h->h_small.as<unsigned char>() + 2048);
-        LR_CUDA(cudaMemcpyAsync(h_key, d_gkey, sizeof(unsigned long long), cudaMemcpyDeviceToHost, h->stream));
-        LR_CUDA(cudaStreamSynchronize(h->stream));  // the owner of the winner is a host decision (the root of the broadcast)
-        const uint32_t gi = static_cast<uint32_t>(*h_key & 0xFFFFFFFFull);
-        const bool none = gi == 0xFFFFFFFFu;  // no rank had a hypothesis
-        const unsigned int owner = none ? 0u : gi % world;
-        if (owner == rank && !none) {
-            const size_t li = (gi - rank) / world;
-            LR_CUDA(cudaMemcpyAsync(d_b, h->d_poses_out.as<double>() + li * 7, 7 * sizeof(double), cudaMemcpyDeviceToDevice, h->stream));
-            LR_CUDA(cudaMemcpyAsync(d_b + 7, h->d_scores.as<double>() + li, sizeof(double), cudaMemcpyDeviceToDevice, h->stream));
-        }
-        if (h->comm) {
-            NvtxRange r("locreg:relocalise:broadcast_pose");
-            LR_NCCL(nc.Broadcast(d_b, d_b, 8, ncclDouble, static_cast<int>(owner), h->comm, h->stream));
-        }
-        double* h_b = h->h_small.as<double>() + 128;
-        LR_CUDA(cudaMemcpyAsync(h_b, d_b, 8 * sizeof(double), cudaMemcpyDeviceToHost, h->stream));
-        h->end_timing();  // synchronises the stream: kernels + both collectives
-        if (best_idx) *best_idx = none ? -1 : static_cast<int64_t>(gi);
-        if (best_pose && !none) std::memcpy(best_pose, h_b, 7 * sizeof(double));
-        if (best_score) *best_score = none ? INFINITY : h_b[7];
+    } else {  // no hypothesis on this rank: edge's cloud copy still joins surf's stream
+        LR_CUDA(cudaEventRecord(surf->loam_ev[1], edge->stream));
+        LR_CUDA(cudaStreamWaitEvent(surf->stream, surf->loam_ev[1], 0));
+    }
+    LR_CUDA(cudaMemsetAsync(d_key, 0xFF, sizeof(unsigned long long), surf->stream));
+    if (n_local)
+        LR_LAUNCH(k_score_argmin, static_cast<unsigned int>((n_local + 255) / 256), 256, 0, surf->stream, surf->d_results.as<DevResult>(),
+                  static_cast<unsigned int>(n_local), index_base, index_stride, surf->d_scores.as<double>(), d_key);
+    return d_key;
+}
+
+static int loam_relocalise_check(const locreg_handle* surf, const locreg_handle* edge, const float* surf_xyz, size_t n_surf,
+                                 const float* edge_xyz, size_t n_edge, size_t stride, const double* poses_in, size_t n_hyp) {
+    int rc = loam_check_handles(surf, edge);
+    if (rc) return rc;
+    rc = check_cloud_args(surf_xyz, n_surf, stride);
+    if (rc) return rc;
+    rc = check_cloud_args(edge_xyz, n_edge, stride);
+    if (rc) return rc;
+    if (!poses_in || n_hyp == 0 || n_hyp >= (1ull << 31)) { g_last_error = "invalid hypotheses"; return LOCREG_E_ARG; }
+    return LOCREG_OK;
+}
+
+int locreg_relocalise_loam(locreg_handle* surf, locreg_handle* edge, const float* surf_xyz, size_t n_surf, const float* edge_xyz,
+                           size_t n_edge, size_t stride, const double* poses_in, size_t n_hyp, int32_t max_iteration, double eps,
+                           double* best_pose, int64_t* best_idx, double* best_score, double* scores, double* poses_out) {
+    const int rc = loam_relocalise_check(surf, edge, surf_xyz, n_surf, edge_xyz, n_edge, stride, poses_in, n_hyp);
+    if (rc) return rc;
+    return guarded(surf, [&]() {
+        const int st = loam_prepare(surf, edge);
+        if (st) return st;
+        const float4* src_s = stage_cloud(surf, surf_xyz, n_surf, stride, false);
+        const float4* src_e = stage_cloud(edge, edge_xyz, n_edge, stride, false);
+        unsigned long long* d_key = loam_relocalise_core(surf, edge, src_s, n_surf, src_e, n_edge, poses_in, n_hyp, max_iteration, eps, 0u, 1u);
+        surf->end_timing();
+        cudaStream_t const s = surf->stream;
+        surf->h_small.reserve(4096);
+        unsigned long long* h_key = reinterpret_cast<unsigned long long*>(surf->h_small.as<unsigned char>() + 2048);
+        LR_CUDA(cudaMemcpyAsync(h_key, d_key, sizeof(unsigned long long), cudaMemcpyDeviceToHost, s));
+        LR_CUDA(cudaStreamSynchronize(s));
+        const uint32_t bi = static_cast<uint32_t>(*h_key & 0xFFFFFFFFull);
+        if (best_idx) *best_idx = bi;
+        if (best_score) LR_CUDA(cudaMemcpyAsync(best_score, surf->d_scores.as<double>() + bi, sizeof(double), cudaMemcpyDeviceToHost, s));
+        if (best_pose) LR_CUDA(cudaMemcpyAsync(best_pose, surf->d_poses_out.as<double>() + static_cast<size_t>(bi) * 7, 7 * sizeof(double), cudaMemcpyDeviceToHost, s));
+        if (scores) LR_CUDA(cudaMemcpyAsync(scores, surf->d_scores.p, n_hyp * sizeof(double), cudaMemcpyDeviceToHost, s));
+        if (poses_out) LR_CUDA(cudaMemcpyAsync(poses_out, surf->d_poses_out.p, n_hyp * 7 * sizeof(double), cudaMemcpyDeviceToHost, s));
+        LR_CUDA(cudaStreamSynchronize(s));
+        return LOCREG_OK;
+    });
+}
+
+int locreg_relocalise_loam_sharded(locreg_handle* surf, locreg_handle* edge, const float* surf_xyz, size_t n_surf, const float* edge_xyz,
+                                   size_t n_edge, size_t stride, const double* poses_in, size_t n_hyp, int32_t max_iteration, double eps,
+                                   double* best_pose, int64_t* best_idx, double* best_score) {
+    const int rc = loam_relocalise_check(surf, edge, surf_xyz, n_surf, edge_xyz, n_edge, stride, poses_in, n_hyp);
+    if (rc) return rc;
+    return guarded(surf, [&]() {
+        const int st = loam_prepare(surf, edge);
+        if (st) return st;
+        const float4* src_s = stage_cloud(surf, surf_xyz, n_surf, stride, false);
+        const float4* src_e = stage_cloud(edge, edge_xyz, n_edge, stride, false);
+        // surf's communicator (and stream) carry the exchange; edge's communicator is not used
+        relocalise_exchange(surf, poses_in, n_hyp, best_pose, best_idx, best_score,
+                            [&](const double* mine, size_t n_local, unsigned int rank, unsigned int world) {
+                                return loam_relocalise_core(surf, edge, src_s, n_surf, src_e, n_edge, mine, n_local, max_iteration, eps,
+                                                            rank, world);
+                            });
         return LOCREG_OK;
     });
 }

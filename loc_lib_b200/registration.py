@@ -400,6 +400,52 @@ class LoamRegistration:
                                                       pout.ctypes.data, res))
         return pout, [(res[2 * s].as_dict(), res[2 * s + 1].as_dict()) for s in range(S)]
 
+    def Relocalise(self, surf_cloud, edge_cloud, hypotheses, want_all=False):
+        """Global relocalisation of one surf / edge scan (locreg_relocalise_loam): every hypothesis runs the ScanMatch
+        loop, then both halves are scored once more at its final pose, score = (sum_sq_res_surf + sum_sq_res_edge) /
+        (n_inlier_surf + n_inlier_edge), +inf when the summed H is singular or no half has an inlier.  Returns
+        (best_pose, best_idx, best_score, scores, poses) as IcpRegistration.Relocalise; scores (n,) and poses (n, 7)
+        only with want_all."""
+        a, n_s, s_s, b, n_e = self._clouds(surf_cloud, edge_cloud)
+        hyp = np.ascontiguousarray(hypotheses, np.float64).reshape(-1, 7)
+        nh = hyp.shape[0]
+        best_pose = np.zeros(7)
+        best_idx = C.c_int64(-1)
+        best_score = C.c_double(np.inf)
+        scores = np.zeros(nh) if want_all else None
+        poses = np.zeros((nh, 7)) if want_all else None
+        _lib.check(_lib.lib().locreg_relocalise_loam(self.surf._h, self.edge._h, a.ctypes.data, n_s, b.ctypes.data, n_e, s_s,
+                                                     hyp.ctypes.data, nh, self.max_iteration, self.eps, best_pose.ctypes.data,
+                                                     C.byref(best_idx), C.byref(best_score),
+                                                     scores.ctypes.data if want_all else None,
+                                                     poses.ctypes.data if want_all else None))
+        return best_pose, int(best_idx.value), float(best_score.value), scores, poses
+
+    def RelocaliseSharded(self, surf_cloud, edge_cloud, hypotheses):
+        """Relocalise over the ranks of the surf handle's communicator (CommInit): every rank passes the same clouds and
+        hypotheses.  Returns (best_pose, best GLOBAL index, best_score), identical on every rank."""
+        a, n_s, s_s, b, n_e = self._clouds(surf_cloud, edge_cloud)
+        hyp = np.ascontiguousarray(hypotheses, np.float64).reshape(-1, 7)
+        best_pose = np.zeros(7)
+        best_idx = C.c_int64(-1)
+        best_score = C.c_double(np.inf)
+        _lib.check(_lib.lib().locreg_relocalise_loam_sharded(self.surf._h, self.edge._h, a.ctypes.data, n_s, b.ctypes.data, n_e,
+                                                             s_s, hyp.ctypes.data, hyp.shape[0], self.max_iteration, self.eps,
+                                                             best_pose.ctypes.data, C.byref(best_idx), C.byref(best_score)))
+        return best_pose, int(best_idx.value), float(best_score.value)
+
+    # the communicator of the sharded relocalisation is the surf handle's (loc_lib_b200.dist.comm_init works unchanged)
+    CommUniqueId = staticmethod(_Registration.CommUniqueId)
+
+    def CommInit(self, unique_id, rank, world):
+        self.surf.CommInit(unique_id, rank, world)
+
+    def CommInfo(self):
+        return self.surf.CommInfo()
+
+    def CommDestroy(self):
+        self.surf.CommDestroy()
+
     @staticmethod
     def _clouds(surf_cloud, edge_cloud):
         a, n_s, s_s = _cloud(surf_cloud)
