@@ -188,6 +188,33 @@ int locreg_relocalise(locreg_handle* h, const float* src, size_t n, size_t strid
 /* (float32 score bits << 32) | index: unsigned order = (score, index) order for score >= 0. */
 uint64_t locreg_pack_score(double score, uint32_t index);
 
+/* Staged global relocalisation: locreg_relocalise in n_rounds rounds, with the hypotheses that score worst dropped
+ * between rounds, so that far-off hypotheses do not pay for every trip.  It is the chain
+ *     alive = [0, n_hyp) (ascending original index); pose[i] = poses_in[i]
+ *     for r in 0 .. n_rounds-1:
+ *         every alive i runs locreg_relocalise's loop and score pass from pose[i] with trips[r] trips (the handle's eps
+ *         and gates; zero_initial_translation applies in round 0 only; later rounds start from the pose exactly as the
+ *         previous round left it) -> pose[i], score[i] (score as in locreg_relocalise)
+ *         if r < n_rounds-1: alive = the min(keep[r], |alive|) alive i with the smallest locreg_pack_score(score[i], i)
+ *     best = argmin over the last round's alive of locreg_pack_score(score[i], i) (lowest index on ties)
+ * Each round is a fresh loop: only the pose is carried over, no search state, so round r of hypothesis i is bit for
+ * bit what locreg_relocalise returns from that pose on a handle whose max_iteration is trips[r].  The handle's own
+ * max_iteration is not used, and its options are unchanged afterwards; trips[r] == 0 is a score-only round.  The
+ * cut ranks each hypothesis by its own score, so it does not depend on how hypotheses are grouped on the device.
+ * Every handle type locreg_relocalise accepts works (ICP and both NDT methods).  All rounds are queued back to back
+ * (the survivors are selected and gathered on the device) and the call synchronises once.
+ *   trips      n_rounds entries >= 0
+ *   keep       n_rounds - 1 entries >= 1 (may be NULL when n_rounds == 1)
+ *   scores / poses_out / rounds_out (n_hyp, n_hyp * 7, n_hyp; each may be NULL): every hypothesis's score and pose of
+ *              the last round it ran, and how many rounds it ran (1 .. n_rounds)
+ *   best_pose  poses_out[best_idx] bit for bit; best_score its score
+ * locreg_last_timing covers the kernels of all rounds.  Arguments are checked before any device work: LOCREG_E_ARG
+ * for bad cloud arguments (as locreg_relocalise), a null poses_in, n_hyp == 0 or n_hyp >= 2^31, n_rounds outside
+ * [1, 32], a null trips or trips[r] < 0, a null keep with n_rounds > 1, keep[r] < 1; LOCREG_E_STATE without a target. */
+int locreg_relocalise_staged(locreg_handle* h, const float* src, size_t n, size_t stride_bytes, const double* poses_in,
+                             size_t n_hyp, const int32_t* trips, const int64_t* keep, int32_t n_rounds, double* best_pose,
+                             int64_t* best_idx, double* best_score, double* scores, double* poses_out, int32_t* rounds_out);
+
 /* ---- multi-GPU (SURVEY.md 8e): one process (or thread) per GPU, one handle each, NCCL inside this library -----------
  * The two workloads that shard keep a replica of the map per GPU and need ONE exchange step each; it runs on the
  * handle's stream right behind the kernels, so nothing returns to the host in between.  NCCL is bound at run time

@@ -18,6 +18,7 @@
 #include "icp_fused.cuh"
 #include "icp_staged.cuh"
 #include "icp_persist.cuh"
+#include "reloc_select.cuh"
 #include "nccl_dyn.h"
 
 #include <nvtx3/nvToolsExt.h>
@@ -107,6 +108,9 @@ struct locreg_handle {
     DevBuf d_gather_pose, d_gather_res, d_bcast;
     DevBuf d_raw, d_src4, d_out, d_partials, d_state, d_acc, d_gate, d_nn, d_offsets, d_poses_in, d_poses_out, d_results,
         d_scores, d_misc, d_target, d_nnpos, d_tile_begin, d_tiles, d_states, d_ringq, d_ringc, d_sortq, d_sortb, d_sorth, d_rescanq, d_rescanc, d_loam, d_lmap_new, d_global, d_local, d_same, d_plane, d_pstat, d_track;
+    // locreg_relocalise_staged: the cut's keys, flags / slots, the two index maps of the rounds, the caller-order
+    // outputs, and the select state + histogram + best
+    DevBuf d_stage_keys, d_stage_slot, d_stage_idx, d_stage_poses, d_stage_scores, d_stage_rounds, d_stage_sel;
     size_t n_global = 0, global_stride = 0;  // Loc's global map kept on the device (locreg_set_global_map)
     // Lio's sliding local map (locreg_local_map_add_keyframe): transformed key frames + the filtered local map
     struct KeyFrame { void* p = nullptr; size_t n = 0; };
@@ -1459,9 +1463,11 @@ static IcpJob hypothesis_job(const float4* src4, size_t n, unsigned int W, Align
 
 // n_local hypotheses (host, 7 doubles each) of ONE scan -> h->d_poses_out / d_results / d_scores and the packed best key
 // in device memory (returned pointer); the index in the key is index_base + i * index_stride.  Everything is queued on
-// the handle's stream; nothing is synchronised.
+// the handle's stream; nothing is synchronised.  poses_in == nullptr: h->d_poses_in already holds the poses (a round of
+// locreg_relocalise_staged).  begin_timing: the handle's timing starts here, after the poses' upload; a staged call
+// starts it once before its first round instead.  The loop reads max_iteration and zero_initial_translation from h->opt.
 static unsigned long long* relocalise_core(locreg_handle* h, const float4* src4, size_t n, const double* poses_in, size_t n_local,
-                                           unsigned int index_base, unsigned int index_stride) {
+                                           unsigned int index_base, unsigned int index_stride, bool begin_timing) {
     NvtxRange r("locreg:relocalise");
     h->d_poses_in.reserve(std::max<size_t>(n_local, 1) * 7 * sizeof(double));
     h->d_poses_out.reserve(std::max<size_t>(n_local, 1) * 7 * sizeof(double));
@@ -1470,10 +1476,10 @@ static unsigned long long* relocalise_core(locreg_handle* h, const float4* src4,
     h->d_misc.reserve(64);
     unsigned long long* d_key = reinterpret_cast<unsigned long long*>(h->d_misc.as<unsigned char>() + 32);
     if (n_local) {
-        LR_CUDA(cudaMemcpyAsync(h->d_poses_in.p, poses_in, n_local * 7 * sizeof(double), cudaMemcpyHostToDevice, h->stream));
+        if (poses_in) LR_CUDA(cudaMemcpyAsync(h->d_poses_in.p, poses_in, n_local * 7 * sizeof(double), cudaMemcpyHostToDevice, h->stream));
         LR_CUDA(cudaMemcpyAsync(h->d_poses_out.p, h->d_poses_in.p, n_local * 7 * sizeof(double), cudaMemcpyDeviceToDevice, h->stream));
     }
-    h->begin_timing();
+    if (begin_timing) h->begin_timing();
     if (n_local && is_ndt(h)) {
         // one CTA per hypothesis: Gauss-Newton loop + one evaluation at the final pose (the score), all inside the CTA
         NDT_DISPATCH(h, ndt_run_batch(h, PB, src4, nullptr, h->d_poses_in.as<double>(), h->d_poses_out.as<double>(),
@@ -1506,7 +1512,7 @@ int locreg_relocalise(locreg_handle* h, const float* src, size_t n, size_t strid
     return guarded(h, [&]() {
         if (!h->has_target) { g_last_error = "SetInputTarget has not been called"; return LOCREG_E_STATE; }
         const float4* src4 = stage_cloud(h, src, n, stride, false);
-        unsigned long long* d_key = relocalise_core(h, src4, n, poses_in, n_hyp, 0u, 1u);
+        unsigned long long* d_key = relocalise_core(h, src4, n, poses_in, n_hyp, 0u, 1u, true);
         h->end_timing();
         unsigned long long key = 0;
         LR_CUDA(cudaMemcpy(&key, d_key, sizeof(key), cudaMemcpyDeviceToHost));
@@ -1516,6 +1522,121 @@ int locreg_relocalise(locreg_handle* h, const float* src, size_t n, size_t strid
         if (best_pose) LR_CUDA(cudaMemcpy(best_pose, h->d_poses_out.as<double>() + static_cast<size_t>(bi) * 7, 7 * sizeof(double), cudaMemcpyDeviceToHost));
         if (scores) LR_CUDA(cudaMemcpy(scores, h->d_scores.p, n_hyp * sizeof(double), cudaMemcpyDeviceToHost));
         if (poses_out) LR_CUDA(cudaMemcpy(poses_out, h->d_poses_out.p, n_hyp * 7 * sizeof(double), cudaMemcpyDeviceToHost));
+        return LOCREG_OK;
+    });
+}
+
+// The handle's loop options as they were, restored when the scope ends (also on an exception): the rounds of a staged
+// relocalisation set their own trip count and zero_initial_translation, and every later call must see the caller's.
+struct ScopedLoopOptions {
+    locreg_handle* h;
+    int32_t max_iteration, zero_initial_translation;
+    explicit ScopedLoopOptions(locreg_handle* hh)
+        : h(hh), max_iteration(hh->opt.max_iteration), zero_initial_translation(hh->opt.zero_initial_translation) {}
+    ~ScopedLoopOptions() {
+        h->opt.max_iteration = max_iteration;
+        h->opt.zero_initial_translation = zero_initial_translation;
+    }
+    ScopedLoopOptions(const ScopedLoopOptions&) = delete;
+    ScopedLoopOptions& operator=(const ScopedLoopOptions&) = delete;
+};
+
+// Staged relocalisation (include/locreg.h): round r is relocalise_core on the alive hypotheses with trips[r] trips;
+// between rounds the survivors are cut on the device (reloc_select.cuh) and their poses gathered into d_poses_in, so
+// all rounds are queued back to back and the call synchronises once.  Round r's positions map to original indices
+// through d_stage_idx half (r & 1) (round 0: the identity, no map).  The winner is the same select with k = 1 over the
+// last round, so the cuts and the winner rank by one key, locreg_pack_score's.
+int locreg_relocalise_staged(locreg_handle* h, const float* src, size_t n, size_t stride, const double* poses_in, size_t n_hyp,
+                             const int32_t* trips, const int64_t* keep, int32_t n_rounds, double* best_pose, int64_t* best_idx,
+                             double* best_score, double* scores, double* poses_out, int32_t* rounds_out) {
+    const int rc = check_cloud_args(src, n, stride);
+    if (rc) return rc;
+    if (!poses_in || n_hyp == 0 || n_hyp >= (1ull << 31)) { g_last_error = "invalid hypotheses"; return LOCREG_E_ARG; }
+    if (n_rounds < 1 || n_rounds > 32) { g_last_error = "n_rounds must be in [1, 32]"; return LOCREG_E_ARG; }
+    if (!trips) { g_last_error = "invalid trips (null)"; return LOCREG_E_ARG; }
+    for (int32_t r = 0; r < n_rounds; ++r)
+        if (trips[r] < 0) { g_last_error = "invalid trips (negative)"; return LOCREG_E_ARG; }
+    if (n_rounds > 1 && !keep) { g_last_error = "invalid keep (null with more than one round)"; return LOCREG_E_ARG; }
+    for (int32_t r = 0; r + 1 < n_rounds; ++r)
+        if (keep[r] < 1) { g_last_error = "invalid keep (< 1)"; return LOCREG_E_ARG; }
+    return guarded(h, [&]() {
+        if (!h->has_target) { g_last_error = "SetInputTarget has not been called"; return LOCREG_E_STATE; }
+        NvtxRange nr("locreg:relocalise_staged");
+        std::vector<size_t> alive(n_rounds);  // hypotheses in round r, known before anything runs
+        alive[0] = n_hyp;
+        for (int32_t r = 1; r < n_rounds; ++r) alive[r] = std::min<size_t>(static_cast<size_t>(keep[r - 1]), alive[r - 1]);
+        const float4* src4 = stage_cloud(h, src, n, stride, false);
+        // every per-hypothesis buffer at its full size before the first launch (relocalise_core's reserves are then no-ops)
+        h->d_poses_in.reserve(n_hyp * 7 * sizeof(double));
+        h->d_poses_out.reserve(n_hyp * 7 * sizeof(double));
+        h->d_results.reserve(n_hyp * sizeof(DevResult));
+        h->d_scores.reserve(n_hyp * sizeof(double));
+        h->d_misc.reserve(64);
+        h->d_stage_keys.reserve(n_hyp * sizeof(unsigned long long));
+        h->d_stage_slot.reserve(n_hyp * sizeof(unsigned int));
+        h->d_stage_idx.reserve(2 * n_hyp * sizeof(unsigned int));
+        h->d_stage_poses.reserve(n_hyp * 7 * sizeof(double));
+        h->d_stage_scores.reserve(n_hyp * sizeof(double));
+        h->d_stage_rounds.reserve(n_hyp * sizeof(int32_t));
+        // select state | histogram | best pose + score | best index
+        constexpr size_t kHistOff = 64, kBestOff = kHistOff + kSelectBins * sizeof(unsigned int), kBestIdxOff = kBestOff + 8 * sizeof(double);
+        h->d_stage_sel.reserve(kBestIdxOff + sizeof(long long));
+        unsigned char* sel = h->d_stage_sel.as<unsigned char>();
+        SelectState* st = reinterpret_cast<SelectState*>(sel);
+        unsigned int* hist = reinterpret_cast<unsigned int*>(sel + kHistOff);
+        double* d_best = reinterpret_cast<double*>(sel + kBestOff);
+        long long* d_best_idx = reinterpret_cast<long long*>(sel + kBestIdxOff);
+        unsigned int* idx[2] = {h->d_stage_idx.as<unsigned int>(), h->d_stage_idx.as<unsigned int>() + n_hyp};
+        LR_CUDA(cudaMemcpyAsync(h->d_poses_in.p, poses_in, n_hyp * 7 * sizeof(double), cudaMemcpyHostToDevice, h->stream));
+        LR_CUDA(cudaMemsetAsync(hist, 0, kSelectBins * sizeof(unsigned int), h->stream));  // k_select_digit re-zeroes it
+        h->begin_timing();
+        {
+            ScopedLoopOptions saved(h);
+            unsigned long long* keys = h->d_stage_keys.as<unsigned long long>();
+            // st->prefix = the k-th smallest key of the round's m scores (in h->d_scores)
+            const auto select_kth = [&](unsigned int m, unsigned int k) {
+                const unsigned int g = (m + 255) / 256;
+                LR_LAUNCH(k_reloc_keys, g, 256, 0, h->stream, h->d_scores.as<double>(), m, keys);
+                const unsigned int gh = std::min<unsigned int>(g, 2u * static_cast<unsigned int>(h->num_sms));
+                for (int d = 0; d < 8; ++d) {
+                    LR_LAUNCH(k_select_hist, gh, 256, 0, h->stream, keys, m, st, d, hist);
+                    LR_LAUNCH(k_select_digit, 1, kSelectBins, 0, h->stream, st, hist, d, k);
+                }
+            };
+            for (int32_t r = 0; r < n_rounds; ++r) {
+                const unsigned int m = static_cast<unsigned int>(alive[r]);
+                const unsigned int g = (m + 255) / 256;
+                const unsigned int* idx_r = r == 0 ? nullptr : idx[r & 1];
+                h->opt.max_iteration = trips[r];
+                if (r > 0) h->opt.zero_initial_translation = 0;  // later rounds start from the pose as the last one left it
+                relocalise_core(h, src4, n, nullptr, m, 0u, 1u, false);
+                LR_LAUNCH(k_reloc_scatter, g, 256, 0, h->stream, m, idx_r, h->d_poses_out.as<double>(), h->d_scores.as<double>(), r,
+                          h->d_stage_poses.as<double>(), h->d_stage_scores.as<double>(), h->d_stage_rounds.as<int>());
+                if (r + 1 == n_rounds) {
+                    select_kth(m, 1u);
+                    break;
+                }
+                select_kth(m, static_cast<unsigned int>(alive[r + 1]));
+                unsigned int* slot = h->d_stage_slot.as<unsigned int>();
+                LR_LAUNCH(k_select_flags, g, 256, 0, h->stream, keys, m, st, slot);
+                exclusive_scan_u32(slot, slot, m, nullptr, h->stream);
+                LR_LAUNCH(k_reloc_compact, g, 256, 0, h->stream, keys, m, st, slot, h->d_poses_out.as<double>(), idx_r,
+                          h->d_poses_in.as<double>(), idx[(r + 1) & 1]);
+            }
+            LR_LAUNCH(k_reloc_best, 1, 32, 0, h->stream, st, n_rounds > 1 ? idx[(n_rounds - 1) & 1] : nullptr,
+                      h->d_stage_poses.as<double>(), h->d_stage_scores.as<double>(), d_best, d_best_idx);
+        }
+        h->end_timing();
+        double b[8];
+        long long bi = 0;
+        LR_CUDA(cudaMemcpy(b, d_best, sizeof(b), cudaMemcpyDeviceToHost));
+        LR_CUDA(cudaMemcpy(&bi, d_best_idx, sizeof(bi), cudaMemcpyDeviceToHost));
+        if (best_idx) *best_idx = bi;
+        if (best_pose) std::memcpy(best_pose, b, 7 * sizeof(double));
+        if (best_score) *best_score = b[7];
+        if (scores) LR_CUDA(cudaMemcpy(scores, h->d_stage_scores.p, n_hyp * sizeof(double), cudaMemcpyDeviceToHost));
+        if (poses_out) LR_CUDA(cudaMemcpy(poses_out, h->d_stage_poses.p, n_hyp * 7 * sizeof(double), cudaMemcpyDeviceToHost));
+        if (rounds_out) LR_CUDA(cudaMemcpy(rounds_out, h->d_stage_rounds.p, n_hyp * sizeof(int32_t), cudaMemcpyDeviceToHost));
         return LOCREG_OK;
     });
 }
@@ -1646,7 +1767,7 @@ int locreg_relocalise_sharded(locreg_handle* h, const float* src, size_t n, size
         const float4* src4 = stage_cloud(h, src, n, stride, false);
         relocalise_exchange(h, poses_in, n_hyp, best_pose, best_idx, best_score,
                             [&](const double* mine, size_t n_local, unsigned int rank, unsigned int world) {
-                                return relocalise_core(h, src4, n, mine, n_local, rank, world);
+                                return relocalise_core(h, src4, n, mine, n_local, rank, world, true);
                             });
         return LOCREG_OK;
     });

@@ -167,6 +167,32 @@ class _Registration:
                                                 poses.ctypes.data if want_all else None))
         return best_pose, int(best_idx.value), float(best_score.value), scores, poses
 
+    def RelocaliseStaged(self, cloud, hypotheses, trips, keep, want_all=False):
+        """Relocalise in len(trips) rounds of trips[r] Gauss-Newton trips, keeping the keep[r] best-scoring hypotheses
+        after round r (keep has len(trips) - 1 entries; see locreg_relocalise_staged).  Returns (best_pose, best_idx,
+        best_score, scores, poses, rounds): with want_all, every hypothesis's score and pose of the last round it ran and
+        how many rounds it ran; otherwise the last three are None."""
+        a, n, s = _cloud(cloud)
+        hyp = np.ascontiguousarray(hypotheses, np.float64).reshape(-1, 7)
+        nh = hyp.shape[0]
+        trips = np.ascontiguousarray(trips, np.int32).reshape(-1)
+        keep = np.ascontiguousarray([] if keep is None else keep, np.int64).reshape(-1)
+        if keep.shape[0] != max(trips.shape[0] - 1, 0):
+            raise ValueError("keep must have len(trips) - 1 entries")
+        best_pose = np.zeros(7)
+        best_idx = C.c_int64(-1)
+        best_score = C.c_double(np.inf)
+        scores = np.zeros(nh) if want_all else None
+        poses = np.zeros((nh, 7)) if want_all else None
+        rounds = np.zeros(nh, np.int32) if want_all else None
+        _lib.check(_lib.lib().locreg_relocalise_staged(self._h, a.ctypes.data, n, s, hyp.ctypes.data, nh, trips.ctypes.data,
+                                                       keep.ctypes.data if keep.size else None, trips.shape[0],
+                                                       best_pose.ctypes.data, C.byref(best_idx), C.byref(best_score),
+                                                       scores.ctypes.data if want_all else None,
+                                                       poses.ctypes.data if want_all else None,
+                                                       rounds.ctypes.data if want_all else None))
+        return best_pose, int(best_idx.value), float(best_score.value), scores, poses, rounds
+
     # ---- multi-GPU: NCCL inside liblocreg.so (one process per GPU; see loc_lib_b200/dist.py for the torchrun plumbing) ----
     @staticmethod
     def CommUniqueId():
