@@ -243,6 +243,23 @@ int locreg_shard_range(size_t n, int32_t rank, int32_t world, size_t* lo, size_t
 int locreg_relocalise_sharded(locreg_handle* h, const float* src, size_t n, size_t stride_bytes, const double* poses_in,
                               size_t n_hyp, double* best_pose, int64_t* best_idx, double* best_score);
 
+/* locreg_relocalise_staged over all ranks of the handle's communicator (none, or a one-rank communicator: it IS
+ * locreg_relocalise_staged).  EVERY rank passes the same scan, the same n_hyp hypotheses and the same schedule.  In
+ * round r the m alive hypotheses (positions 0 .. m-1 in ascending original index, the same list on every rank) are
+ * dealt by position: rank q runs positions q, q + world, ... (round 0 is locreg_relocalise_sharded's deal; after every
+ * cut the survivors are dealt afresh, so the ranks stay balanced to one hypothesis).  Then, on the handle's stream,
+ *     ncclAllGather(ceil(m / world) records of 8 doubles: pose + score, in place)
+ * gives every rank the whole round, and every rank makes the same cut (and at the end picks the same winner) on the
+ * device.  Every output - best_pose, best_idx, best_score, scores, poses_out, rounds_out (each may be NULL) - is bit
+ * for bit what locreg_relocalise_staged returns on one GPU with the same arguments, on every rank.  Each round moves
+ * m * 64 bytes through the all-gather; a rank with no hypothesis in a round runs no registration but joins the
+ * collective.  Argument checks and error codes are those of locreg_relocalise_staged; the handle's options are
+ * unchanged afterwards; locreg_last_timing covers all rounds and their collectives. */
+int locreg_relocalise_staged_sharded(locreg_handle* h, const float* src, size_t n, size_t stride_bytes,
+                                     const double* poses_in, size_t n_hyp, const int32_t* trips, const int64_t* keep,
+                                     int32_t n_rounds, double* best_pose, int64_t* best_idx, double* best_score,
+                                     double* scores, double* poses_out, int32_t* rounds_out);
+
 /* LOAM global relocalisation: n_hyp locreg_align_loam calls of ONE surf / edge scan from different initial poses, in
  * one device-resident loop (hypotheses run in waves that bound the per-point scratch; the waves do not change results).
  *   loop     hypothesis i runs the LOAM loop of locreg_align_loam from poses_in[i] (7 doubles) as given, with the same

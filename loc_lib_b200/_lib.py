@@ -22,6 +22,7 @@ SYMBOLS = [
     "locreg_comm_unique_id", "locreg_comm_init", "locreg_comm_destroy", "locreg_comm_info", "locreg_shard_range",
     "locreg_relocalise_sharded", "locreg_align_batch_sharded", "locreg_index_info", "locreg_align_loam",
     "locreg_align_loam_batch", "locreg_relocalise_loam", "locreg_relocalise_loam_sharded", "locreg_relocalise_staged",
+    "locreg_relocalise_staged_sharded",
 ]
 
 
@@ -72,6 +73,7 @@ def lib():
         L.locreg_align_batch_device.argtypes = [vp, vp, vp, vp, sz, sz, vp, vp]
         L.locreg_relocalise.argtypes = [vp, vp, sz, sz, vp, sz, vp, vp, vp, vp, vp]
         L.locreg_relocalise_staged.argtypes = [vp, vp, sz, sz, vp, sz, vp, vp, i32, vp, vp, vp, vp, vp, vp]
+        L.locreg_relocalise_staged_sharded.argtypes = [vp, vp, sz, sz, vp, sz, vp, vp, i32, vp, vp, vp, vp, vp, vp]
         L.locreg_pack_score.restype = C.c_uint64
         L.locreg_pack_score.argtypes = [C.c_double, C.c_uint32]
         L.locreg_transform_cloud.argtypes = [vp, vp, sz, sz, vp, vp]

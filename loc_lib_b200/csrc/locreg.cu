@@ -111,6 +111,9 @@ struct locreg_handle {
     // locreg_relocalise_staged: the cut's keys, flags / slots, the two index maps of the rounds, the caller-order
     // outputs, and the select state + histogram + best
     DevBuf d_stage_keys, d_stage_slot, d_stage_idx, d_stage_poses, d_stage_scores, d_stage_rounds, d_stage_sel;
+    // ... and across ranks (locreg_relocalise_staged_sharded): every round's full pose array, which each rank deals its
+    // share from, and the all-gather buffer of the round's results
+    DevBuf d_stage_full, d_stage_gather;
     size_t n_global = 0, global_stride = 0;  // Loc's global map kept on the device (locreg_set_global_map)
     // Lio's sliding local map (locreg_local_map_add_keyframe): transformed key frames + the filtered local map
     struct KeyFrame { void* p = nullptr; size_t n = 0; };
@@ -1541,14 +1544,9 @@ struct ScopedLoopOptions {
     ScopedLoopOptions& operator=(const ScopedLoopOptions&) = delete;
 };
 
-// Staged relocalisation (include/locreg.h): round r is relocalise_core on the alive hypotheses with trips[r] trips;
-// between rounds the survivors are cut on the device (reloc_select.cuh) and their poses gathered into d_poses_in, so
-// all rounds are queued back to back and the call synchronises once.  Round r's positions map to original indices
-// through d_stage_idx half (r & 1) (round 0: the identity, no map).  The winner is the same select with k = 1 over the
-// last round, so the cuts and the winner rank by one key, locreg_pack_score's.
-int locreg_relocalise_staged(locreg_handle* h, const float* src, size_t n, size_t stride, const double* poses_in, size_t n_hyp,
-                             const int32_t* trips, const int64_t* keep, int32_t n_rounds, double* best_pose, int64_t* best_idx,
-                             double* best_score, double* scores, double* poses_out, int32_t* rounds_out) {
+// Argument checks of locreg_relocalise_staged[_sharded], before any device work.
+static int staged_check(const float* src, size_t n, size_t stride, const double* poses_in, size_t n_hyp, const int32_t* trips,
+                        const int64_t* keep, int32_t n_rounds) {
     const int rc = check_cloud_args(src, n, stride);
     if (rc) return rc;
     if (!poses_in || n_hyp == 0 || n_hyp >= (1ull << 31)) { g_last_error = "invalid hypotheses"; return LOCREG_E_ARG; }
@@ -1559,85 +1557,152 @@ int locreg_relocalise_staged(locreg_handle* h, const float* src, size_t n, size_
     if (n_rounds > 1 && !keep) { g_last_error = "invalid keep (null with more than one round)"; return LOCREG_E_ARG; }
     for (int32_t r = 0; r + 1 < n_rounds; ++r)
         if (keep[r] < 1) { g_last_error = "invalid keep (< 1)"; return LOCREG_E_ARG; }
-    return guarded(h, [&]() {
-        if (!h->has_target) { g_last_error = "SetInputTarget has not been called"; return LOCREG_E_STATE; }
-        NvtxRange nr("locreg:relocalise_staged");
-        std::vector<size_t> alive(n_rounds);  // hypotheses in round r, known before anything runs
-        alive[0] = n_hyp;
-        for (int32_t r = 1; r < n_rounds; ++r) alive[r] = std::min<size_t>(static_cast<size_t>(keep[r - 1]), alive[r - 1]);
-        const float4* src4 = stage_cloud(h, src, n, stride, false);
-        // every per-hypothesis buffer at its full size before the first launch (relocalise_core's reserves are then no-ops)
-        h->d_poses_in.reserve(n_hyp * 7 * sizeof(double));
-        h->d_poses_out.reserve(n_hyp * 7 * sizeof(double));
-        h->d_results.reserve(n_hyp * sizeof(DevResult));
-        h->d_scores.reserve(n_hyp * sizeof(double));
-        h->d_misc.reserve(64);
-        h->d_stage_keys.reserve(n_hyp * sizeof(unsigned long long));
-        h->d_stage_slot.reserve(n_hyp * sizeof(unsigned int));
-        h->d_stage_idx.reserve(2 * n_hyp * sizeof(unsigned int));
-        h->d_stage_poses.reserve(n_hyp * 7 * sizeof(double));
-        h->d_stage_scores.reserve(n_hyp * sizeof(double));
-        h->d_stage_rounds.reserve(n_hyp * sizeof(int32_t));
-        // select state | histogram | best pose + score | best index
-        constexpr size_t kHistOff = 64, kBestOff = kHistOff + kSelectBins * sizeof(unsigned int), kBestIdxOff = kBestOff + 8 * sizeof(double);
-        h->d_stage_sel.reserve(kBestIdxOff + sizeof(long long));
-        unsigned char* sel = h->d_stage_sel.as<unsigned char>();
-        SelectState* st = reinterpret_cast<SelectState*>(sel);
-        unsigned int* hist = reinterpret_cast<unsigned int*>(sel + kHistOff);
-        double* d_best = reinterpret_cast<double*>(sel + kBestOff);
-        long long* d_best_idx = reinterpret_cast<long long*>(sel + kBestIdxOff);
-        unsigned int* idx[2] = {h->d_stage_idx.as<unsigned int>(), h->d_stage_idx.as<unsigned int>() + n_hyp};
-        LR_CUDA(cudaMemcpyAsync(h->d_poses_in.p, poses_in, n_hyp * 7 * sizeof(double), cudaMemcpyHostToDevice, h->stream));
-        LR_CUDA(cudaMemsetAsync(hist, 0, kSelectBins * sizeof(unsigned int), h->stream));  // k_select_digit re-zeroes it
-        h->begin_timing();
-        {
-            ScopedLoopOptions saved(h);
-            unsigned long long* keys = h->d_stage_keys.as<unsigned long long>();
-            // st->prefix = the k-th smallest key of the round's m scores (in h->d_scores)
-            const auto select_kth = [&](unsigned int m, unsigned int k) {
-                const unsigned int g = (m + 255) / 256;
-                LR_LAUNCH(k_reloc_keys, g, 256, 0, h->stream, h->d_scores.as<double>(), m, keys);
-                const unsigned int gh = std::min<unsigned int>(g, 2u * static_cast<unsigned int>(h->num_sms));
-                for (int d = 0; d < 8; ++d) {
-                    LR_LAUNCH(k_select_hist, gh, 256, 0, h->stream, keys, m, st, d, hist);
-                    LR_LAUNCH(k_select_digit, 1, kSelectBins, 0, h->stream, st, hist, d, k);
-                }
-            };
-            for (int32_t r = 0; r < n_rounds; ++r) {
-                const unsigned int m = static_cast<unsigned int>(alive[r]);
-                const unsigned int g = (m + 255) / 256;
-                const unsigned int* idx_r = r == 0 ? nullptr : idx[r & 1];
-                h->opt.max_iteration = trips[r];
-                if (r > 0) h->opt.zero_initial_translation = 0;  // later rounds start from the pose as the last one left it
-                relocalise_core(h, src4, n, nullptr, m, 0u, 1u, false);
-                LR_LAUNCH(k_reloc_scatter, g, 256, 0, h->stream, m, idx_r, h->d_poses_out.as<double>(), h->d_scores.as<double>(), r,
-                          h->d_stage_poses.as<double>(), h->d_stage_scores.as<double>(), h->d_stage_rounds.as<int>());
-                if (r + 1 == n_rounds) {
-                    select_kth(m, 1u);
-                    break;
-                }
-                select_kth(m, static_cast<unsigned int>(alive[r + 1]));
-                unsigned int* slot = h->d_stage_slot.as<unsigned int>();
-                LR_LAUNCH(k_select_flags, g, 256, 0, h->stream, keys, m, st, slot);
-                exclusive_scan_u32(slot, slot, m, nullptr, h->stream);
-                LR_LAUNCH(k_reloc_compact, g, 256, 0, h->stream, keys, m, st, slot, h->d_poses_out.as<double>(), idx_r,
-                          h->d_poses_in.as<double>(), idx[(r + 1) & 1]);
+    return LOCREG_OK;
+}
+
+// Staged relocalisation (include/locreg.h) over `world` ranks of comm (world 1: comm unused): round r is relocalise_core
+// on the alive hypotheses with trips[r] trips; between rounds the survivors are cut on the device (reloc_select.cuh) and
+// their poses gathered into the next round's full pose array, so all rounds are queued back to back and the call
+// synchronises once.  Round r's positions map to original indices through d_stage_idx half (r & 1) (round 0: the
+// identity, no map).  The winner is the same select with k = 1 over the last round, so the cuts and the winner rank by
+// one key, locreg_pack_score's.
+// world 1: the full pose array is d_poses_in itself and relocalise_core runs all m alive hypotheses.  world > 1: it is
+// d_stage_full; rank q deals itself positions q, q + world, ... into d_poses_in and runs those, and the round's results
+// come back to every rank through one ncclAllGather (k_reloc_pack / k_reloc_unpack) into d_poses_out / d_scores at all m
+// positions, as one GPU leaves them.  The cut and the winner then run redundantly on every rank over identical keys.
+static int relocalise_staged_rounds(locreg_handle* h, const float* src, size_t n, size_t stride, const double* poses_in,
+                                    size_t n_hyp, const int32_t* trips, const int64_t* keep, int32_t n_rounds,
+                                    double* best_pose, int64_t* best_idx, double* best_score, double* scores,
+                                    double* poses_out, int32_t* rounds_out, unsigned int rank, unsigned int world,
+                                    ncclComm_t comm) {
+    if (!h->has_target) { g_last_error = "SetInputTarget has not been called"; return LOCREG_E_STATE; }
+    NvtxRange nr("locreg:relocalise_staged");
+    std::vector<size_t> alive(n_rounds);  // hypotheses in round r, known before anything runs
+    alive[0] = n_hyp;
+    for (int32_t r = 1; r < n_rounds; ++r) alive[r] = std::min<size_t>(static_cast<size_t>(keep[r - 1]), alive[r - 1]);
+    const float4* src4 = stage_cloud(h, src, n, stride, false);
+    // every per-hypothesis buffer at its full size before the first launch (relocalise_core's reserves are then no-ops)
+    h->d_poses_in.reserve(n_hyp * 7 * sizeof(double));
+    h->d_poses_out.reserve(n_hyp * 7 * sizeof(double));
+    h->d_results.reserve(n_hyp * sizeof(DevResult));
+    h->d_scores.reserve(n_hyp * sizeof(double));
+    h->d_misc.reserve(64);
+    h->d_stage_keys.reserve(n_hyp * sizeof(unsigned long long));
+    h->d_stage_slot.reserve(n_hyp * sizeof(unsigned int));
+    h->d_stage_idx.reserve(2 * n_hyp * sizeof(unsigned int));
+    h->d_stage_poses.reserve(n_hyp * 7 * sizeof(double));
+    h->d_stage_scores.reserve(n_hyp * sizeof(double));
+    h->d_stage_rounds.reserve(n_hyp * sizeof(int32_t));
+    if (world > 1) {
+        h->d_stage_full.reserve(n_hyp * 7 * sizeof(double));
+        h->d_stage_gather.reserve(world * ((n_hyp + world - 1) / world) * 8 * sizeof(double));
+    }
+    // select state | histogram | best pose + score | best index
+    constexpr size_t kHistOff = 64, kBestOff = kHistOff + kSelectBins * sizeof(unsigned int), kBestIdxOff = kBestOff + 8 * sizeof(double);
+    h->d_stage_sel.reserve(kBestIdxOff + sizeof(long long));
+    unsigned char* sel = h->d_stage_sel.as<unsigned char>();
+    SelectState* st = reinterpret_cast<SelectState*>(sel);
+    unsigned int* hist = reinterpret_cast<unsigned int*>(sel + kHistOff);
+    double* d_best = reinterpret_cast<double*>(sel + kBestOff);
+    long long* d_best_idx = reinterpret_cast<long long*>(sel + kBestIdxOff);
+    unsigned int* idx[2] = {h->d_stage_idx.as<unsigned int>(), h->d_stage_idx.as<unsigned int>() + n_hyp};
+    double* full = world > 1 ? h->d_stage_full.as<double>() : h->d_poses_in.as<double>();  // the round's alive poses
+    LR_CUDA(cudaMemcpyAsync(full, poses_in, n_hyp * 7 * sizeof(double), cudaMemcpyHostToDevice, h->stream));
+    LR_CUDA(cudaMemsetAsync(hist, 0, kSelectBins * sizeof(unsigned int), h->stream));  // k_select_digit re-zeroes it
+    h->begin_timing();
+    {
+        ScopedLoopOptions saved(h);
+        unsigned long long* keys = h->d_stage_keys.as<unsigned long long>();
+        // st->prefix = the k-th smallest key of the round's m scores (in h->d_scores)
+        const auto select_kth = [&](unsigned int m, unsigned int k) {
+            const unsigned int g = (m + 255) / 256;
+            LR_LAUNCH(k_reloc_keys, g, 256, 0, h->stream, h->d_scores.as<double>(), m, keys);
+            const unsigned int gh = std::min<unsigned int>(g, 2u * static_cast<unsigned int>(h->num_sms));
+            for (int d = 0; d < 8; ++d) {
+                LR_LAUNCH(k_select_hist, gh, 256, 0, h->stream, keys, m, st, d, hist);
+                LR_LAUNCH(k_select_digit, 1, kSelectBins, 0, h->stream, st, hist, d, k);
             }
-            LR_LAUNCH(k_reloc_best, 1, 32, 0, h->stream, st, n_rounds > 1 ? idx[(n_rounds - 1) & 1] : nullptr,
-                      h->d_stage_poses.as<double>(), h->d_stage_scores.as<double>(), d_best, d_best_idx);
+        };
+        for (int32_t r = 0; r < n_rounds; ++r) {
+            const unsigned int m = static_cast<unsigned int>(alive[r]);
+            const unsigned int g = (m + 255) / 256;
+            const unsigned int* idx_r = r == 0 ? nullptr : idx[r & 1];
+            h->opt.max_iteration = trips[r];
+            if (r > 0) h->opt.zero_initial_translation = 0;  // later rounds start from the pose as the last one left it
+            if (world == 1) {
+                relocalise_core(h, src4, n, nullptr, m, 0u, 1u, false);
+            } else {
+                const unsigned int m_q = m > rank ? (m - rank + world - 1) / world : 0u, c = (m + world - 1) / world;
+                double* gather = h->d_stage_gather.as<double>();
+                double* slab = gather + static_cast<size_t>(rank) * c * 8;
+                const auto blocks = [](size_t words) { return static_cast<unsigned int>((words + 255) / 256); };  // a thread per double
+                if (m_q) LR_LAUNCH(k_reloc_deal, blocks(static_cast<size_t>(m_q) * 7), 256, 0, h->stream, full, m_q, rank, world,
+                                   h->d_poses_in.as<double>());
+                relocalise_core(h, src4, n, nullptr, m_q, 0u, 1u, false);
+                if (m_q) LR_LAUNCH(k_reloc_pack, blocks(static_cast<size_t>(m_q) * 8), 256, 0, h->stream, h->d_poses_out.as<double>(),
+                                   h->d_scores.as<double>(), m_q, slab);
+                {
+                    NvtxRange ar("locreg:relocalise_staged:allgather");
+                    LR_NCCL(nccl_api().AllGather(slab, gather, static_cast<size_t>(c) * 8, ncclDouble, comm, h->stream));
+                }
+                LR_LAUNCH(k_reloc_unpack, blocks(static_cast<size_t>(m) * 8), 256, 0, h->stream, gather, m, c, world,
+                          h->d_poses_out.as<double>(), h->d_scores.as<double>());
+            }
+            LR_LAUNCH(k_reloc_scatter, g, 256, 0, h->stream, m, idx_r, h->d_poses_out.as<double>(), h->d_scores.as<double>(), r,
+                      h->d_stage_poses.as<double>(), h->d_stage_scores.as<double>(), h->d_stage_rounds.as<int>());
+            if (r + 1 == n_rounds) {
+                select_kth(m, 1u);
+                break;
+            }
+            select_kth(m, static_cast<unsigned int>(alive[r + 1]));
+            unsigned int* slot = h->d_stage_slot.as<unsigned int>();
+            LR_LAUNCH(k_select_flags, g, 256, 0, h->stream, keys, m, st, slot);
+            exclusive_scan_u32(slot, slot, m, nullptr, h->stream);
+            LR_LAUNCH(k_reloc_compact, g, 256, 0, h->stream, keys, m, st, slot, h->d_poses_out.as<double>(), idx_r, full,
+                      idx[(r + 1) & 1]);
         }
-        h->end_timing();
-        double b[8];
-        long long bi = 0;
-        LR_CUDA(cudaMemcpy(b, d_best, sizeof(b), cudaMemcpyDeviceToHost));
-        LR_CUDA(cudaMemcpy(&bi, d_best_idx, sizeof(bi), cudaMemcpyDeviceToHost));
-        if (best_idx) *best_idx = bi;
-        if (best_pose) std::memcpy(best_pose, b, 7 * sizeof(double));
-        if (best_score) *best_score = b[7];
-        if (scores) LR_CUDA(cudaMemcpy(scores, h->d_stage_scores.p, n_hyp * sizeof(double), cudaMemcpyDeviceToHost));
-        if (poses_out) LR_CUDA(cudaMemcpy(poses_out, h->d_stage_poses.p, n_hyp * 7 * sizeof(double), cudaMemcpyDeviceToHost));
-        if (rounds_out) LR_CUDA(cudaMemcpy(rounds_out, h->d_stage_rounds.p, n_hyp * sizeof(int32_t), cudaMemcpyDeviceToHost));
-        return LOCREG_OK;
+        LR_LAUNCH(k_reloc_best, 1, 32, 0, h->stream, st, n_rounds > 1 ? idx[(n_rounds - 1) & 1] : nullptr,
+                  h->d_stage_poses.as<double>(), h->d_stage_scores.as<double>(), d_best, d_best_idx);
+    }
+    h->end_timing();
+    double b[8];
+    long long bi = 0;
+    LR_CUDA(cudaMemcpy(b, d_best, sizeof(b), cudaMemcpyDeviceToHost));
+    LR_CUDA(cudaMemcpy(&bi, d_best_idx, sizeof(bi), cudaMemcpyDeviceToHost));
+    if (best_idx) *best_idx = bi;
+    if (best_pose) std::memcpy(best_pose, b, 7 * sizeof(double));
+    if (best_score) *best_score = b[7];
+    if (scores) LR_CUDA(cudaMemcpy(scores, h->d_stage_scores.p, n_hyp * sizeof(double), cudaMemcpyDeviceToHost));
+    if (poses_out) LR_CUDA(cudaMemcpy(poses_out, h->d_stage_poses.p, n_hyp * 7 * sizeof(double), cudaMemcpyDeviceToHost));
+    if (rounds_out) LR_CUDA(cudaMemcpy(rounds_out, h->d_stage_rounds.p, n_hyp * sizeof(int32_t), cudaMemcpyDeviceToHost));
+    return LOCREG_OK;
+}
+
+int locreg_relocalise_staged(locreg_handle* h, const float* src, size_t n, size_t stride, const double* poses_in, size_t n_hyp,
+                             const int32_t* trips, const int64_t* keep, int32_t n_rounds, double* best_pose, int64_t* best_idx,
+                             double* best_score, double* scores, double* poses_out, int32_t* rounds_out) {
+    const int rc = staged_check(src, n, stride, poses_in, n_hyp, trips, keep, n_rounds);
+    if (rc) return rc;
+    return guarded(h, [&]() {
+        return relocalise_staged_rounds(h, src, n, stride, poses_in, n_hyp, trips, keep, n_rounds, best_pose, best_idx,
+                                        best_score, scores, poses_out, rounds_out, 0u, 1u, nullptr);
+    });
+}
+
+// locreg_relocalise_staged over the handle's communicator (include/locreg.h); a one-rank communicator or none is the
+// single-GPU call itself.
+int locreg_relocalise_staged_sharded(locreg_handle* h, const float* src, size_t n, size_t stride, const double* poses_in,
+                                     size_t n_hyp, const int32_t* trips, const int64_t* keep, int32_t n_rounds,
+                                     double* best_pose, int64_t* best_idx, double* best_score, double* scores,
+                                     double* poses_out, int32_t* rounds_out) {
+    const int rc = staged_check(src, n, stride, poses_in, n_hyp, trips, keep, n_rounds);
+    if (rc) return rc;
+    return guarded(h, [&]() {
+        const bool shard = h->comm && h->comm_world > 1;
+        return relocalise_staged_rounds(h, src, n, stride, poses_in, n_hyp, trips, keep, n_rounds, best_pose, best_idx,
+                                        best_score, scores, poses_out, rounds_out,
+                                        shard ? static_cast<unsigned int>(h->comm_rank) : 0u,
+                                        shard ? static_cast<unsigned int>(h->comm_world) : 1u, shard ? h->comm : nullptr);
     });
 }
 

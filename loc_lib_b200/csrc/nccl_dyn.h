@@ -1,7 +1,8 @@
 // Run-time binding of NCCL for the multi-GPU entry points of the C ABI (locreg_comm_*, locreg_relocalise_sharded,
-// locreg_align_batch_sharded).  liblocreg.so carries no DT_NEEDED on libnccl: a single-GPU user (slam_demo's tracking
-// loop) needs no NCCL, and a process that already holds a copy (torch ships its own libnccl.so.2) must not get a
-// second one.  The first use looks for a loaded libnccl.so.2 (RTLD_NOLOAD), then for the system's.
+// locreg_relocalise_loam_sharded, locreg_relocalise_staged_sharded, locreg_align_batch_sharded).  liblocreg.so carries
+// no DT_NEEDED on libnccl: a single-GPU user (slam_demo's tracking loop) needs no NCCL, and a process that already holds
+// a copy (torch ships its own libnccl.so.2) must not get a second one.  The first use looks for a loaded libnccl.so.2
+// (RTLD_NOLOAD), then for the system's.
 #pragma once
 #include <dlfcn.h>
 #include <nccl.h>

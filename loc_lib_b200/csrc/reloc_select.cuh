@@ -1,4 +1,5 @@
-// Staged relocalisation (locreg_relocalise_staged): the cut between two rounds and the caller-order outputs.
+// Staged relocalisation (locreg_relocalise_staged[_sharded]): the cut between two rounds, the caller-order outputs, and
+// the deal and exchange of a round across ranks.
 // A round's m hypotheses sit at positions 0 .. m-1 in ascending original index.  Position p's key is
 // locreg_pack_score(score[p], p), so unsigned key order is (float32 score, original index) order, and the keys are
 // distinct.  The k survivors are the keys <= the k-th smallest key, which an MSB-first radix select finds 8 bits per
@@ -111,6 +112,43 @@ __global__ void k_reloc_best(const SelectState* __restrict__ st, const unsigned 
     for (int i = 0; i < 7; ++i) out[i] = all_poses[o * 7 + i];
     out[7] = all_scores[o];
     *out_idx = static_cast<long long>(o);
+}
+
+// ---- locreg_relocalise_staged_sharded: a round over `world` ranks ----------------------------------------------------
+// Rank q runs the round's positions q, q + world, q + 2 world, ... (m_q of them); its results travel as records of
+// 8 doubles (7 pose + score) in slab q of c = ceil(m / world) records, one ncclAllGather fills all world slabs on every
+// rank, and slab q record i is position q + i * world again.  Every rank then holds the whole round, as one GPU would.
+
+// One thread per double in all three (consecutive threads touch consecutive words): launch over m_q * 7, m_q * 8 and
+// m * 8 threads.
+
+// rank's share of the round's full pose array -> out (m_q poses)
+__global__ void k_reloc_deal(const double* __restrict__ poses, unsigned int m_q, unsigned int rank, unsigned int world,
+                             double* out) {
+    const size_t t = static_cast<size_t>(blockIdx.x) * blockDim.x + threadIdx.x;
+    if (t >= static_cast<size_t>(m_q) * 7) return;
+    const size_t i = t / 7, k = t % 7;
+    out[t] = poses[(rank + i * world) * 7 + k];
+}
+
+// the rank's m_q poses + scores -> its slab of records
+__global__ void k_reloc_pack(const double* __restrict__ poses, const double* __restrict__ scores, unsigned int m_q,
+                             double* slab) {
+    const size_t t = static_cast<size_t>(blockIdx.x) * blockDim.x + threadIdx.x;
+    if (t >= static_cast<size_t>(m_q) * 8) return;
+    const size_t i = t / 8, k = t % 8;
+    slab[t] = k < 7 ? poses[i * 7 + k] : scores[i];
+}
+
+// the gathered slabs (world * c records) -> the round's poses and scores at positions 0 .. m-1
+__global__ void k_reloc_unpack(const double* __restrict__ gather, unsigned int m, unsigned int c, unsigned int world,
+                               double* poses, double* scores) {
+    const size_t t = static_cast<size_t>(blockIdx.x) * blockDim.x + threadIdx.x;
+    if (t >= static_cast<size_t>(m) * 8) return;
+    const size_t p = t / 8, k = t % 8;
+    const double v = gather[((p % world) * c + p / world) * 8 + k];
+    if (k < 7) poses[p * 7 + k] = v;
+    else scores[p] = v;
 }
 
 }  // namespace locreg

@@ -172,6 +172,9 @@ class _Registration:
         after round r (keep has len(trips) - 1 entries; see locreg_relocalise_staged).  Returns (best_pose, best_idx,
         best_score, scores, poses, rounds): with want_all, every hypothesis's score and pose of the last round it ran and
         how many rounds it ran; otherwise the last three are None."""
+        return self._relocalise_staged("locreg_relocalise_staged", cloud, hypotheses, trips, keep, want_all)
+
+    def _relocalise_staged(self, symbol, cloud, hypotheses, trips, keep, want_all):
         a, n, s = _cloud(cloud)
         hyp = np.ascontiguousarray(hypotheses, np.float64).reshape(-1, 7)
         nh = hyp.shape[0]
@@ -185,12 +188,12 @@ class _Registration:
         scores = np.zeros(nh) if want_all else None
         poses = np.zeros((nh, 7)) if want_all else None
         rounds = np.zeros(nh, np.int32) if want_all else None
-        _lib.check(_lib.lib().locreg_relocalise_staged(self._h, a.ctypes.data, n, s, hyp.ctypes.data, nh, trips.ctypes.data,
-                                                       keep.ctypes.data if keep.size else None, trips.shape[0],
-                                                       best_pose.ctypes.data, C.byref(best_idx), C.byref(best_score),
-                                                       scores.ctypes.data if want_all else None,
-                                                       poses.ctypes.data if want_all else None,
-                                                       rounds.ctypes.data if want_all else None))
+        _lib.check(getattr(_lib.lib(), symbol)(self._h, a.ctypes.data, n, s, hyp.ctypes.data, nh, trips.ctypes.data,
+                      keep.ctypes.data if keep.size else None, trips.shape[0],
+                      best_pose.ctypes.data, C.byref(best_idx), C.byref(best_score),
+                      scores.ctypes.data if want_all else None,
+                      poses.ctypes.data if want_all else None,
+                      rounds.ctypes.data if want_all else None))
         return best_pose, int(best_idx.value), float(best_score.value), scores, poses, rounds
 
     # ---- multi-GPU: NCCL inside liblocreg.so (one process per GPU; see loc_lib_b200/dist.py for the torchrun plumbing) ----
@@ -224,6 +227,13 @@ class _Registration:
         _lib.check(_lib.lib().locreg_relocalise_sharded(self._h, a.ctypes.data, n, s, hyp.ctypes.data, hyp.shape[0],
                                                         best_pose.ctypes.data, C.byref(best_idx), C.byref(best_score)))
         return best_pose, int(best_idx.value), float(best_score.value)
+
+    def RelocaliseStagedSharded(self, cloud, hypotheses, trips, keep, want_all=False):
+        """RelocaliseStaged over all ranks of the handle's communicator (locreg_relocalise_staged_sharded): every rank
+        passes the same scan, hypotheses and schedule; each round's alive hypotheses are dealt over the ranks and
+        their results all-gathered on the handle's stream.  Returns the same 6-tuple as RelocaliseStaged, bit for bit
+        what one GPU returns, on every rank."""
+        return self._relocalise_staged("locreg_relocalise_staged_sharded", cloud, hypotheses, trips, keep, want_all)
 
     def ScanMatchBatchSharded(self, clouds, offsets, predict_poses, S_global):
         """This rank's block of a batch of S_global scans (block partition: shard_range); returns the poses and results
