@@ -289,6 +289,41 @@ int locreg_relocalise_loam_sharded(locreg_handle* surf, locreg_handle* edge, con
                                    size_t n_hyp, int32_t max_iteration, double eps, double* best_pose, int64_t* best_idx,
                                    double* best_score);
 
+/* Staged LOAM relocalisation: locreg_relocalise_staged's rounds over locreg_relocalise_loam's loop and score.  Round r
+ * runs locreg_relocalise_loam over the hypotheses still alive, with max_iteration = trips[r] and the caller's eps, from
+ * the poses the previous round left (round 0: poses_in); after it only the min(keep[r], alive) hypotheses with the
+ * smallest locreg_pack_score(score, original index) go on, in ascending original index.  The winner is the smallest key
+ * of the last round.  Poses are used as given in every round: the LOAM loop ignores zero_initial_translation.
+ * Each round is a fresh loop: only the pose is carried over, so round r of hypothesis i is bit for bit what
+ * locreg_relocalise_loam returns from that pose with max_iteration = trips[r].  The score is locreg_relocalise_loam's;
+ * trips[r] == 0 is a score-only round.  Neither handle's options are used for the schedule or changed.  All rounds are
+ * queued back to back on surf's stream (edge's stream joins it every round) and the call synchronises once.
+ *   trips      n_rounds entries >= 0
+ *   keep       n_rounds - 1 entries >= 1 (may be NULL when n_rounds == 1)
+ *   scores / poses_out / rounds_out (n_hyp, n_hyp * 7, n_hyp; each may be NULL): every hypothesis's score and pose of
+ *              the last round it ran, and how many rounds it ran (1 .. n_rounds)
+ *   best_pose  poses_out[best_idx] bit for bit; best_score its score
+ * locreg_last_timing(surf) covers the kernels of all rounds.  Arguments are checked before any device work: LOCREG_E_ARG
+ * for the handles and clouds as in locreg_relocalise_loam, a null poses_in, n_hyp == 0 or n_hyp >= 2^31, and the
+ * schedule as in locreg_relocalise_staged (n_rounds outside [1, 32], a null trips or trips[r] < 0, a null keep with
+ * n_rounds > 1, keep[r] < 1); LOCREG_E_STATE for a handle without a target. */
+int locreg_relocalise_loam_staged(locreg_handle* surf, locreg_handle* edge, const float* surf_xyz, size_t n_surf,
+                                  const float* edge_xyz, size_t n_edge, size_t stride_bytes, const double* poses_in,
+                                  size_t n_hyp, const int32_t* trips, const int64_t* keep, int32_t n_rounds, double eps,
+                                  double* best_pose, int64_t* best_idx, double* best_score, double* scores,
+                                  double* poses_out, int32_t* rounds_out);
+/* locreg_relocalise_loam_staged over all ranks of the SURF handle's communicator (the edge handle's is not used; none,
+ * or a one-rank communicator: it IS locreg_relocalise_loam_staged, with the same launches).  Every rank passes the same
+ * clouds, hypotheses and schedule.  Each round's alive hypotheses are dealt by position and exchanged with one in-place
+ * ncclAllGather of pose + score on surf's stream, as in locreg_relocalise_staged_sharded.  Every output is bit for bit
+ * what locreg_relocalise_loam_staged returns on one GPU, on every rank.  Argument errors as in
+ * locreg_relocalise_loam_staged; locreg_last_timing(surf) covers all rounds and their collectives. */
+int locreg_relocalise_loam_staged_sharded(locreg_handle* surf, locreg_handle* edge, const float* surf_xyz, size_t n_surf,
+                                          const float* edge_xyz, size_t n_edge, size_t stride_bytes,
+                                          const double* poses_in, size_t n_hyp, const int32_t* trips, const int64_t* keep,
+                                          int32_t n_rounds, double eps, double* best_pose, int64_t* best_idx,
+                                          double* best_score, double* scores, double* poses_out, int32_t* rounds_out);
+
 /* Batch offline mapping over all ranks (BASELINE config 4).  The batch has S_global scans; this rank owns the block
  * [lo, hi) = locreg_shard_range(S_global, rank, world) and passes ONLY that block: srcs / offsets (S_local + 1
  * entries, relative to srcs) / poses_in (S_local * 7) with S_local = hi - lo.  No collective on the data path; at the

@@ -22,7 +22,7 @@ SYMBOLS = [
     "locreg_comm_unique_id", "locreg_comm_init", "locreg_comm_destroy", "locreg_comm_info", "locreg_shard_range",
     "locreg_relocalise_sharded", "locreg_align_batch_sharded", "locreg_index_info", "locreg_align_loam",
     "locreg_align_loam_batch", "locreg_relocalise_loam", "locreg_relocalise_loam_sharded", "locreg_relocalise_staged",
-    "locreg_relocalise_staged_sharded",
+    "locreg_relocalise_staged_sharded", "locreg_relocalise_loam_staged", "locreg_relocalise_loam_staged_sharded",
 ]
 
 
@@ -67,6 +67,9 @@ def lib():
         L.locreg_align_loam_batch.argtypes = [vp, vp, vp, vp, vp, vp, sz, vp, sz, i32, C.c_double, vp, vp]
         L.locreg_relocalise_loam.argtypes = [vp, vp, vp, sz, vp, sz, sz, vp, sz, i32, C.c_double, vp, vp, vp, vp, vp]
         L.locreg_relocalise_loam_sharded.argtypes = [vp, vp, vp, sz, vp, sz, sz, vp, sz, i32, C.c_double, vp, vp, vp]
+        L.locreg_relocalise_loam_staged.argtypes = [vp, vp, vp, sz, vp, sz, sz, vp, sz, vp, vp, i32, C.c_double, vp, vp, vp,
+                                                    vp, vp, vp]
+        L.locreg_relocalise_loam_staged_sharded.argtypes = L.locreg_relocalise_loam_staged.argtypes
         L.locreg_knn.argtypes = [vp, vp, sz, sz, i32, vp]
         L.locreg_debug_points.argtypes = [vp, vp, sz, sz, vp, vp, vp]
         L.locreg_align_batch.argtypes = [vp, vp, vp, sz, vp, sz, vp, vp]

@@ -1529,6 +1529,8 @@ int locreg_relocalise(locreg_handle* h, const float* src, size_t n, size_t strid
     });
 }
 
+}  // extern "C"
+
 // The handle's loop options as they were, restored when the scope ends (also on an exception): the rounds of a staged
 // relocalisation set their own trip count and zero_initial_translation, and every later call must see the caller's.
 struct ScopedLoopOptions {
@@ -1544,12 +1546,8 @@ struct ScopedLoopOptions {
     ScopedLoopOptions& operator=(const ScopedLoopOptions&) = delete;
 };
 
-// Argument checks of locreg_relocalise_staged[_sharded], before any device work.
-static int staged_check(const float* src, size_t n, size_t stride, const double* poses_in, size_t n_hyp, const int32_t* trips,
-                        const int64_t* keep, int32_t n_rounds) {
-    const int rc = check_cloud_args(src, n, stride);
-    if (rc) return rc;
-    if (!poses_in || n_hyp == 0 || n_hyp >= (1ull << 31)) { g_last_error = "invalid hypotheses"; return LOCREG_E_ARG; }
+// The schedule checks of every staged relocalisation (ICP and LOAM), before any device work.
+static int schedule_check(const int32_t* trips, const int64_t* keep, int32_t n_rounds) {
     if (n_rounds < 1 || n_rounds > 32) { g_last_error = "n_rounds must be in [1, 32]"; return LOCREG_E_ARG; }
     if (!trips) { g_last_error = "invalid trips (null)"; return LOCREG_E_ARG; }
     for (int32_t r = 0; r < n_rounds; ++r)
@@ -1560,28 +1558,41 @@ static int staged_check(const float* src, size_t n, size_t stride, const double*
     return LOCREG_OK;
 }
 
-// Staged relocalisation (include/locreg.h) over `world` ranks of comm (world 1: comm unused): round r is relocalise_core
-// on the alive hypotheses with trips[r] trips; between rounds the survivors are cut on the device (reloc_select.cuh) and
-// their poses gathered into the next round's full pose array, so all rounds are queued back to back and the call
-// synchronises once.  Round r's positions map to original indices through d_stage_idx half (r & 1) (round 0: the
-// identity, no map).  The winner is the same select with k = 1 over the last round, so the cuts and the winner rank by
-// one key, locreg_pack_score's.
-// world 1: the full pose array is d_poses_in itself and relocalise_core runs all m alive hypotheses.  world > 1: it is
+// Argument checks of locreg_relocalise_staged[_sharded], before any device work.
+static int staged_check(const float* src, size_t n, size_t stride, const double* poses_in, size_t n_hyp, const int32_t* trips,
+                        const int64_t* keep, int32_t n_rounds) {
+    const int rc = check_cloud_args(src, n, stride);
+    if (rc) return rc;
+    if (!poses_in || n_hyp == 0 || n_hyp >= (1ull << 31)) { g_last_error = "invalid hypotheses"; return LOCREG_E_ARG; }
+    return schedule_check(trips, keep, n_rounds);
+}
+
+// The positions rank `rank` of `world` runs in a round of m alive hypotheses: rank, rank + world, ...
+static unsigned int dealt(unsigned int m, unsigned int rank, unsigned int world) {
+    return m > rank ? (m - rank + world - 1) / world : 0u;
+}
+
+// Staged relocalisation (include/locreg.h) over `world` ranks of comm (world 1: comm unused), on h's stream, with the
+// caller's cloud(s) already staged: run(r, m_q) queues round r on the m_q hypotheses whose poses are in h->d_poses_in
+// and leaves their poses and scores in h->d_poses_out / d_scores (relocalise_core for ICP / NDT, loam_relocalise_core
+// for LOAM).  Between rounds the survivors are cut on the device (reloc_select.cuh) and their poses gathered into the
+// next round's full pose array, so all rounds are queued back to back and the call synchronises once.  Round r's
+// positions map to original indices through d_stage_idx half (r & 1) (round 0: the identity, no map).  The winner is the
+// same select with k = 1 over the last round, so the cuts and the winner rank by one key, locreg_pack_score's.
+// world 1: the full pose array is d_poses_in itself and run() gets all m alive hypotheses.  world > 1: it is
 // d_stage_full; rank q deals itself positions q, q + world, ... into d_poses_in and runs those, and the round's results
 // come back to every rank through one ncclAllGather (k_reloc_pack / k_reloc_unpack) into d_poses_out / d_scores at all m
 // positions, as one GPU leaves them.  The cut and the winner then run redundantly on every rank over identical keys.
-static int relocalise_staged_rounds(locreg_handle* h, const float* src, size_t n, size_t stride, const double* poses_in,
-                                    size_t n_hyp, const int32_t* trips, const int64_t* keep, int32_t n_rounds,
-                                    double* best_pose, int64_t* best_idx, double* best_score, double* scores,
-                                    double* poses_out, int32_t* rounds_out, unsigned int rank, unsigned int world,
-                                    ncclComm_t comm) {
-    if (!h->has_target) { g_last_error = "SetInputTarget has not been called"; return LOCREG_E_STATE; }
+template <class Round>
+static int relocalise_staged_rounds(locreg_handle* h, const double* poses_in, size_t n_hyp, const int32_t* trips,
+                                    const int64_t* keep, int32_t n_rounds, double* best_pose, int64_t* best_idx,
+                                    double* best_score, double* scores, double* poses_out, int32_t* rounds_out,
+                                    unsigned int rank, unsigned int world, ncclComm_t comm, Round&& run) {
     NvtxRange nr("locreg:relocalise_staged");
     std::vector<size_t> alive(n_rounds);  // hypotheses in round r, known before anything runs
     alive[0] = n_hyp;
     for (int32_t r = 1; r < n_rounds; ++r) alive[r] = std::min<size_t>(static_cast<size_t>(keep[r - 1]), alive[r - 1]);
-    const float4* src4 = stage_cloud(h, src, n, stride, false);
-    // every per-hypothesis buffer at its full size before the first launch (relocalise_core's reserves are then no-ops)
+    // every per-hypothesis buffer at its full size before the first launch (the round's own reserves are then no-ops)
     h->d_poses_in.reserve(n_hyp * 7 * sizeof(double));
     h->d_poses_out.reserve(n_hyp * 7 * sizeof(double));
     h->d_results.reserve(n_hyp * sizeof(DevResult));
@@ -1611,7 +1622,6 @@ static int relocalise_staged_rounds(locreg_handle* h, const float* src, size_t n
     LR_CUDA(cudaMemsetAsync(hist, 0, kSelectBins * sizeof(unsigned int), h->stream));  // k_select_digit re-zeroes it
     h->begin_timing();
     {
-        ScopedLoopOptions saved(h);
         unsigned long long* keys = h->d_stage_keys.as<unsigned long long>();
         // st->prefix = the k-th smallest key of the round's m scores (in h->d_scores)
         const auto select_kth = [&](unsigned int m, unsigned int k) {
@@ -1627,18 +1637,16 @@ static int relocalise_staged_rounds(locreg_handle* h, const float* src, size_t n
             const unsigned int m = static_cast<unsigned int>(alive[r]);
             const unsigned int g = (m + 255) / 256;
             const unsigned int* idx_r = r == 0 ? nullptr : idx[r & 1];
-            h->opt.max_iteration = trips[r];
-            if (r > 0) h->opt.zero_initial_translation = 0;  // later rounds start from the pose as the last one left it
             if (world == 1) {
-                relocalise_core(h, src4, n, nullptr, m, 0u, 1u, false);
+                run(r, m);
             } else {
-                const unsigned int m_q = m > rank ? (m - rank + world - 1) / world : 0u, c = (m + world - 1) / world;
+                const unsigned int m_q = dealt(m, rank, world), c = (m + world - 1) / world;
                 double* gather = h->d_stage_gather.as<double>();
                 double* slab = gather + static_cast<size_t>(rank) * c * 8;
                 const auto blocks = [](size_t words) { return static_cast<unsigned int>((words + 255) / 256); };  // a thread per double
                 if (m_q) LR_LAUNCH(k_reloc_deal, blocks(static_cast<size_t>(m_q) * 7), 256, 0, h->stream, full, m_q, rank, world,
                                    h->d_poses_in.as<double>());
-                relocalise_core(h, src4, n, nullptr, m_q, 0u, 1u, false);
+                run(r, m_q);
                 if (m_q) LR_LAUNCH(k_reloc_pack, blocks(static_cast<size_t>(m_q) * 8), 256, 0, h->stream, h->d_poses_out.as<double>(),
                                    h->d_scores.as<double>(), m_q, slab);
                 {
@@ -1678,14 +1686,33 @@ static int relocalise_staged_rounds(locreg_handle* h, const float* src, size_t n
     return LOCREG_OK;
 }
 
+// The rounds of locreg_relocalise_staged[_sharded]: relocalise_core with the round's trip count set on the handle, and
+// zero_initial_translation cleared after round 0 (later rounds start from the pose as the last one left it).
+static int relocalise_staged_icp(locreg_handle* h, const float* src, size_t n, size_t stride, const double* poses_in,
+                                 size_t n_hyp, const int32_t* trips, const int64_t* keep, int32_t n_rounds, double* best_pose,
+                                 int64_t* best_idx, double* best_score, double* scores, double* poses_out,
+                                 int32_t* rounds_out, unsigned int rank, unsigned int world, ncclComm_t comm) {
+    if (!h->has_target) { g_last_error = "SetInputTarget has not been called"; return LOCREG_E_STATE; }
+    const float4* src4 = stage_cloud(h, src, n, stride, false);
+    ScopedLoopOptions saved(h);
+    return relocalise_staged_rounds(h, poses_in, n_hyp, trips, keep, n_rounds, best_pose, best_idx, best_score, scores,
+                                    poses_out, rounds_out, rank, world, comm, [&](int32_t r, unsigned int m_q) {
+                                        h->opt.max_iteration = trips[r];
+                                        if (r > 0) h->opt.zero_initial_translation = 0;
+                                        relocalise_core(h, src4, n, nullptr, m_q, 0u, 1u, false);
+                                    });
+}
+
+extern "C" {
+
 int locreg_relocalise_staged(locreg_handle* h, const float* src, size_t n, size_t stride, const double* poses_in, size_t n_hyp,
                              const int32_t* trips, const int64_t* keep, int32_t n_rounds, double* best_pose, int64_t* best_idx,
                              double* best_score, double* scores, double* poses_out, int32_t* rounds_out) {
     const int rc = staged_check(src, n, stride, poses_in, n_hyp, trips, keep, n_rounds);
     if (rc) return rc;
     return guarded(h, [&]() {
-        return relocalise_staged_rounds(h, src, n, stride, poses_in, n_hyp, trips, keep, n_rounds, best_pose, best_idx,
-                                        best_score, scores, poses_out, rounds_out, 0u, 1u, nullptr);
+        return relocalise_staged_icp(h, src, n, stride, poses_in, n_hyp, trips, keep, n_rounds, best_pose, best_idx,
+                                     best_score, scores, poses_out, rounds_out, 0u, 1u, nullptr);
     });
 }
 
@@ -1699,10 +1726,10 @@ int locreg_relocalise_staged_sharded(locreg_handle* h, const float* src, size_t 
     if (rc) return rc;
     return guarded(h, [&]() {
         const bool shard = h->comm && h->comm_world > 1;
-        return relocalise_staged_rounds(h, src, n, stride, poses_in, n_hyp, trips, keep, n_rounds, best_pose, best_idx,
-                                        best_score, scores, poses_out, rounds_out,
-                                        shard ? static_cast<unsigned int>(h->comm_rank) : 0u,
-                                        shard ? static_cast<unsigned int>(h->comm_world) : 1u, shard ? h->comm : nullptr);
+        return relocalise_staged_icp(h, src, n, stride, poses_in, n_hyp, trips, keep, n_rounds, best_pose, best_idx,
+                                     best_score, scores, poses_out, rounds_out,
+                                     shard ? static_cast<unsigned int>(h->comm_rank) : 0u,
+                                     shard ? static_cast<unsigned int>(h->comm_world) : 1u, shard ? h->comm : nullptr);
     });
 }
 
@@ -1838,16 +1865,29 @@ int locreg_relocalise_sharded(locreg_handle* h, const float* src, size_t n, size
     });
 }
 
+// The wave size of a LOAM relocalisation of n_local hypotheses, with the scratch both halves share reserved for it: the
+// states (one per hypothesis, both jobs point at them) and the halves' records, which k_loam_solve writes.  One wave
+// size serves both halves: its memory is sized by n_s + n_e points per hypothesis, its 32-bit scratch rows by the
+// larger half.
+static size_t loam_reloc_reserve(locreg_handle* surf, size_t n_local, size_t n_s, size_t n_e) {
+    const size_t wave = reloc_wave_size(n_local, n_s + n_e, std::max(n_s, n_e), 5);
+    surf->d_states.reserve(wave * sizeof(AlignState));
+    surf->d_loam.reserve(2 * wave * sizeof(DevResult));
+    return wave;
+}
+
 // LOAM relocalisation: n_local hypotheses (host, 7 doubles each) of ONE surf / edge scan.  Each runs the LOAM loop of
 // locreg_align_loam from its pose; then the score pass evaluates both halves once more at the final pose and an
 // evaluation-only k_loam_solve leaves the summed counts in the loop's result, from which k_score_argmin takes
 // (sum_sq_surf + sum_sq_edge) / (n_inlier_surf + n_inlier_edge), +inf for a singular summed H or no inlier.  Poses,
 // results and scores land in surf's d_poses_out / d_results / d_scores; returns the device key of the best (index
-// index_base + i * index_stride).  Queued on surf's stream, which joins edge's; nothing is synchronised.  One wave size
-// serves both halves: its memory is sized by n_s + n_e points per hypothesis, its 32-bit scratch rows by the larger half.
+// index_base + i * index_stride).  Queued on surf's stream, which joins edge's; nothing is synchronised.
+// poses_in == nullptr: surf->d_poses_in already holds the poses (a round of locreg_relocalise_loam_staged).
+// begin_timing: surf's timing starts here, after the poses' upload; a staged call starts it once before its first round.
 static unsigned long long* loam_relocalise_core(locreg_handle* surf, locreg_handle* edge, const float4* src_s, size_t n_s,
                                                 const float4* src_e, size_t n_e, const double* poses_in, size_t n_local,
-                                                int32_t max_iteration, double eps, unsigned int index_base, unsigned int index_stride) {
+                                                int32_t max_iteration, double eps, unsigned int index_base, unsigned int index_stride,
+                                                bool begin_timing) {
     NvtxRange r("locreg:relocalise_loam");
     const size_t cap = std::max<size_t>(n_local, 1);
     surf->d_poses_in.reserve(cap * 7 * sizeof(double));
@@ -1856,12 +1896,11 @@ static unsigned long long* loam_relocalise_core(locreg_handle* surf, locreg_hand
     surf->d_scores.reserve(cap * sizeof(double));
     surf->d_misc.reserve(64);
     unsigned long long* d_key = reinterpret_cast<unsigned long long*>(surf->d_misc.as<unsigned char>() + 32);
-    if (n_local) LR_CUDA(cudaMemcpyAsync(surf->d_poses_in.p, poses_in, n_local * 7 * sizeof(double), cudaMemcpyHostToDevice, surf->stream));
-    surf->begin_timing();
+    if (n_local && poses_in)
+        LR_CUDA(cudaMemcpyAsync(surf->d_poses_in.p, poses_in, n_local * 7 * sizeof(double), cudaMemcpyHostToDevice, surf->stream));
+    if (begin_timing) surf->begin_timing();
     if (n_local) {
-        const size_t wave = reloc_wave_size(n_local, n_s + n_e, std::max(n_s, n_e), 5);
-        surf->d_states.reserve(wave * sizeof(AlignState));
-        surf->d_loam.reserve(2 * wave * sizeof(DevResult));  // the halves' own records, which k_loam_solve writes
+        const size_t wave = loam_reloc_reserve(surf, n_local, n_s, n_e);
         for (size_t w0 = 0; w0 < n_local; w0 += wave) {
             const unsigned int W = static_cast<unsigned int>(std::min(wave, n_local - w0));
             const IcpJob js = hypothesis_job(src_s, n_s, W, surf->d_states.as<AlignState>());
@@ -1905,7 +1944,7 @@ int locreg_relocalise_loam(locreg_handle* surf, locreg_handle* edge, const float
         if (st) return st;
         const float4* src_s = stage_cloud(surf, surf_xyz, n_surf, stride, false);
         const float4* src_e = stage_cloud(edge, edge_xyz, n_edge, stride, false);
-        unsigned long long* d_key = loam_relocalise_core(surf, edge, src_s, n_surf, src_e, n_edge, poses_in, n_hyp, max_iteration, eps, 0u, 1u);
+        unsigned long long* d_key = loam_relocalise_core(surf, edge, src_s, n_surf, src_e, n_edge, poses_in, n_hyp, max_iteration, eps, 0u, 1u, true);
         surf->end_timing();
         cudaStream_t const s = surf->stream;
         surf->h_small.reserve(4096);
@@ -1937,9 +1976,71 @@ int locreg_relocalise_loam_sharded(locreg_handle* surf, locreg_handle* edge, con
         relocalise_exchange(surf, poses_in, n_hyp, best_pose, best_idx, best_score,
                             [&](const double* mine, size_t n_local, unsigned int rank, unsigned int world) {
                                 return loam_relocalise_core(surf, edge, src_s, n_surf, src_e, n_edge, mine, n_local, max_iteration, eps,
-                                                            rank, world);
+                                                            rank, world, true);
                             });
         return LOCREG_OK;
+    });
+}
+
+// Argument checks of locreg_relocalise_loam_staged[_sharded]: locreg_relocalise_loam's, then the schedule's.
+static int loam_staged_check(const locreg_handle* surf, const locreg_handle* edge, const float* surf_xyz, size_t n_surf,
+                             const float* edge_xyz, size_t n_edge, size_t stride, const double* poses_in, size_t n_hyp,
+                             const int32_t* trips, const int64_t* keep, int32_t n_rounds) {
+    const int rc = loam_relocalise_check(surf, edge, surf_xyz, n_surf, edge_xyz, n_edge, stride, poses_in, n_hyp);
+    if (rc) return rc;
+    return schedule_check(trips, keep, n_rounds);
+}
+
+// The rounds of locreg_relocalise_loam_staged[_sharded]: loam_relocalise_core with trips[r] trips and the caller's eps,
+// on surf's stream and surf's staged buffers.  The handles' options are not touched.
+static int relocalise_loam_staged(locreg_handle* surf, locreg_handle* edge, const float* surf_xyz, size_t n_surf,
+                                  const float* edge_xyz, size_t n_edge, size_t stride, const double* poses_in, size_t n_hyp,
+                                  const int32_t* trips, const int64_t* keep, int32_t n_rounds, double eps, double* best_pose,
+                                  int64_t* best_idx, double* best_score, double* scores, double* poses_out,
+                                  int32_t* rounds_out, unsigned int rank, unsigned int world, ncclComm_t comm) {
+    const int st = loam_prepare(surf, edge);
+    if (st) return st;
+    const float4* src_s = stage_cloud(surf, surf_xyz, n_surf, stride, false);
+    const float4* src_e = stage_cloud(edge, edge_xyz, n_edge, stride, false);
+    // round 0 has the most hypotheses: the scratch the halves share is sized for its wave before the first launch, so
+    // that round 0's own reserve does not grow (free and reallocate) a buffer once the rounds are being queued
+    if (const unsigned int m_q0 = dealt(static_cast<unsigned int>(n_hyp), rank, world)) loam_reloc_reserve(surf, m_q0, n_surf, n_edge);
+    return relocalise_staged_rounds(surf, poses_in, n_hyp, trips, keep, n_rounds, best_pose, best_idx, best_score, scores,
+                                    poses_out, rounds_out, rank, world, comm, [&](int32_t r, unsigned int m_q) {
+                                        loam_relocalise_core(surf, edge, src_s, n_surf, src_e, n_edge, nullptr, m_q, trips[r],
+                                                             eps, 0u, 1u, false);
+                                    });
+}
+
+int locreg_relocalise_loam_staged(locreg_handle* surf, locreg_handle* edge, const float* surf_xyz, size_t n_surf,
+                                  const float* edge_xyz, size_t n_edge, size_t stride, const double* poses_in, size_t n_hyp,
+                                  const int32_t* trips, const int64_t* keep, int32_t n_rounds, double eps, double* best_pose,
+                                  int64_t* best_idx, double* best_score, double* scores, double* poses_out,
+                                  int32_t* rounds_out) {
+    const int rc = loam_staged_check(surf, edge, surf_xyz, n_surf, edge_xyz, n_edge, stride, poses_in, n_hyp, trips, keep, n_rounds);
+    if (rc) return rc;
+    return guarded(surf, [&]() {
+        return relocalise_loam_staged(surf, edge, surf_xyz, n_surf, edge_xyz, n_edge, stride, poses_in, n_hyp, trips, keep,
+                                      n_rounds, eps, best_pose, best_idx, best_score, scores, poses_out, rounds_out, 0u, 1u,
+                                      nullptr);
+    });
+}
+
+// locreg_relocalise_loam_staged over the surf handle's communicator (include/locreg.h); a one-rank communicator or none
+// is the single-GPU call itself.  The edge handle's communicator is not used.
+int locreg_relocalise_loam_staged_sharded(locreg_handle* surf, locreg_handle* edge, const float* surf_xyz, size_t n_surf,
+                                          const float* edge_xyz, size_t n_edge, size_t stride, const double* poses_in,
+                                          size_t n_hyp, const int32_t* trips, const int64_t* keep, int32_t n_rounds,
+                                          double eps, double* best_pose, int64_t* best_idx, double* best_score,
+                                          double* scores, double* poses_out, int32_t* rounds_out) {
+    const int rc = loam_staged_check(surf, edge, surf_xyz, n_surf, edge_xyz, n_edge, stride, poses_in, n_hyp, trips, keep, n_rounds);
+    if (rc) return rc;
+    return guarded(surf, [&]() {
+        const bool shard = surf->comm && surf->comm_world > 1;
+        return relocalise_loam_staged(surf, edge, surf_xyz, n_surf, edge_xyz, n_edge, stride, poses_in, n_hyp, trips, keep,
+                                      n_rounds, eps, best_pose, best_idx, best_score, scores, poses_out, rounds_out,
+                                      shard ? static_cast<unsigned int>(surf->comm_rank) : 0u,
+                                      shard ? static_cast<unsigned int>(surf->comm_world) : 1u, shard ? surf->comm : nullptr);
     });
 }
 

@@ -85,6 +85,15 @@ def _pose(p):
     return p
 
 
+def _schedule(trips, keep):
+    """(trips int32, keep int64) of a staged relocalisation; keep has len(trips) - 1 entries."""
+    trips = np.ascontiguousarray(trips, np.int32).reshape(-1)
+    keep = np.ascontiguousarray([] if keep is None else keep, np.int64).reshape(-1)
+    if keep.shape[0] != max(trips.shape[0] - 1, 0):
+        raise ValueError("keep must have len(trips) - 1 entries")
+    return trips, keep
+
+
 class _Registration:
     """Common C-ABI plumbing; subclasses only build the options."""
 
@@ -178,10 +187,7 @@ class _Registration:
         a, n, s = _cloud(cloud)
         hyp = np.ascontiguousarray(hypotheses, np.float64).reshape(-1, 7)
         nh = hyp.shape[0]
-        trips = np.ascontiguousarray(trips, np.int32).reshape(-1)
-        keep = np.ascontiguousarray([] if keep is None else keep, np.int64).reshape(-1)
-        if keep.shape[0] != max(trips.shape[0] - 1, 0):
-            raise ValueError("keep must have len(trips) - 1 entries")
+        trips, keep = _schedule(trips, keep)
         best_pose = np.zeros(7)
         best_idx = C.c_int64(-1)
         best_score = C.c_double(np.inf)
@@ -469,6 +475,39 @@ class LoamRegistration:
                                                              s_s, hyp.ctypes.data, hyp.shape[0], self.max_iteration, self.eps,
                                                              best_pose.ctypes.data, C.byref(best_idx), C.byref(best_score)))
         return best_pose, int(best_idx.value), float(best_score.value)
+
+    def RelocaliseStaged(self, surf_cloud, edge_cloud, hypotheses, trips, keep, want_all=False):
+        """Relocalise in len(trips) rounds of trips[r] LOAM trips (eps: self.eps), keeping the keep[r] best-scoring
+        hypotheses after round r (locreg_relocalise_loam_staged; self.max_iteration is not used).  Returns (best_pose,
+        best_idx, best_score, scores, poses, rounds) as IcpRegistration.RelocaliseStaged."""
+        return self._relocalise_staged("locreg_relocalise_loam_staged", surf_cloud, edge_cloud, hypotheses, trips, keep,
+                                       want_all)
+
+    def RelocaliseStagedSharded(self, surf_cloud, edge_cloud, hypotheses, trips, keep, want_all=False):
+        """RelocaliseStaged over all ranks of the surf handle's communicator (locreg_relocalise_loam_staged_sharded):
+        every rank passes the same clouds, hypotheses and schedule.  Returns the same 6-tuple as RelocaliseStaged, bit
+        for bit what one GPU returns, on every rank."""
+        return self._relocalise_staged("locreg_relocalise_loam_staged_sharded", surf_cloud, edge_cloud, hypotheses, trips,
+                                       keep, want_all)
+
+    def _relocalise_staged(self, symbol, surf_cloud, edge_cloud, hypotheses, trips, keep, want_all):
+        a, n_s, s_s, b, n_e = self._clouds(surf_cloud, edge_cloud)
+        hyp = np.ascontiguousarray(hypotheses, np.float64).reshape(-1, 7)
+        nh = hyp.shape[0]
+        trips, keep = _schedule(trips, keep)
+        best_pose = np.zeros(7)
+        best_idx = C.c_int64(-1)
+        best_score = C.c_double(np.inf)
+        scores = np.zeros(nh) if want_all else None
+        poses = np.zeros((nh, 7)) if want_all else None
+        rounds = np.zeros(nh, np.int32) if want_all else None
+        _lib.check(getattr(_lib.lib(), symbol)(self.surf._h, self.edge._h, a.ctypes.data, n_s, b.ctypes.data, n_e, s_s,
+                      hyp.ctypes.data, nh, trips.ctypes.data, keep.ctypes.data if keep.size else None, trips.shape[0],
+                      self.eps, best_pose.ctypes.data, C.byref(best_idx), C.byref(best_score),
+                      scores.ctypes.data if want_all else None,
+                      poses.ctypes.data if want_all else None,
+                      rounds.ctypes.data if want_all else None))
+        return best_pose, int(best_idx.value), float(best_score.value), scores, poses, rounds
 
     # the communicator of the sharded relocalisation is the surf handle's (loc_lib_b200.dist.comm_init works unchanged)
     CommUniqueId = staticmethod(_Registration.CommUniqueId)
