@@ -153,6 +153,24 @@ int locreg_align_loam(locreg_handle* surf, locreg_handle* edge, const float* sur
 int locreg_align_loam_batch(locreg_handle* surf, locreg_handle* edge, const float* surf_xyz, const int64_t* surf_offsets,
                             const float* edge_xyz, const int64_t* edge_offsets, size_t stride_bytes, const double* poses_in,
                             size_t S, int32_t max_iteration, double eps, double* poses_out, locreg_result* results);
+/* locreg_align_loam_batch over all ranks of the SURF handle's communicator (the edge handle's is not used; none, or a
+ * one-rank communicator: it IS locreg_align_loam_batch, with the same launches and no NCCL call).  The batch has
+ * S_global scans; this rank owns the block [lo, hi) = locreg_shard_range(S_global, rank, world) and passes ONLY that
+ * block, as in locreg_align_batch_sharded: surf_offsets / edge_offsets (S_local + 1 entries each, relative to their
+ * cloud pointer) and poses_in (S_local * 7) with S_local = hi - lo.  EVERY rank passes the same S_global,
+ * max_iteration and eps.  A rank may own no scan (S_global < world): it runs no registration but joins the exchange,
+ * and may pass NULL offsets and poses_in.  No collective on the data path; at the end, on surf's stream, each block's
+ * poses, loop results and half records (200 bytes per scan) reach every rank with one grouped ncclBroadcast per rank
+ * block (an all-gather with ragged counts).  poses_out (S_global * 7, always written) and results (2 * S_global
+ * entries or NULL, [2s] surf and [2s+1] edge as in locreg_align_loam_batch) are complete on every rank and bit for bit
+ * what locreg_align_loam_batch returns on one GPU for the whole batch.  Arguments are checked before any device work
+ * and any collective (LOCREG_E_ARG: handles as in locreg_align_loam, S_global >= 2^31, S_local not this rank's block,
+ * this block's offsets negative or decreasing, stride or pointers, a null poses_out; LOCREG_E_STATE: a handle
+ * without a target).  S_global == 0 does nothing.  locreg_last_timing(surf) covers the kernels and the exchange. */
+int locreg_align_loam_batch_sharded(locreg_handle* surf, locreg_handle* edge, const float* surf_xyz,
+                                    const int64_t* surf_offsets, const float* edge_xyz, const int64_t* edge_offsets,
+                                    size_t stride_bytes, const double* poses_in, size_t S_local, size_t S_global,
+                                    int32_t max_iteration, double eps, double* poses_out, locreg_result* results);
 
 /* Parity probe for SearchPointInterface::FindNearstPoints (search_point_interface.h:9-24; kdtree.cpp:272-283):
  * exact k-NN (k = 1 or 5) under the total order (float32 dis2, index); idx is nq*k, -1 padded. ICP handles only.

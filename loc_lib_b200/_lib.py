@@ -23,6 +23,7 @@ SYMBOLS = [
     "locreg_relocalise_sharded", "locreg_align_batch_sharded", "locreg_index_info", "locreg_align_loam",
     "locreg_align_loam_batch", "locreg_relocalise_loam", "locreg_relocalise_loam_sharded", "locreg_relocalise_staged",
     "locreg_relocalise_staged_sharded", "locreg_relocalise_loam_staged", "locreg_relocalise_loam_staged_sharded",
+    "locreg_align_loam_batch_sharded",
 ]
 
 
@@ -65,6 +66,7 @@ def lib():
         L.locreg_compute_hb.argtypes = [vp, vp, sz, sz, vp, vp, vp, C.POINTER(Result)]
         L.locreg_align_loam.argtypes = [vp, vp, vp, sz, vp, sz, sz, vp, i32, C.c_double, vp, vp]
         L.locreg_align_loam_batch.argtypes = [vp, vp, vp, vp, vp, vp, sz, vp, sz, i32, C.c_double, vp, vp]
+        L.locreg_align_loam_batch_sharded.argtypes = [vp, vp, vp, vp, vp, vp, sz, vp, sz, sz, i32, C.c_double, vp, vp]
         L.locreg_relocalise_loam.argtypes = [vp, vp, vp, sz, vp, sz, sz, vp, sz, i32, C.c_double, vp, vp, vp, vp, vp]
         L.locreg_relocalise_loam_sharded.argtypes = [vp, vp, vp, sz, vp, sz, sz, vp, sz, i32, C.c_double, vp, vp, vp]
         L.locreg_relocalise_loam_staged.argtypes = [vp, vp, vp, sz, vp, sz, sz, vp, sz, vp, vp, i32, C.c_double, vp, vp, vp,

@@ -994,9 +994,10 @@ static IcpJob loam_half_job(locreg_handle* h, const LoamHalf& c, const float4* s
     return job;
 }
 
-// locreg_align_loam (S = 1, no offsets) and locreg_align_loam_batch: S independent LOAM loops in one.  The states live
-// with the surf job (the edge job points at them); surf->d_loam holds the poses, the loop results and the halves'
-// records, copied back in one piece through surf->h_out.
+// locreg_align_loam (S = 1, no offsets), locreg_align_loam_batch and each rank's block of
+// locreg_align_loam_batch_sharded: S independent LOAM loops in one.  The states live with the surf job (the edge job
+// points at them); surf->d_loam holds the poses, the loop results and the halves' records, copied back in one piece
+// through surf->h_out.
 static int loam_prepare(locreg_handle* surf, const locreg_handle* edge) {
     if (!surf->has_target || !edge->has_target) {
         g_last_error = surf->has_target ? "SetInputTarget has not been called on the edge handle"
@@ -1008,20 +1009,26 @@ static int loam_prepare(locreg_handle* surf, const locreg_handle* edge) {
     return LOCREG_OK;
 }
 
-static int loam_align(locreg_handle* surf, locreg_handle* edge, const LoamHalf& cs, const LoamHalf& ce, size_t stride,
-                      const double* poses_in, size_t S, int32_t max_iteration, double eps, double* poses_out, locreg_result* results) {
-    const int rc = loam_prepare(surf, edge);
-    if (rc) return rc;
+// The byte layout of d_loam / h_out for S scans: [S x 7 poses][S loop results][2S halves]
+struct LoamLayout {
+    size_t res_off, half_off, bytes;
+    explicit LoamLayout(size_t S)
+        : res_off(S * 7 * sizeof(double)), half_off(res_off + S * sizeof(DevResult)), bytes(half_off + 2 * S * sizeof(DevResult)) {}
+};
+
+// Queues the S > 0 LOAM loops on surf's stream, which joins edge's; the results are left in surf->d_loam.  surf's
+// timing starts after the uploads.
+static void loam_queue(locreg_handle* surf, locreg_handle* edge, const LoamHalf& cs, const LoamHalf& ce, size_t stride,
+                       const double* poses_in, size_t S, int32_t max_iteration, double eps) {
     const unsigned int Su = static_cast<unsigned int>(S);
-    // d_loam / h_out: [S x 7 poses][S loop results][2S halves]
-    const size_t res_off = S * 7 * sizeof(double), half_off = res_off + S * sizeof(DevResult), bytes = half_off + 2 * S * sizeof(DevResult);
-    surf->d_loam.reserve(bytes);
-    surf->h_out.reserve(bytes);
+    const LoamLayout lay(S);
+    surf->d_loam.reserve(lay.bytes);
+    surf->h_out.reserve(lay.bytes);
     unsigned char* const d = surf->d_loam.as<unsigned char>();
     unsigned char* const hb = surf->h_out.as<unsigned char>();
     double* const d_poses = reinterpret_cast<double*>(d);
-    DevResult* const d_res = reinterpret_cast<DevResult*>(d + res_off);
-    DevResult* const d_half = reinterpret_cast<DevResult*>(d + half_off);
+    DevResult* const d_res = reinterpret_cast<DevResult*>(d + lay.res_off);
+    DevResult* const d_half = reinterpret_cast<DevResult*>(d + lay.half_off);
     const float4* src_s = loam_stage_half(surf, cs, stride, S);
     const float4* src_e = loam_stage_half(edge, ce, stride, S);
     std::memcpy(hb, poses_in, S * 7 * sizeof(double));
@@ -1035,12 +1042,21 @@ static int loam_align(locreg_handle* surf, locreg_handle* edge, const LoamHalf& 
     LR_LAUNCH(k_states_init, (Su + 255) / 256, 256, 0, surf->stream, d_poses, Su, max_iteration, 0, js.states);
     loam_run_loop(surf, edge, js, je, max_iteration, eps, d_half);
     LR_LAUNCH(k_states_export, (Su + 255) / 256, 256, 0, surf->stream, js.states, Su, d_poses, d_res);
-    LR_CUDA(cudaMemcpyAsync(hb, d, bytes, cudaMemcpyDeviceToHost, surf->stream));
-    surf->end_timing();  // synchronises surf's stream, which has joined edge's
+}
+
+// Copies S scans' LoamLayout at device address d back through surf->h_out, ends surf's timing (which synchronises its
+// stream) and writes poses_out and the (surf, edge) result pairs: each half's last evaluation with the loop's
+// bookkeeping.
+static void loam_copy_back(locreg_handle* surf, const unsigned char* d, size_t S, double* poses_out, locreg_result* results) {
+    const LoamLayout lay(S);
+    surf->h_out.reserve(lay.bytes);
+    unsigned char* const hb = surf->h_out.as<unsigned char>();
+    LR_CUDA(cudaMemcpyAsync(hb, d, lay.bytes, cudaMemcpyDeviceToHost, surf->stream));
+    surf->end_timing();
     std::memcpy(poses_out, hb, S * 7 * sizeof(double));
-    const DevResult* hr = reinterpret_cast<const DevResult*>(hb + res_off);
-    const DevResult* hh = reinterpret_cast<const DevResult*>(hb + half_off);
-    for (size_t i = 0; results && i < 2 * S; ++i) {  // the loop's bookkeeping, the half's last evaluation
+    const DevResult* hr = reinterpret_cast<const DevResult*>(hb + lay.res_off);
+    const DevResult* hh = reinterpret_cast<const DevResult*>(hb + lay.half_off);
+    for (size_t i = 0; results && i < 2 * S; ++i) {
         DevResult r = hh[i];
         const DevResult& loop = hr[i / 2];
         r.iters = loop.iters;
@@ -1049,6 +1065,14 @@ static int loam_align(locreg_handle* surf, locreg_handle* edge, const LoamHalf& 
         r.pose_written = loop.pose_written;
         fill_result(results + i, r);
     }
+}
+
+static int loam_align(locreg_handle* surf, locreg_handle* edge, const LoamHalf& cs, const LoamHalf& ce, size_t stride,
+                      const double* poses_in, size_t S, int32_t max_iteration, double eps, double* poses_out, locreg_result* results) {
+    const int rc = loam_prepare(surf, edge);
+    if (rc) return rc;
+    loam_queue(surf, edge, cs, ce, stride, poses_in, S, max_iteration, eps);
+    loam_copy_back(surf, surf->d_loam.as<unsigned char>(), S, poses_out, results);
     return LOCREG_OK;
 }
 
@@ -1082,6 +1106,65 @@ int locreg_align_loam_batch(locreg_handle* surf, locreg_handle* edge, const floa
     if (rc) return rc;
     if (!poses_in || !poses_out) { g_last_error = "null pose"; return LOCREG_E_ARG; }
     return guarded(surf, [&]() { return loam_align(surf, edge, cs, ce, stride, poses_in, S, max_iteration, eps, poses_out, results); });
+}
+
+// locreg_align_loam_batch over the surf handle's communicator (include/locreg.h); none, or a one-rank one, is
+// locreg_align_loam_batch itself.  The edge handle's communicator is not used.
+int locreg_align_loam_batch_sharded(locreg_handle* surf, locreg_handle* edge, const float* surf_xyz, const int64_t* surf_offsets,
+                                    const float* edge_xyz, const int64_t* edge_offsets, size_t stride, const double* poses_in,
+                                    size_t S_local, size_t S_global, int32_t max_iteration, double eps, double* poses_out,
+                                    locreg_result* results) {
+    int rc = loam_check_handles(surf, edge);
+    if (rc) return rc;
+    if (S_global >= (1ull << 31)) { g_last_error = "too many scans"; return LOCREG_E_ARG; }
+    size_t lo = 0, hi = 0;
+    locreg_shard_range(S_global, surf->comm_rank, surf->comm_world, &lo, &hi);
+    if (S_local != hi - lo) { g_last_error = "S_local must be this rank's block of locreg_shard_range(S_global, rank, world)"; return LOCREG_E_ARG; }
+    if (S_global == 0) return LOCREG_OK;
+    const LoamHalf cs{surf_xyz, surf_offsets, 0}, ce{edge_xyz, edge_offsets, 0};
+    if (S_local) {
+        rc = loam_check_half(cs, stride, S_local, "surf");
+        if (rc) return rc;
+        rc = loam_check_half(ce, stride, S_local, "edge");
+        if (rc) return rc;
+    }
+    if ((S_local && !poses_in) || !poses_out) { g_last_error = "null pose"; return LOCREG_E_ARG; }
+    return guarded(surf, [&]() {
+        if (!surf->comm || surf->comm_world == 1)
+            return loam_align(surf, edge, cs, ce, stride, poses_in, S_global, max_iteration, eps, poses_out, results);
+        const int st = loam_prepare(surf, edge);
+        if (st) return st;
+        // the whole batch's LoamLayout is gathered in d_gather_pose; both buffers are sized before the first launch
+        const LoamLayout gl(S_global), ll(S_local);
+        surf->d_gather_pose.reserve(gl.bytes);
+        surf->h_out.reserve(gl.bytes);
+        if (S_local) loam_queue(surf, edge, cs, ce, stride, poses_in, S_local, max_iteration, eps);
+        else surf->begin_timing();
+        // exchange on surf's stream, which has joined edge's: each rank block's three sections into the global arrays
+        // (a ragged all-gather = one grouped broadcast per rank block)
+        const unsigned char* const dl = surf->d_loam.as<unsigned char>();
+        unsigned char* const dg = surf->d_gather_pose.as<unsigned char>();
+        const NcclApi& nc = nccl_api();
+        {
+            NvtxRange nr("locreg:align_loam_batch:allgather");
+            LR_NCCL(nc.GroupStart());
+            for (int r = 0; r < surf->comm_world; ++r) {
+                size_t rlo = 0, rhi = 0;
+                locreg_shard_range(S_global, r, surf->comm_world, &rlo, &rhi);
+                const size_t n = rhi - rlo;
+                if (n == 0) continue;
+                const bool me = r == surf->comm_rank;
+                LR_NCCL(nc.Broadcast(me ? dl : nullptr, dg + rlo * 7 * sizeof(double), n * 7, ncclDouble, r, surf->comm, surf->stream));
+                LR_NCCL(nc.Broadcast(me ? dl + ll.res_off : nullptr, dg + gl.res_off + rlo * sizeof(DevResult), n * sizeof(DevResult),
+                                     ncclUint8, r, surf->comm, surf->stream));
+                LR_NCCL(nc.Broadcast(me ? dl + ll.half_off : nullptr, dg + gl.half_off + 2 * rlo * sizeof(DevResult),
+                                     2 * n * sizeof(DevResult), ncclUint8, r, surf->comm, surf->stream));
+            }
+            LR_NCCL(nc.GroupEnd());
+        }
+        loam_copy_back(surf, dg, S_global, poses_out, results);
+        return LOCREG_OK;
+    });
 }
 
 int locreg_knn(locreg_handle* h, const float* queries, size_t nq, size_t stride, int32_t k, int32_t* idx) {

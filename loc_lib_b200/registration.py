@@ -428,19 +428,37 @@ class LoamRegistration:
         """S independent ScanMatch calls in one device-resident loop (locreg_align_loam_batch).  Scan s is
         surf_clouds[surf_offsets[s]:surf_offsets[s + 1]] and edge_clouds[edge_offsets[s]:edge_offsets[s + 1]].
         Returns (poses (S, 7), [(res_surf, res_edge)] * S), each scan's exactly what its ScanMatch call returns."""
-        a, _, s_s, b, _ = self._clouds(surf_clouds, edge_clouds)
-        so = np.ascontiguousarray(surf_offsets, np.int64)
-        eo = np.ascontiguousarray(edge_offsets, np.int64)
-        S = so.shape[0] - 1
-        if S < 0 or eo.shape != so.shape:
-            raise _lib.LocregError("surf_offsets and edge_offsets need S + 1 entries each")
-        pin = np.ascontiguousarray(predict_poses, np.float64).reshape(S, 7)
+        a, so, b, eo, s_s, pin = self._batch(surf_clouds, surf_offsets, edge_clouds, edge_offsets, predict_poses)
+        S = pin.shape[0]
         pout = pin.copy()
         res = (_lib.Result * (2 * S))()
         _lib.check(_lib.lib().locreg_align_loam_batch(self.surf._h, self.edge._h, a.ctypes.data, so.ctypes.data, b.ctypes.data,
                                                       eo.ctypes.data, s_s, pin.ctypes.data, S, self.max_iteration, self.eps,
                                                       pout.ctypes.data, res))
         return pout, [(res[2 * s].as_dict(), res[2 * s + 1].as_dict()) for s in range(S)]
+
+    def ScanMatchBatchSharded(self, surf_clouds, surf_offsets, edge_clouds, edge_offsets, predict_poses, S_global):
+        """ScanMatchBatch over the ranks of the surf handle's communicator (locreg_align_loam_batch_sharded): this rank
+        passes only its block of a batch of S_global scans (block partition: shard_range; offsets relative to its
+        clouds).  Returns (poses (S_global, 7), [(res_surf, res_edge)] * S_global) of ALL scans, bit for bit what
+        ScanMatchBatch of the whole batch returns on one GPU, on every rank."""
+        a, so, b, eo, s_s, pin = self._batch(surf_clouds, surf_offsets, edge_clouds, edge_offsets, predict_poses)
+        pout = np.zeros((S_global, 7))
+        res = (_lib.Result * (2 * S_global))()
+        _lib.check(_lib.lib().locreg_align_loam_batch_sharded(self.surf._h, self.edge._h, a.ctypes.data, so.ctypes.data,
+                                                              b.ctypes.data, eo.ctypes.data, s_s, pin.ctypes.data, pin.shape[0],
+                                                              S_global, self.max_iteration, self.eps, pout.ctypes.data, res))
+        return pout, [(res[2 * s].as_dict(), res[2 * s + 1].as_dict()) for s in range(S_global)]
+
+    def _batch(self, surf_clouds, surf_offsets, edge_clouds, edge_offsets, predict_poses):
+        """(surf cloud, surf offsets, edge cloud, edge offsets, stride, poses (S, 7)) of a batch's C-ABI arguments."""
+        a, _, s_s, b, _ = self._clouds(surf_clouds, edge_clouds)
+        so = np.ascontiguousarray(surf_offsets, np.int64)
+        eo = np.ascontiguousarray(edge_offsets, np.int64)
+        S = so.shape[0] - 1
+        if S < 0 or eo.shape != so.shape:
+            raise _lib.LocregError("surf_offsets and edge_offsets need S + 1 entries each")
+        return a, so, b, eo, s_s, np.ascontiguousarray(predict_poses, np.float64).reshape(S, 7)
 
     def Relocalise(self, surf_cloud, edge_cloud, hypotheses, want_all=False):
         """Global relocalisation of one surf / edge scan (locreg_relocalise_loam): every hypothesis runs the ScanMatch
@@ -509,7 +527,7 @@ class LoamRegistration:
                       rounds.ctypes.data if want_all else None))
         return best_pose, int(best_idx.value), float(best_score.value), scores, poses, rounds
 
-    # the communicator of the sharded relocalisation is the surf handle's (loc_lib_b200.dist.comm_init works unchanged)
+    # the communicator of the sharded calls is the surf handle's (loc_lib_b200.dist.comm_init works unchanged)
     CommUniqueId = staticmethod(_Registration.CommUniqueId)
 
     def CommInit(self, unique_id, rank, world):
