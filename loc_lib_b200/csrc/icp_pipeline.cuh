@@ -586,8 +586,13 @@ __device__ __forceinline__ void icp_rings_warps(unsigned int n, unsigned int war
         icp_rings_query<K>(queue.entries[e], map, coarse, bv, states, nn_pos, track);
     }
 }
+// Stage 2 of the warp-per-query kernels below: launched with 128 threads.  Without a register budget ptxas settles at 80
+// registers and spills (68 B stored, 136 B loaded per thread in k_icp_nn_rings<5>); with one of 96 it uses 89 and none.
+#ifndef LR_RINGS_MAXNREG
+#define LR_RINGS_MAXNREG 96
+#endif
 template <int K>
-__global__ void __launch_bounds__(128) k_icp_nn_rings(VoxelMapView map, CoarseLevels coarse, BatchView bv,
+__global__ void __maxnreg__(LR_RINGS_MAXNREG) k_icp_nn_rings(VoxelMapView map, CoarseLevels coarse, BatchView bv,
                                                       const AlignState* __restrict__ states, unsigned int* __restrict__ nn_pos,
                                                       KnnTrack* track, RingQueue queue, unsigned int max_count) {
     const unsigned int n = *queue.count;
@@ -618,7 +623,7 @@ __global__ void __launch_bounds__(kTile, LR_NN_MIN_BLOCKS) k_knn_stage1(VoxelMap
     tile_queue_append(!done, i, 0u, &blk_pending, &blk_done, staged, queue);
 }
 template <int K>
-__global__ void __launch_bounds__(128) k_knn_rings(VoxelMapView map, CoarseLevels coarse, const float4* __restrict__ q,
+__global__ void __maxnreg__(LR_RINGS_MAXNREG) k_knn_rings(VoxelMapView map, CoarseLevels coarse, const float4* __restrict__ q,
                                                    unsigned int* __restrict__ nn_pos, RingQueue queue) {
     const unsigned int n = *queue.count;
     const unsigned int lane = threadIdx.x & 31;
@@ -645,8 +650,9 @@ __global__ void __launch_bounds__(128) k_knn_rings(VoxelMapView map, CoarseLevel
         }
     }
 }
+// (launched with 128 threads; the budget keeps ptxas at 79 registers without spills, where it picks 72 and spills)
 template <int K>
-__global__ void __launch_bounds__(128) k_knn_finish(VoxelMapView map, CoarseLevels coarse, const float4* __restrict__ q,
+__global__ void __maxnreg__(80) k_knn_finish(VoxelMapView map, CoarseLevels coarse, const float4* __restrict__ q,
                                                     unsigned int* __restrict__ nn_pos, RingQueue queue) {
     const unsigned int n = *queue.count;
     for (unsigned int e = blockIdx.x * blockDim.x + threadIdx.x; e < n; e += gridDim.x * blockDim.x) {

@@ -184,14 +184,28 @@ LR_HD bool knn_accepts(const float4* pts, const KnnResult<K>& r, float d2, unsig
     if (d2 == r.d2[K - 1]) return knn_index_of(pts, pos) < knn_index_of(pts, r.pos[K - 1]);
     return true;
 }
-// Sorted insertion of an accepted candidate (precondition: it precedes r[K-1]); straight-line selects, no branches
-// besides the tie lookups.
+// Sorted insertion of an accepted candidate (precondition: it precedes r[K-1]); straight-line selects.  Exact distance
+// ties between distinct points are rare, so the comparisons are made on dis2 alone: where the candidate's dis2 differs
+// from a slot's, `d2 < r.d2[j]` IS the (dis2, original index) order.  Only a candidate whose dis2 equals that of one of
+// the slots it is compared with looks the indices up, and only for those slots.
 template <int K>
 LR_HD void knn_insert(const float4* pts, KnnResult<K>& r, float d2, unsigned int pos) {
+    unsigned int before = 0u;  // bit j: the candidate precedes slot j
+    bool tie = false;
+#pragma unroll
+    for (int j = 0; j + 1 < K; ++j) {
+        before |= (d2 < r.d2[j] ? 1u : 0u) << j;
+        tie = tie || d2 == r.d2[j];
+    }
+    if (tie) {
+#pragma unroll
+        for (int j = 0; j + 1 < K; ++j)
+            if (d2 == r.d2[j] && knn_index_of(pts, pos) < knn_index_of(pts, r.pos[j])) before |= 1u << j;
+    }
     bool before_old = true;  // candidate precedes the element that sat in slot j before this insertion
 #pragma unroll
     for (int j = K - 1; j >= 1; --j) {
-        const bool before_prev = knn_less(pts, d2, pos, r.d2[j - 1], r.pos[j - 1]);
+        const bool before_prev = (before >> (j - 1)) & 1u;
         const float nd = before_prev ? r.d2[j - 1] : (before_old ? d2 : r.d2[j]);
         const unsigned int np = before_prev ? r.pos[j - 1] : (before_old ? pos : r.pos[j]);
         r.d2[j] = nd;
@@ -408,13 +422,28 @@ LR_HD void knn_seed(const VoxelMapView& m, float qx, float qy, float qz, const u
         res.pos[j] = seeds[j];
     }
     if (K == 5) {
+        // on dis2 alone first (as knn_insert); if a comparator met two equal distances the (dis2, original index) order
+        // decides: the exact network sorts any permutation of the K distinct seeds into that one order, so it runs over
+        // what the first pass left
         constexpr int net[9][2] = {{0, 1}, {3, 4}, {2, 4}, {2, 3}, {1, 4}, {0, 3}, {0, 2}, {1, 3}, {1, 2}};
+        bool tie = false;
 #pragma unroll
         for (int c = 0; c < 9; ++c) {
             const int a = net[c][0], b = net[c][1];
-            if (knn_less(m.pts, res.d2[b], res.pos[b], res.d2[a], res.pos[a])) {
-                const float td = res.d2[a]; res.d2[a] = res.d2[b]; res.d2[b] = td;
-                const unsigned int tp = res.pos[a]; res.pos[a] = res.pos[b]; res.pos[b] = tp;
+            tie = tie || res.d2[b] == res.d2[a];
+            const bool sw = res.d2[b] < res.d2[a];
+            const float da = sw ? res.d2[b] : res.d2[a], db = sw ? res.d2[a] : res.d2[b];
+            const unsigned int pa = sw ? res.pos[b] : res.pos[a], pb = sw ? res.pos[a] : res.pos[b];
+            res.d2[a] = da; res.d2[b] = db; res.pos[a] = pa; res.pos[b] = pb;
+        }
+        if (tie) {
+#pragma unroll
+            for (int c = 0; c < 9; ++c) {
+                const int a = net[c][0], b = net[c][1];
+                if (knn_less(m.pts, res.d2[b], res.pos[b], res.d2[a], res.pos[a])) {
+                    const float td = res.d2[a]; res.d2[a] = res.d2[b]; res.d2[b] = td;
+                    const unsigned int tp = res.pos[a]; res.pos[a] = res.pos[b]; res.pos[b] = tp;
+                }
             }
         }
     }
