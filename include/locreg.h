@@ -369,6 +369,33 @@ int locreg_filter_crop_box(locreg_handle* h, const float* xyz, size_t n, size_t 
                            const float* max3, float* out_xyz, size_t* n_out);
 int locreg_filter_voxel_grid(locreg_handle* h, const float* xyz, size_t n, size_t stride_bytes, float leaf_size,
                              float* out_xyz, size_t* n_out);
+/* pcl::removeNaNFromPointCloud / pcl::VoxelGrid of every scan of a batch; scan s = points [offsets[s], offsets[s+1])
+ * of xyz (offsets relative to xyz, non-decreasing).  out_xyz has room for offsets[S] - offsets[0] points of the same
+ * stride; out_offsets (S + 1, relative to out_xyz, out_offsets[0] = 0) receives the filtered batch's offsets.  Segment s
+ * is byte for byte locreg_filter_remove_nan / locreg_filter_voxel_grid of scan s alone (empty scans, scans without a
+ * finite point and scans whose grid would overflow PCL's int index included).  One pass over the whole batch: the
+ * launches do not depend on S, and the call synchronises twice (voxel grid: once after the per-scan bounding boxes,
+ * once at the end; NaN removal: once).  The voxel grid's per-scan bitmaps are processed in waves of at most
+ * LOCREG_FILTER_WAVE_MIB MiB (default 1 GiB, less when free memory is short); the waves do not change results.
+ * Arguments are checked before any device work: LOCREG_E_ARG for a null offsets / out_offsets, a null out_xyz with
+ * points in the batch, decreasing or negative offsets, bad cloud arguments, S >= 2^31, leaf_size <= 0.
+ * locreg_last_timing covers the filter kernels. */
+int locreg_filter_remove_nan_batch(locreg_handle* h, const float* xyz, const int64_t* offsets, size_t S,
+                                   size_t stride_bytes, float* out_xyz, int64_t* out_offsets);
+int locreg_filter_voxel_grid_batch(locreg_handle* h, const float* xyz, const int64_t* offsets, size_t S,
+                                   size_t stride_bytes, float leaf_size, float* out_xyz, int64_t* out_offsets);
+
+/* Loc::Update's front end and ScanMatch for every scan of a batch: scan s is RemoveNanPoint then VoxelFilter(leaf_size)
+ * (the order of loc.cpp:217-218; lio.cpp's order gives the same cloud), then registered exactly as locreg_align_batch
+ * registers it.  The filtered clouds never leave the device.  poses_in / poses_out / results as in locreg_align_batch;
+ * n_filtered (S entries or NULL) receives each filtered scan's size.  Poses and results are bit for bit those of
+ * locreg_align_batch on the concatenation of locreg_filter_voxel_grid(locreg_filter_remove_nan(scan s)).  Every handle
+ * type locreg_align_batch accepts works.  The raw batch goes to the device in one copy (not in chunks).  Arguments are
+ * checked before any device work as in locreg_align_batch, plus LOCREG_E_ARG for leaf_size <= 0; a failing call
+ * writes nothing.  locreg_last_timing covers the filter and the registration kernels. */
+int locreg_align_batch_filtered(locreg_handle* h, const float* srcs, const int64_t* offsets, size_t stride_bytes,
+                                const double* poses_in, size_t S, float leaf_size, double* poses_out,
+                                locreg_result* results, int64_t* n_filtered);
 
 /* Caller state kept on the device (Loc, LocUtils/src/slam/3d/loc.cpp): the global map is uploaded once
  * (Loc::InitGlobalMap, loc.cpp:268-283); locreg_reset_local_map is Loc::ResetLocalMap (loc.cpp:187-206) -

@@ -23,7 +23,8 @@ SYMBOLS = [
     "locreg_relocalise_sharded", "locreg_align_batch_sharded", "locreg_index_info", "locreg_align_loam",
     "locreg_align_loam_batch", "locreg_relocalise_loam", "locreg_relocalise_loam_sharded", "locreg_relocalise_staged",
     "locreg_relocalise_staged_sharded", "locreg_relocalise_loam_staged", "locreg_relocalise_loam_staged_sharded",
-    "locreg_align_loam_batch_sharded",
+    "locreg_align_loam_batch_sharded", "locreg_filter_remove_nan_batch", "locreg_filter_voxel_grid_batch",
+    "locreg_align_batch_filtered",
 ]
 
 
@@ -95,6 +96,9 @@ def lib():
         L.locreg_filter_remove_nan.argtypes = [vp, vp, sz, sz, vp, C.POINTER(sz)]
         L.locreg_filter_crop_box.argtypes = [vp, vp, sz, sz, vp, vp, vp, C.POINTER(sz)]
         L.locreg_filter_voxel_grid.argtypes = [vp, vp, sz, sz, C.c_float, vp, C.POINTER(sz)]
+        L.locreg_filter_remove_nan_batch.argtypes = [vp, vp, vp, sz, sz, vp, vp]
+        L.locreg_filter_voxel_grid_batch.argtypes = [vp, vp, vp, sz, sz, C.c_float, vp, vp]
+        L.locreg_align_batch_filtered.argtypes = [vp, vp, vp, sz, vp, sz, C.c_float, vp, vp, vp]
         L.locreg_comm_unique_id.argtypes = [vp]
         L.locreg_comm_init.argtypes = [vp, vp, i32, i32]
         L.locreg_comm_destroy.argtypes = [vp]

@@ -108,6 +108,7 @@ struct locreg_handle {
     DevBuf d_gather_pose, d_gather_res, d_bcast;
     DevBuf d_raw, d_src4, d_out, d_partials, d_state, d_acc, d_gate, d_nn, d_offsets, d_poses_in, d_poses_out, d_results,
         d_scores, d_misc, d_target, d_nnpos, d_tile_begin, d_tiles, d_states, d_ringq, d_ringc, d_sortq, d_sortb, d_sorth, d_rescanq, d_rescanc, d_loam, d_lmap_new, d_global, d_local, d_same, d_plane, d_pstat, d_track;
+    DevBuf d_filt;  // locreg_align_batch_filtered: the filtered batch
     // locreg_relocalise_staged: the cut's keys, flags / slots, the two index maps of the rounds, the caller-order
     // outputs, and the select state + histogram + best
     DevBuf d_stage_keys, d_stage_slot, d_stage_idx, d_stage_poses, d_stage_scores, d_stage_rounds, d_stage_sel;
@@ -174,11 +175,9 @@ namespace { void prof_collect(locreg_handle* h); }
 
 namespace {
 
-// Copies a host (or device) cloud into h->d_raw as-is and produces the float4 view kernels read.
-// Returns the float4 device pointer.
-const float4* stage_cloud(locreg_handle* h, const float* src, size_t n, size_t stride, bool src_on_device) {
+// Copies a host (or device) cloud into h->d_raw as-is (n > 0).
+void stage_raw(locreg_handle* h, const float* src, size_t n, size_t stride, bool src_on_device) {
     const size_t bytes = n * stride;
-    if (n == 0) return nullptr;
     h->d_raw.reserve(bytes);
     if (src_on_device) {
         LR_CUDA(cudaMemcpyAsync(h->d_raw.p, src, bytes, cudaMemcpyDeviceToDevice, h->stream));
@@ -189,11 +188,21 @@ const float4* stage_cloud(locreg_handle* h, const float* src, size_t n, size_t s
         std::memcpy(h->h_in.p, src, bytes);
         LR_CUDA(cudaMemcpyAsync(h->d_raw.p, h->h_in.p, bytes, cudaMemcpyHostToDevice, h->stream));
     }
-    if (stride == 16) return h->d_raw.as<float4>();
+}
+// The float4 view kernels read of a device cloud (in place when the stride is already 16, else packed into h->d_src4).
+const float4* float4_view(locreg_handle* h, const unsigned char* d_cloud, size_t n, size_t stride) {
+    if (stride == 16) return reinterpret_cast<const float4*>(d_cloud);
     h->d_src4.reserve(n * sizeof(float4));
     const unsigned int grid = static_cast<unsigned int>(std::min<size_t>((n + 255) / 256, 4096));
-    LR_LAUNCH(k_pack_float4, grid, 256, 0, h->stream, h->d_raw.as<unsigned char>(), n, stride, h->d_src4.as<float4>());
+    LR_LAUNCH(k_pack_float4, grid, 256, 0, h->stream, d_cloud, n, stride, h->d_src4.as<float4>());
     return h->d_src4.as<float4>();
+}
+// Copies a host (or device) cloud into h->d_raw as-is and produces the float4 view kernels read.
+// Returns the float4 device pointer.
+const float4* stage_cloud(locreg_handle* h, const float* src, size_t n, size_t stride, bool src_on_device) {
+    if (n == 0) return nullptr;
+    stage_raw(h, src, n, stride, src_on_device);
+    return float4_view(h, h->d_raw.as<unsigned char>(), n, stride);
 }
 
 // align = true: the pose starts an Align* loop, which honours zero_initial_translation (see locreg.h)
@@ -1260,6 +1269,33 @@ int locreg_align_batch_device(locreg_handle* h, const float* d_srcs, const int64
     });
 }
 
+// A batch's offsets (S + 1, relative to its first point) and poses -> h->d_offsets / d_poses_in / d_poses_out;
+// poses_out_init = the IN values of the IN/OUT poses_out.
+static void load_batch_args(locreg_handle* h, const long long* rel, const double* poses_in, const double* poses_out_init, size_t S) {
+    h->d_offsets.reserve((S + 1) * sizeof(long long));
+    h->d_poses_in.reserve(S * 7 * sizeof(double));
+    h->d_poses_out.reserve(S * 7 * sizeof(double));
+    h->d_results.reserve(S * sizeof(DevResult));
+    LR_CUDA(cudaMemcpyAsync(h->d_offsets.p, rel, (S + 1) * sizeof(long long), cudaMemcpyHostToDevice, h->stream));
+    LR_CUDA(cudaMemcpyAsync(h->d_poses_in.p, poses_in, S * 7 * sizeof(double), cudaMemcpyHostToDevice, h->stream));
+    LR_CUDA(cudaMemcpyAsync(h->d_poses_out.p, poses_out_init, S * 7 * sizeof(double), cudaMemcpyHostToDevice, h->stream));
+    LR_CUDA(cudaStreamSynchronize(h->stream));  // rel[] is pageable
+}
+// The registration of a batch resident on the device: S scans of float4 points src4 (n_pts in all), offsets and poses
+// in h->d_offsets / d_poses_in / d_poses_out (load_batch_args); poses and results are left in h->d_poses_out / d_results.
+static void align_batch_loaded(locreg_handle* h, const float4* src4, size_t n_pts, size_t S) {
+    const unsigned int Su = static_cast<unsigned int>(S);
+    if (is_ndt(h)) {
+        NDT_DISPATCH(h, ndt_run_batch(h, PB, src4, h->d_offsets.as<long long>(), h->d_poses_in.as<double>(),
+                                      h->d_poses_out.as<double>(), h->d_results.as<DevResult>(), Su));
+    } else {
+        const IcpJob job = icp_batch_job(h, src4, h->d_offsets.as<long long>(), Su, n_pts);
+        LR_LAUNCH(k_states_init, (Su + 255) / 256, 256, 0, h->stream, h->d_poses_in.as<double>(), Su, h->opt.max_iteration, h->opt.zero_initial_translation, job.states);
+        ICP_DISPATCH(h, icp_run_loop<M>(h, job, 0));
+        LR_LAUNCH(k_states_export, (Su + 255) / 256, 256, 0, h->stream, job.states, Su, h->d_poses_out.as<double>(), h->d_results.as<DevResult>());
+    }
+}
+
 // S ScanMatch calls of a host batch; the poses and results stay in h->d_poses_out / h->d_results (S entries, device).
 // offsets[0..S] are relative to srcs; poses_out_init = the IN values of the IN/OUT poses_out.
 static void align_batch_resident(locreg_handle* h, const float* srcs, const int64_t* offsets, size_t stride, const double* poses_in,
@@ -1274,17 +1310,9 @@ static void align_batch_resident(locreg_handle* h, const float* srcs, const int6
     // chunk c + 1 runs on a second stream while chunk c is being registered (scans are independent).
     const bool pipelined = !is_ndt(h) && S >= 16 && n_pts >= (1u << 20) && is_pinned_or_device(first);
     const float4* src4 = pipelined ? nullptr : stage_cloud(h, first, n_pts, stride, false);
-    h->d_offsets.reserve((S + 1) * sizeof(long long));
-    h->d_poses_in.reserve(S * 7 * sizeof(double));
-    h->d_poses_out.reserve(S * 7 * sizeof(double));
-    h->d_results.reserve(S * sizeof(DevResult));
     std::vector<long long> rel(S + 1);
     for (size_t s = 0; s <= S; ++s) rel[s] = offsets[s] - static_cast<long long>(base);
-    LR_CUDA(cudaMemcpyAsync(h->d_offsets.p, rel.data(), (S + 1) * sizeof(long long), cudaMemcpyHostToDevice, h->stream));
-    LR_CUDA(cudaMemcpyAsync(h->d_poses_in.p, poses_in, S * 7 * sizeof(double), cudaMemcpyHostToDevice, h->stream));
-    LR_CUDA(cudaMemcpyAsync(h->d_poses_out.p, poses_out, S * 7 * sizeof(double), cudaMemcpyHostToDevice, h->stream));
-    LR_CUDA(cudaStreamSynchronize(h->stream));  // rel[] is pageable
-    const unsigned int Su = static_cast<unsigned int>(S);
+    load_batch_args(h, rel.data(), poses_in, poses_out, S);
     if (pipelined) {
         // LOCREG_CHUNK_STREAMS (default 1): every chunk runs its Gauss-Newton loop on its own stream as soon as its copy has
         // landed, concurrently with the chunks before it.  A chunk's loop is ~70 dependent kernels, each ending in a tail
@@ -1426,27 +1454,24 @@ static void align_batch_resident(locreg_handle* h, const float* srcs, const int6
         h->end_timing();
     } else {
         h->begin_timing();
-        if (is_ndt(h)) {
-            NDT_DISPATCH(h, ndt_run_batch(h, PB, src4, h->d_offsets.as<long long>(), h->d_poses_in.as<double>(),
-                                          h->d_poses_out.as<double>(), h->d_results.as<DevResult>(), Su));
-        } else {
-            const IcpJob job = icp_batch_job(h, src4, h->d_offsets.as<long long>(), Su, n_pts);
-            LR_LAUNCH(k_states_init, (Su + 255) / 256, 256, 0, h->stream, h->d_poses_in.as<double>(), Su, h->opt.max_iteration, h->opt.zero_initial_translation, job.states);
-            ICP_DISPATCH(h, icp_run_loop<M>(h, job, 0));
-            LR_LAUNCH(k_states_export, (Su + 255) / 256, 256, 0, h->stream, job.states, Su, h->d_poses_out.as<double>(), h->d_results.as<DevResult>());
-        }
+        align_batch_loaded(h, src4, n_pts, S);
         h->end_timing();
     }
 }
 
-static int align_batch_check(const float* srcs, const int64_t* offsets, size_t stride, const double* poses_in, size_t S, double* poses_out) {
-    if (!offsets || !poses_in || !poses_out) { g_last_error = "null argument"; return LOCREG_E_ARG; }
+// offsets (S + 1, relative to srcs, non-decreasing) and the cloud they cut
+static int batch_cloud_check(const float* srcs, const int64_t* offsets, size_t stride, size_t S) {
+    if (!offsets) { g_last_error = "null argument"; return LOCREG_E_ARG; }
     if (S >= (1ull << 31)) { g_last_error = "too many scans"; return LOCREG_E_ARG; }
     for (size_t s = 0; s < S; ++s)
         if (offsets[s + 1] < offsets[s] || offsets[s] < 0) { g_last_error = "offsets must be non-decreasing"; return LOCREG_E_ARG; }
     const size_t total = static_cast<size_t>(offsets[S]);
     const float* first = reinterpret_cast<const float*>(reinterpret_cast<const char*>(srcs) + static_cast<size_t>(offsets[0]) * stride);
     return check_cloud_args(first, total - static_cast<size_t>(offsets[0]), stride);
+}
+static int align_batch_check(const float* srcs, const int64_t* offsets, size_t stride, const double* poses_in, size_t S, double* poses_out) {
+    if (!offsets || !poses_in || !poses_out) { g_last_error = "null argument"; return LOCREG_E_ARG; }
+    return batch_cloud_check(srcs, offsets, stride, S);
 }
 
 int locreg_align_batch(locreg_handle* h, const float* srcs, const int64_t* offsets, size_t stride, const double* poses_in,
@@ -2310,6 +2335,81 @@ int locreg_filter_crop_box(locreg_handle* h, const float* xyz, size_t n, size_t 
 }
 int locreg_filter_voxel_grid(locreg_handle* h, const float* xyz, size_t n, size_t stride, float leaf_size, float* out_xyz, size_t* n_out) {
     return filter_impl(h, 2, xyz, n, stride, &leaf_size, nullptr, out_xyz, n_out);
+}
+
+// kind: 0 remove NaN, 2 voxel grid (as filter_impl).  The batch is relative to its first point on the device.
+static int filter_batch_impl(locreg_handle* h, int kind, const float* xyz, const int64_t* offsets, size_t S, size_t stride,
+                             float leaf, float* out_xyz, int64_t* out_offsets) {
+    const int rc = batch_cloud_check(xyz, offsets, stride, S);
+    if (rc) return rc;
+    const size_t n = static_cast<size_t>(offsets[S] - offsets[0]);
+    if (!out_offsets || (n && !out_xyz)) { g_last_error = "null argument"; return LOCREG_E_ARG; }
+    if (kind == 2 && !(leaf > 0)) { g_last_error = "leaf size must be > 0"; return LOCREG_E_ARG; }
+    return guarded(h, [&]() {
+        std::vector<long long> rel(S + 1), out(S + 1, 0);
+        for (size_t s = 0; s <= S; ++s) rel[s] = offsets[s] - offsets[0];
+        if (n) {
+            stage_raw(h, reinterpret_cast<const float*>(reinterpret_cast<const char*>(xyz) + static_cast<size_t>(offsets[0]) * stride), n,
+                      stride, false);
+            h->d_out.reserve(n * stride);
+        }
+        h->begin_timing();
+        if (n && kind == 0) filter_remove_nan_batch(h->d_raw.as<unsigned char>(), rel.data(), S, stride, h->d_out.as<unsigned char>(), out.data(), h->stream);
+        else if (n) filter_voxel_grid_batch(h->d_raw.as<unsigned char>(), rel.data(), S, stride, leaf, h->d_out.as<unsigned char>(), out.data(), h->stream);
+        h->end_timing();
+        if (out[S]) LR_CUDA(cudaMemcpy(out_xyz, h->d_out.p, static_cast<size_t>(out[S]) * stride, cudaMemcpyDeviceToHost));
+        std::copy(out.begin(), out.end(), out_offsets);
+        return LOCREG_OK;
+    });
+}
+int locreg_filter_remove_nan_batch(locreg_handle* h, const float* xyz, const int64_t* offsets, size_t S, size_t stride_bytes,
+                                   float* out_xyz, int64_t* out_offsets) {
+    return filter_batch_impl(h, 0, xyz, offsets, S, stride_bytes, 0.0f, out_xyz, out_offsets);
+}
+int locreg_filter_voxel_grid_batch(locreg_handle* h, const float* xyz, const int64_t* offsets, size_t S, size_t stride_bytes,
+                                   float leaf_size, float* out_xyz, int64_t* out_offsets) {
+    return filter_batch_impl(h, 2, xyz, offsets, S, stride_bytes, leaf_size, out_xyz, out_offsets);
+}
+
+// Loc::Update's front end (loc.cpp:217-218) in front of locreg_align_batch: the raw batch goes up in one copy, is
+// filtered per scan on the device and registered from there, as align_batch_resident registers a resident batch.
+int locreg_align_batch_filtered(locreg_handle* h, const float* srcs, const int64_t* offsets, size_t stride_bytes,
+                                const double* poses_in, size_t S, float leaf_size, double* poses_out, locreg_result* results,
+                                int64_t* n_filtered) {
+    if (S == 0) return LOCREG_OK;
+    const int rc = align_batch_check(srcs, offsets, stride_bytes, poses_in, S, poses_out);
+    if (rc) return rc;
+    if (!(leaf_size > 0)) { g_last_error = "leaf size must be > 0"; return LOCREG_E_ARG; }
+    return guarded(h, [&]() {
+        if (!h->has_target) { g_last_error = "SetInputTarget has not been called"; return LOCREG_E_STATE; }
+        NvtxRange nvtx_r("locreg:align_batch_filtered");
+        const size_t stride = stride_bytes;
+        const size_t n = static_cast<size_t>(offsets[S] - offsets[0]);
+        std::vector<long long> rel(S + 1), kept(S + 1, 0), filt(S + 1, 0);
+        for (size_t s = 0; s <= S; ++s) rel[s] = offsets[s] - offsets[0];
+        if (n) {
+            stage_raw(h, reinterpret_cast<const float*>(reinterpret_cast<const char*>(srcs) + static_cast<size_t>(offsets[0]) * stride), n,
+                      stride, false);
+            h->d_out.reserve(n * stride);
+            h->d_filt.reserve(n * stride);
+        }
+        h->begin_timing();
+        const float4* src4 = nullptr;
+        if (n) {
+            filter_remove_nan_batch(h->d_raw.as<unsigned char>(), rel.data(), S, stride, h->d_out.as<unsigned char>(), kept.data(), h->stream);
+            filter_voxel_grid_batch(h->d_out.as<unsigned char>(), kept.data(), S, stride, leaf_size, h->d_filt.as<unsigned char>(),
+                                    filt.data(), h->stream);
+            if (filt[S]) src4 = float4_view(h, h->d_filt.as<unsigned char>(), static_cast<size_t>(filt[S]), stride);
+        }
+        load_batch_args(h, filt.data(), poses_in, poses_out, S);
+        align_batch_loaded(h, src4, static_cast<size_t>(filt[S]), S);
+        h->end_timing();
+        LR_CUDA(cudaMemcpy(poses_out, h->d_poses_out.p, S * 7 * sizeof(double), cudaMemcpyDeviceToHost));
+        if (results) LR_CUDA(cudaMemcpy(results, h->d_results.p, S * sizeof(DevResult), cudaMemcpyDeviceToHost));
+        if (n_filtered)
+            for (size_t s = 0; s < S; ++s) n_filtered[s] = filt[s + 1] - filt[s];
+        return LOCREG_OK;
+    });
 }
 
 int locreg_ndt_num_voxels(locreg_handle* h, size_t* nv) {

@@ -161,6 +161,21 @@ class _Registration:
                                                  pout.ctypes.data, res))
         return pout, [r.as_dict() for r in res]
 
+    def ScanMatchBatchFiltered(self, clouds, offsets, predict_poses, voxel_size, result_poses_init=None):
+        """ScanMatchBatch of raw scans: each scan is RemoveNanPoint'ed and VoxelFilter'ed (voxel_size) on the device first
+        (Loc::Update's front end, locreg_align_batch_filtered).  Returns (poses, results, n_filtered): poses and results
+        as ScanMatchBatch returns them for the filtered scans, n_filtered the size of each filtered scan."""
+        a, n, s = _cloud(clouds)
+        offsets = np.ascontiguousarray(offsets, np.int64)
+        S = offsets.shape[0] - 1
+        pin = np.ascontiguousarray(predict_poses, np.float64).reshape(S, 7)
+        pout = pin.copy() if result_poses_init is None else np.ascontiguousarray(result_poses_init, np.float64).copy()
+        res = (_lib.Result * S)()
+        n_filtered = np.zeros(S, np.int64)
+        _lib.check(_lib.lib().locreg_align_batch_filtered(self._h, a.ctypes.data, offsets.ctypes.data, s, pin.ctypes.data, S,
+                                                          C.c_float(voxel_size), pout.ctypes.data, res, n_filtered.ctypes.data))
+        return pout, [r.as_dict() for r in res], n_filtered
+
     def Relocalise(self, cloud, hypotheses, want_all=False):
         a, n, s = _cloud(cloud)
         hyp = np.ascontiguousarray(hypotheses, np.float64).reshape(-1, 7)
@@ -302,6 +317,24 @@ class _Registration:
     def VoxelFilter(self, cloud, voxel_size):
         """VoxelFilter::Filter = pcl::VoxelGrid with a cubic leaf (voxel_filter.cpp:10-26)."""
         return self._filter(_lib.lib().locreg_filter_voxel_grid, cloud, C.c_float(voxel_size))
+
+    def _filter_batch(self, fn, clouds, offsets, *args):
+        a, n, s = _cloud(clouds)
+        offsets = np.ascontiguousarray(offsets, np.int64)
+        S = offsets.shape[0] - 1
+        out = np.empty_like(a)
+        out_offsets = np.zeros(S + 1, np.int64)
+        _lib.check(fn(self._h, a.ctypes.data, offsets.ctypes.data, S, s, *args, out.ctypes.data, out_offsets.ctypes.data))
+        return out[:out_offsets[-1]], out_offsets
+
+    def RemoveNanPointBatch(self, clouds, offsets):
+        """RemoveNanPoint of every scan of a batch (scan s = clouds[offsets[s]:offsets[s + 1]]) in one device pass.
+        Returns (filtered, out_offsets): scan s's result is filtered[out_offsets[s]:out_offsets[s + 1]]."""
+        return self._filter_batch(_lib.lib().locreg_filter_remove_nan_batch, clouds, offsets)
+
+    def VoxelFilterBatch(self, clouds, offsets, voxel_size):
+        """VoxelFilter of every scan of a batch in one device pass; returns (filtered, out_offsets) as RemoveNanPointBatch."""
+        return self._filter_batch(_lib.lib().locreg_filter_voxel_grid_batch, clouds, offsets, C.c_float(voxel_size))
 
     # ---- Loc's map state on the device (loc.cpp:187-206, 268-283) ----
     def SetGlobalMap(self, cloud):
